@@ -23,6 +23,11 @@ read back to the host.  Beside them, in the same line:
   workloads   BASELINE.json's other configs: c2a (attention over the 7x7x2048 grid), c3 (Monte-Carlo rollouts),
               c4 (hidden 1024, vocab 30k: one GPU's 128 rows), c5 (discriminator-only, 4096 + 4096 captions of length 32)
   comm        (N > 1) exposed milliseconds of the gradient exchange, its transport, and whether the replicas are bit-identical
+
+--dump-outputs DIR writes what the last timed step computed (see dump_outputs) so that two builds can be compared output for
+output: the inputs and the weights are seeded, so the same arguments give the same inputs on every run.  The step itself
+is not bit-reproducible (two runs of one build differ in the last bits, and the Adam updates carry that over the steps
+before the dumped one), so compare with a tolerance.
 """
 from __future__ import annotations
 
@@ -36,6 +41,7 @@ import sys
 import threading
 import time
 
+sys.dont_write_bytecode = True                   # the benchmark leaves the tree it runs from as it found it
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
@@ -117,6 +123,34 @@ class ClockSampler:
                     reasons=sorted(reasons), samples=len(sm))
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path, out, modules):
+    """--dump-outputs: one step's results as <path>/<name>.npy -- every tensor of the dict the step returned, under its key,
+    and the state of each model after the step (the updated weights and buffers) as <tag>.<state_dict key>.  Floating
+    tensors are written in float32 (float64 stays float64), integer ones in float64, which holds them exactly.  When the
+    whole set would exceed DUMP_BYTES, every array of more than `cap` entries is replaced by `cap` of its flattened
+    entries, drawn with a fixed seed: the same entries on every run, so that two builds compare entry for entry."""
+    import numpy as np
+    import torch
+    arrays = {k: v.detach() for k, v in out.items() if isinstance(v, torch.Tensor)}
+    for tag, m in modules.items():
+        arrays.update({f"{tag}.{k}": v.detach() for k, v in m.state_dict().items()})
+    wide = {k for k, v in arrays.items() if v.dtype == torch.float64 or not v.is_floating_point()}
+    cap = 1 << 24
+    while sum(min(v.numel(), cap) * (8 if k in wide else 4) for k, v in arrays.items()) > DUMP_BYTES:
+        cap //= 2
+    os.makedirs(path, exist_ok=True)
+    for k, v in arrays.items():
+        if v.numel() > cap:
+            idx = np.sort(np.random.default_rng(1008).choice(v.numel(), cap, replace=False))
+            v = v.reshape(-1)[torch.from_numpy(idx).to(v.device)]
+        np.save(os.path.join(path, k + ".npy"), (v.double() if k in wide else v.float()).cpu().numpy())
+    print("bench: %d arrays of the last timed step written to %s (arrays of more than %d entries sampled)" % (len(arrays), path, cap),
+          file=sys.stderr, flush=True)
+
+
 # ------------------------------------------------------------------------------------------------------
 # reference arm: the reference's CPU implementation (oracle port with the same torch library ops)
 # ------------------------------------------------------------------------------------------------------
@@ -158,7 +192,7 @@ def run_reference(args):
     cfg = WORKLOADS[args.workload]
     threads = os.cpu_count() or 1
     sample_B = min(cfg["B"], args.cpu_sample_rows or cfg["B"])
-    steps, warmup = max(1, min(args.steps, 3)), max(1, min(args.warmup, 1))
+    steps, warmup = args.steps, args.warmup
     t = cpu_reference_step_time(cfg, sample_B, steps, warmup, threads)
     scale = cfg["B"] / sample_B
     step_s = t * scale
@@ -240,10 +274,12 @@ def run_ours(args):
     h_pool = [s["pooled"].cpu().pin_memory() for s in sets]
 
     use_graph = not args.no_graph
+    last = {}
 
     def step_resident(i):
         s = sets[i % 2]
-        return inst.adv_step(s["caps"], pooled=s["pooled"], u=s["u"], keep=s["keep"], graph="static" if use_graph else False)
+        last["out"] = inst.adv_step(s["caps"], pooled=s["pooled"], u=s["u"], keep=s["keep"], graph="static" if use_graph else False)
+        return last["out"]
 
     # end to end: host buffers in, losses out.  Every step's two losses are copied to pinned host memory and READ on the host;
     # the read of step i happens while step i + 1 runs (one step of pipelining: the host never idles the GPU to fetch a number
@@ -310,6 +346,8 @@ def run_ours(args):
         step_resident(i)
     torch.cuda.synchronize()
     ms, launches, clocks = timed(step_resident, args.steps, args.warmup, sample_clocks=True)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last["out"], {"gen": inst.gen, "disc": inst.disc})
     ms_step = ms / args.steps
     value = world / (ms_step * 1e-3)             # global steps/s: every rank completes one 256-row step per iteration
 
@@ -597,9 +635,10 @@ def run_ours(args):
     shutdown()
 
 
-def run_workload(w, mode, dev, peaks, steps=None, world=1, rank=0):
+def run_workload(w, mode, dev, peaks, steps=None, world=1, rank=0, dump=None):
     """One of BASELINE.json's other configs on its own models: a dict for the `workloads` block of the headline line (or a
-    line of its own with --workload).  Device-resident synthetic inputs, two input sets alternating, CUDA events."""
+    line of its own with --workload).  Device-resident synthetic inputs, two input sets alternating, CUDA events.
+    dump: directory for dump_outputs of the last timed step (rank 0)."""
     import torch
     import torch.distributed as dist
     import gic_b200
@@ -666,8 +705,10 @@ def run_workload(w, mode, dev, peaks, steps=None, world=1, rank=0):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for i in range(k):
-        fn(i)
+        r = fn(i)
     e1.record(); torch.cuda.synchronize()
+    if dump and rank == 0:
+        dump_outputs(dump, r, {"gen": inst.gen, "disc": inst.disc})
     ms = e0.elapsed_time(e1)
     if world > 1:
         t = torch.tensor([ms], device=dev); dist.all_reduce(t, op=dist.ReduceOp.MAX); ms = float(t.item())
@@ -706,7 +747,7 @@ def run_secondary(args):
     dev = torch.device("cuda", local)
     if world > 1:
         dist.init_process_group("nccl", device_id=dev)
-    r = run_workload(args.workload, args.mode, dev, load_peaks(), steps=args.steps, world=world, rank=rank)
+    r = run_workload(args.workload, args.mode, dev, load_peaks(), steps=args.steps, world=world, rank=rank, dump=args.dump_outputs)
     if rank == 0:
         r.update({"n_gpus": world, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "secondary": True})
         print(json.dumps(r), flush=True)
@@ -731,7 +772,13 @@ def main():
     ap.add_argument("--no-modes", action="store_true", help="skip the tf32 / fp32 measurements of the same step")
     ap.add_argument("--no-workloads", action="store_true", help="skip the c2a / c3 / c4 / c5 block")
     ap.add_argument("--no-graph", action="store_true", help="enqueue every kernel from the host instead of replaying the captured step")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed as DIR/<name>.npy "
+                                                          "(float32 / float64, at most 64 MB: larger arrays as a fixed, seeded sample)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)

@@ -1,17 +1,17 @@
 """Generate tests/golden/*.npz by running the UNMODIFIED reference modules on CPU.
 
-Run in the build container only (needs /root/reference):
+Needs a checkout of the original project (kawshik8/GAN-Image-Captioning):
 
-    python oracle/make_golden.py
+    python oracle/make_golden.py <checkout>/src
 
-It imports ``/root/reference/src/{generator,discriminator,utils}.py`` as they are, loads the
+It imports ``<checkout>/src/{generator,discriminator,utils}.py`` as they are, loads the
 seeded synthetic weights from ``oracle.ref_port.make_inputs`` into the reference's own
 ``Decoder`` / ``Encoder`` / ``Discriminator`` modules via ``load_state_dict``, injects the
 caller-supplied uniforms (by overriding ``Decoder.add_gumbel`` on the instance, keeping its
 ``eps`` arithmetic) and dropout keep-masks (by replacing the ``nn.Dropout`` instance), runs
 one adversarial step exactly as ``src/training.py:144-169,194-199`` does except for the Q1
 ordering fix (both grads on pre-update weights; SURVEY.md §0.1), and stores the results.
-Nothing under /root/reference is copied; only numeric outputs are committed.
+Nothing of the original project is copied; only numeric outputs are committed.
 """
 from __future__ import annotations
 
@@ -26,7 +26,6 @@ import torch.nn.functional as F
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-REF = "/root/reference/src"
 
 from oracle import ref_port as rp  # noqa: E402
 
@@ -44,16 +43,16 @@ class SuppliedDropout(nn.Module):
         return x * self.keep / (1.0 - self.p)
 
 
-def load_reference():
-    sys.path.insert(0, REF)
+def load_reference(src):
+    sys.path.insert(0, src)
     import generator as ref_gen       # noqa
     import discriminator as ref_disc  # noqa
     import utils as ref_utils         # noqa
     return ref_gen, ref_disc, ref_utils
 
 
-def run_reference(cfg, temperature, loss_type, train=True):
-    ref_gen, ref_disc, ref_utils = load_reference()
+def run_reference(src, cfg, temperature, loss_type, train=True):
+    ref_gen, ref_disc, ref_utils = load_reference(src)
     inp = rp.make_inputs(cfg)
     a = inp["args"]
     B, L = inp["captions"].shape
@@ -176,11 +175,13 @@ CASES = [
 
 
 def main():
+    if len(sys.argv) != 2:
+        sys.exit("usage: python oracle/make_golden.py <checkout of the original project>/src")
     torch.manual_seed(1008)
     torch.set_num_threads(4)
     os.makedirs(os.path.join(ROOT, "tests", "golden"), exist_ok=True)
     for name, cfg, T, loss, train, full in CASES:
-        inp, res = run_reference(rp.CONFIGS[cfg], T, loss, train)
+        inp, res = run_reference(sys.argv[1], rp.CONFIGS[cfg], T, loss, train)
         blob = pack(res, full)
         blob["meta_temperature"] = np.float64(T)
         path = os.path.join(ROOT, "tests", "golden", name + ".npz")

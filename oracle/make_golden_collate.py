@@ -1,6 +1,6 @@
 """Generate tests/golden/collate.npz by running the reference's UNMODIFIED ``collate_fn`` (src/tasks.py:138-158) on CPU.
 
-Run in the build container only (needs /root/reference):   python oracle/make_golden_collate.py
+Needs a checkout of the original project:   python oracle/make_golden_collate.py <checkout>/src
 
 ``tasks.py`` imports ``h5py`` and ``scipy.misc.imread/imresize`` (absent / removed, SURVEY.md Q9) without using them in
 ``collate_fn``; the three names are stubbed in ``sys.modules`` so that the module imports.  Only numeric outputs are
@@ -14,10 +14,9 @@ import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference/src"
 
 
-def load_collate():
+def load_collate(src):
     for name in ("h5py", "torchtext"):
         sys.modules.setdefault(name, types.ModuleType(name))
     import scipy
@@ -25,7 +24,7 @@ def load_collate():
     misc.imread = misc.imresize = lambda *a, **k: None
     sys.modules["scipy.misc"] = misc
     scipy.misc = misc
-    sys.path.insert(0, REF)
+    sys.path.insert(0, src)
     import tasks
     return tasks.collate_fn
 
@@ -42,7 +41,9 @@ def cases():
 
 
 def main():
-    collate = load_collate()
+    if len(sys.argv) != 2:
+        sys.exit("usage: python oracle/make_golden_collate.py <checkout of the original project>/src")
+    collate = load_collate(sys.argv[1])
     blob = {}
     for name, lists in cases().items():
         batch = [(torch.zeros(3, 4, 4), [int(t) for t in toks]) for toks in lists]

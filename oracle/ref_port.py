@@ -7,8 +7,8 @@ package (``gan-image-captioning_b200/``) never does and fails loudly without its
 library.
 
 Parity pinning: the reference ships no tests or golden vectors (SURVEY.md §4), so this
-oracle is pinned by *executing the reference's own modules* in the build container:
-``oracle/make_golden.py`` imports ``/root/reference/src/{generator,discriminator,utils}.py``
+oracle is pinned by *executing the reference's own modules*:
+``oracle/make_golden.py`` imports ``<checkout>/src/{generator,discriminator,utils}.py``
 unmodified, runs them on the seeded inputs produced by :func:`make_inputs`, and commits
 the outputs under ``tests/golden/``.  ``tests/test_oracle_golden.py`` checks this
 restatement against those fixtures.  Extensions the reference does not contain

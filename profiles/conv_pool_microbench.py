@@ -1,5 +1,6 @@
 import os, sys, torch
-sys.path.insert(0, '/root/repo'); sys.path.insert(0,'/root/repo/tests')
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, 'tests'))
 import gic_b200
 from gic_b200 import _lib
 from gic_b200.discriminator import disc_fwd_raw

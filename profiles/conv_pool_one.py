@@ -1,5 +1,5 @@
 import os, sys, torch
-sys.path.insert(0, '/root/repo')
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import gic_b200
 from gic_b200 import _lib
 from gic_b200.discriminator import disc_fwd_raw
