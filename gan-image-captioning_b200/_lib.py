@@ -166,6 +166,12 @@ def _declare(L):
     L.gic_ctx_clear_option.restype = None
     L.gic_ctx_clear_option.argtypes = [C.c_char_p]
     L.gic_ctx_get_option.argtypes = [C.c_char_p, I]
+    L.gic_vocab_topk_workspace_floats.restype = Z
+    L.gic_vocab_topk_workspace_floats.argtypes = [I] * 3
+    L.gic_vocab_topk.argtypes = [I, P, P, P, I, I, I, I, P, P, P, P, P]
+    L.gic_decode_beam_workspace_floats.restype = Z
+    L.gic_decode_beam_workspace_floats.argtypes = [I] * 7
+    L.gic_decode_beam.argtypes = [I, P, P, P, P, P, P, P, P, I, I, I, I, I, I, I, C.c_int64, F, P, P, P, P, P, P]
     for name in header_symbols():      # every declared entry point must be exported
         getattr(L, name)
 

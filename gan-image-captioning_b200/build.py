@@ -12,7 +12,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libgic_b200.so")
 STAMP = LIB + ".srchash"
-SOURCES = ["gemm_f32.cu", "gemm_dispatch.cu", "gemm_tcgen05.cu", "gemm_persistent.cu", "gemm_pair_tcgen05.cu", "attn.cu", "lstm_tcgen05.cu", "bptt_tcgen05.cu", "vocab_sample_tcgen05.cu", "dz_fused_tcgen05.cu", "decode.cu", "disc.cu", "loss_optim.cu", "allreduce.cu", "capi.cu"]
+SOURCES = ["gemm_f32.cu", "gemm_dispatch.cu", "gemm_tcgen05.cu", "gemm_persistent.cu", "gemm_pair_tcgen05.cu", "attn.cu", "lstm_tcgen05.cu", "bptt_tcgen05.cu", "vocab_sample_tcgen05.cu", "dz_fused_tcgen05.cu", "beam_tcgen05.cu", "decode.cu", "disc.cu", "loss_optim.cu", "allreduce.cu", "capi.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-shared"]
 

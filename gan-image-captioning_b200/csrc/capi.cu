@@ -52,6 +52,15 @@ int decode_step_tc(const float* hs_t1, const float* W_out, const float* b_out, c
                    float* h_out, float* acts, float* htop, float* scratch, cudaStream_t stream, bool* handled);
 int lstm_step_tc(const float*, int, const float*, const float*, const float*, const float*, const float*, const float*,
                  int, int, float*, float*, float*, float*, int, int, cudaStream_t, bool*);
+// beam_tcgen05.cu
+size_t vocab_topk_ws_floats(int M, int V, int K);
+int vocab_topk(int mode, const float* h, const float* W_out, const float* b_out, int M, int V, int H, int K, float* logp,
+               int64_t* tokens, float* lse, float* ws, cudaStream_t s);
+size_t decode_beam_ws_floats(int B, int K, int L, int V, int E, int H, int layers);
+int decode_beam(int mode, const float* features, const float* W_emb, const float* const* W_ih, const float* const* W_hh,
+                const float* const* b_ih, const float* const* b_hh, const float* W_out, const float* b_out, int B, int K,
+                int L, int V, int E, int H, int layers, int64_t eos, float length_penalty, int64_t* ids, float* scores,
+                int32_t* lengths, int32_t* trace, float* ws, cudaStream_t s);
 // disc.cu
 size_t disc_saved_floats(int, int, int, int, int);
 size_t disc_fwd_workspace_floats(int);
@@ -854,6 +863,38 @@ int gic_pg_loss_fwd_bwd(const float* logits, const int64_t* ids, const float* Q,
                         float* loss, float* dlogits, float* logp, gic_stream_t stream) {
   GIC_TRY(require_device());
   return pg_loss(logits, ids, Q, baseline_mode, B, L, V, loss, dlogits, logp, S(stream));
+}
+
+size_t gic_vocab_topk_workspace_floats(int M, int V, int K) { return vocab_topk_ws_floats(M, V, K); }
+int gic_vocab_topk(int mode, const float* h, const float* W_out, const float* b_out, int M, int V, int H, int K,
+                   float* logp, int64_t* tokens, float* lse, float* workspace, gic_stream_t stream) {
+  GIC_TRY(require_device());
+  GIC_REQUIRE(M >= 0 && V >= 1 && H >= 1 && K >= 1 && K <= 16 && K <= V, GIC_ERR_SHAPE,
+              "vocab_topk: bad shape M=%d V=%d H=%d K=%d", M, V, H, K);
+  if (M == 0) return GIC_OK;
+  GIC_REQUIRE(h && W_out && b_out && logp && tokens && workspace, GIC_ERR_NULL, "vocab_topk: NULL pointer");
+  return vocab_topk(mode, h, W_out, b_out, M, V, H, K, logp, tokens, lse, workspace, S(stream));
+}
+size_t gic_decode_beam_workspace_floats(int B, int K, int L, int V, int E, int H, int layers) {
+  return decode_beam_ws_floats(B, K, L, V, E, H, layers);
+}
+int gic_decode_beam(int mode, const float* features, const float* W_emb, const float* const* W_ih,
+                    const float* const* W_hh, const float* const* b_ih, const float* const* b_hh,
+                    const float* W_out, const float* b_out, int B, int K, int L, int V, int E, int H, int layers,
+                    int64_t eos_id, float length_penalty, int64_t* ids, float* scores, int32_t* lengths, int32_t* trace,
+                    float* workspace, gic_stream_t stream) {
+  GIC_TRY(require_device());
+  GIC_REQUIRE(B >= 0 && K >= 1 && K <= 16 && K <= V && L >= 1 && V >= 1 && E >= 1 && H >= 1 && layers >= 1 && layers <= 8 &&
+                  eos_id >= 0 && eos_id < V,
+              GIC_ERR_SHAPE, "decode_beam: bad shape B=%d K=%d L=%d V=%d E=%d H=%d layers=%d eos_id=%lld", B, K, L, V, E, H,
+              layers, (long long)eos_id);
+  if (B == 0) return GIC_OK;
+  GIC_REQUIRE(features && W_emb && W_ih && W_hh && b_ih && b_hh && W_out && b_out && ids && scores && lengths && workspace,
+              GIC_ERR_NULL, "decode_beam: NULL pointer");
+  for (int l = 0; l < layers; ++l)
+    GIC_REQUIRE(W_ih[l] && W_hh[l] && b_ih[l] && b_hh[l], GIC_ERR_NULL, "decode_beam: NULL weight of layer %d", l);
+  return decode_beam(mode, features, W_emb, W_ih, W_hh, b_ih, b_hh, W_out, b_out, B, K, L, V, E, H, layers, eos_id,
+                     length_penalty, ids, scores, lengths, trace, workspace, S(stream));
 }
 
 size_t gic_disc_saved_floats(int N, int L, int De, int R, int F) { return disc_saved_floats(N, L, De, R, F); }

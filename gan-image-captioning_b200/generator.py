@@ -237,6 +237,32 @@ class _DecodeSampleAttn(torch.autograd.Function):
                 db_ih, db_hh)
 
 
+def decode_beam(dec, features, beam_size, max_caption_len, length_penalty=0.0, eos_id=2, mode=None, trace=None):
+    """gic_decode_beam over the decoder's weights -> (ids[B,K,L] int64, scores[B,K], lengths[B,K] int32).  trace[L,B,K,2]
+    (int32, optional) receives the (parent slot, token) chosen at every step."""
+    _lib.require_cuda()
+    lib = _lib.lib()
+    mode = gic_b200.get_gemm_mode() if mode is None else mode
+    features = _f32c(features)
+    B, E = features.shape
+    K, L = int(beam_size), int(max_caption_len)
+    V, H = dec.linear.weight.shape
+    layers = dec.lstm.num_layers
+    dev = features.device
+    lp = [_f32c(w) for w in dec.lstm_params()]
+    W_ih, W_hh, b_ih, b_hh = lp[0::4], lp[1::4], lp[2::4], lp[3::4]
+    W_emb, W_out, b_out = _f32c(dec.embed.weight), _f32c(dec.linear.weight), _f32c(dec.linear.bias)
+    ids = torch.empty(B, K, L, dtype=torch.int64, device=dev)
+    scores = torch.empty(B, K, device=dev)
+    lengths = torch.empty(B, K, dtype=torch.int32, device=dev)
+    ws = torch.empty(lib.gic_decode_beam_workspace_floats(B, K, L, V, E, H, layers), device=dev)
+    _lib.check(lib.gic_decode_beam(mode, _lib.ptr(features), _lib.ptr(W_emb), _lib.ptr_array(W_ih), _lib.ptr_array(W_hh),
+                                   _lib.ptr_array(b_ih), _lib.ptr_array(b_hh), _lib.ptr(W_out), _lib.ptr(b_out), B, K, L, V,
+                                   E, H, layers, int(eos_id), float(length_penalty), _lib.ptr(ids), _lib.ptr(scores),
+                                   _lib.ptr(lengths), _lib.ptr(trace), _lib.ptr(ws), _lib.stream()), "gic_decode_beam")
+    return ids, scores, lengths
+
+
 class Decoder(nn.Module):
     """LSTM caption decoder (src/generator.py:27-96).  ``embed``/``lstm``/``linear`` are parameter
     containers with the reference's state_dict keys; ``sample`` runs on the B200 kernels."""
@@ -291,6 +317,16 @@ class Decoder(nn.Module):
         return _DecodeSample.apply(features, u, float(self.temperature), bool(pretrain), L, forced_ids,
                                    gic_b200.get_gemm_mode(), self.lstm.num_layers, self.embed.weight,
                                    self.linear.weight, self.linear.bias, *self.lstm_params())
+
+    @torch.no_grad()
+    def beam_search(self, features, beam_size=3, max_caption_len=34, length_penalty=0.0, eos_id=2):
+        """The most likely captions of features[B,E] (the step-0 input, as in sample) by beam search (EXTENSION; the
+        reference has none, oracle/ref_beam.py defines it) -> (ids[B,K,L], scores[B,K], lengths[B,K]), the K beams of each
+        image best first by score / length ** length_penalty.  ids hold PAD (0) after <E> (eos_id); scores are sums of
+        log-probabilities; lengths count tokens up to and including <E>.  beam_size = 1 is greedy decoding."""
+        if self.attention:
+            raise NotImplementedError("beam search is implemented for the plain LSTM decoder, not the attention cell")
+        return decode_beam(self, features, beam_size, max_caption_len, length_penalty, eos_id)
 
     def add_gumbel(self, o_t, eps=1e-10, gpu=0):
         """Kept for interface parity (src/generator.py:84-96); the hot path fuses this into the sampler."""

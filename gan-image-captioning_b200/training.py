@@ -20,7 +20,7 @@ import torch.nn as nn
 import gic_b200
 from . import _lib, parallel
 from .discriminator import Discriminator, disc_fwd_raw
-from .generator import Generator, bn_running_update
+from .generator import Generator, bn_running_update, encoder_eval
 from .utils import get_fixed_temperature, get_losses
 
 
@@ -777,6 +777,30 @@ class GANInstructor:
         if st["g_has_grad"]:
             self._flat_g.step += 1
         return st["out"]
+
+    # ---- EXTENSION: caption generation by beam search (the reference has none) -------------------------------------
+    @_in_ctx
+    @torch.no_grad()
+    def generate(self, pooled=None, batch_size=None, beam_size=3, max_caption_len=34, length_penalty=0.0):
+        """Captions of a trained generator -> (ids[B,K,L], scores[B,K], lengths[B,K]) (Decoder.beam_search).  Conditional
+        mode: the pooled CNN features [B, feature_dim] go through the encoder projection in eval mode (running statistics,
+        as gen.eval() would); unconditional mode: every caption starts from embed.weight[1] (<S>), batch_size of them.
+        Inference only: parameters, gradients, optimizer state, step counters, temperature and the library's random stream
+        are left as they were."""
+        _lib.require_cuda()
+        dev = self.device
+        dec = self.gen.decoder
+        if self.cgan:
+            if pooled is None:
+                raise ValueError("conditional generation needs the pooled image features")
+            feats = encoder_eval(self.gen.encoder, pooled.to(dev).float(), gic_b200.get_gemm_mode())
+        else:
+            if batch_size is None:
+                if pooled is None:
+                    raise ValueError("unconditional generation needs batch_size")
+                batch_size = pooled.shape[0]
+            feats = dec.embed.weight[1].expand(int(batch_size), dec.embed.weight.shape[1]).contiguous()
+        return dec.beam_search(feats, beam_size=beam_size, max_caption_len=max_caption_len, length_penalty=length_penalty)
 
     # ---- generator pre-training step (src/training.py:53-95; SURVEY.md 8f rank 1) -------------------------------
     @_in_ctx

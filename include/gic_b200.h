@@ -249,6 +249,30 @@ int gic_rollout_rewards(const float* roll_logits, const float* main_logits, int 
 int gic_pg_loss_fwd_bwd(const float* logits, const int64_t* ids, const float* Q, int baseline_mode, int B, int L, int V,
                         float* loss, float* dlogits, float* logp, gic_stream_t stream);
 
+/* ---- caption generation by beam search (EXTENSION, parity unpinned by reference: the reference has no beam search;
+ * oracle/ref_beam.py beam_search defines it).
+ * gic_vocab_topk: per row of h[M,H]: lse[m] = logsumexp(h W_out^T + b_out), the K largest log-probabilities logp[M,K]
+ *   (descending, ties -> lower token) and their tokens[M,K]; nothing of size V is written in the tensor-core modes.
+ *   workspace: gic_vocab_topk_workspace_floats(M, V, K); lse may be NULL.  1 <= K <= 16, K <= V.
+ * gic_decode_beam: Decoder.sample's LSTM (any number of layers; step 0's input is features[B,E], h = c = 0) with K beams per
+ *   image.  Every step each live beam k offers (k, w) at score_k + log_softmax(h W_out^T + b_out)[w]; a beam that has emitted
+ *   eos_id is frozen and offers only (k, PAD = 0) at its own score.  The image keeps its K best candidates (higher score, then
+ *   lower parent beam, then lower token); beam 0 starts at 0, beams 1..K-1 at -inf.  Always L steps, no host sync (the call
+ *   can be captured into a CUDA graph).  Output, per image, the K beams ordered by score / length^length_penalty (ties ->
+ *   lower beam slot): ids[B,K,L] (PAD after EOS), scores[B,K] (raw sums of log-probabilities), lengths[B,K] (tokens up to and
+ *   including EOS, L when none).  trace[L,B,K,2] (may be NULL): for step t and slot k the parent slot and token chosen.
+ *   K = 1 is greedy decoding.  GIC_ERR_SHAPE: K < 1, K > 16, K > V, L < 1, eos_id outside [0, V), layers outside 1..8. */
+size_t gic_vocab_topk_workspace_floats(int M, int V, int K);
+int gic_vocab_topk(int mode, const float* h, const float* W_out, const float* b_out, int M, int V, int H, int K,
+                   float* logp, int64_t* tokens, float* lse, float* workspace, gic_stream_t stream);
+size_t gic_decode_beam_workspace_floats(int B, int K, int L, int V, int E, int H, int layers);
+int gic_decode_beam(int mode, const float* features, const float* W_emb, const float* const* W_ih,
+                    const float* const* W_hh, const float* const* b_ih, const float* const* b_hh,
+                    const float* W_out, const float* b_out, int B, int K, int L, int V, int E, int H, int layers,
+                    int64_t eos_id, float length_penalty, int64_t* ids /*[B,K,L]*/, float* scores /*[B,K]*/,
+                    int32_t* lengths /*[B,K]*/, int32_t* trace /*[L,B,K,2] (parent, token) or NULL*/,
+                    float* workspace, gic_stream_t stream);
+
 /* ---- B1 (EXTENSION, parity unpinned by reference): additive attention over the CNN feature grid in the decode step.
  * The reference feeds one pooled vector at step 0 (src/generator.py:19-25,58) and has no attention.  Definition:
  *   once per image: Ak = grid W_k^T [B,P,Da], Av = grid W_v^T [B,P,E];  every step: q = h_{t-1} W_q^T,
