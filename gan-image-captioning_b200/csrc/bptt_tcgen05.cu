@@ -5,27 +5,28 @@
 // It replaces, per step, a stream-K GEMM whose 8 partial tiles met through red.global.add in L2 (~12 us for 0.5 GFLOP)
 // plus the separate cell kernel (~4 us): 19 serial pairs on the generator's critical path at c2.
 //
-// Split-K over a thread-block cluster: the CL CTAs of a cluster (4, or 8) share one 128-row x 8 CL-column tile of dh_rec
-// and each contracts 1 / CL of K = 4H (TMA ring -> tcgen05.mma kind::tf32 -> TMEM).  The partial tiles meet over
-// distributed shared memory: every CTA stages its partial grouped by destination rank, the cluster synchronises, and CTA r
-// adds the CL partials of columns 8r .. 8r+7 in rank order (deterministic) and applies the cell backward to those 8 hidden
-// units -- the cell update is elementwise in (row, unit), so no further exchange is needed.
+// Split-K over a thread-block cluster: the 4 CTAs of a cluster share one 128-row x 32-column tile of dh_rec and each
+// contracts 1 / 4 of K = 4H (TMA ring -> tcgen05.mma kind::tf32 -> TMEM).  The partial tiles meet over distributed
+// shared memory: every CTA stages its partial grouped by destination rank, the cluster synchronises, and CTA r adds the
+// 4 partials of columns 8r .. 8r+7 in rank order (deterministic) and applies the cell backward to those 8 hidden units
+// -- the cell update is elementwise in (row, unit), so no further exchange is needed.
 // Measured (ncu, c2): 13.4 us per step against 12.0 + 4.3 us for the stream-K GEMM + cell kernel.
+// Clusters of 8 (64 columns) would need 16 co-resident clusters at c2, and a B200 fits 15 (cudaOccupancyMaxActiveClusters):
+// the grid ran in two waves, 2.585 ms per training step against 2.503 with clusters of 4.
 #include "tcgen05_common.cuh"
 
 namespace gic {
 namespace tc {
 
-// CL = cluster size = K splits = column groups of the tile; tile width BN = 8 * CL hidden units (every rank finishes 8)
+// BP_CL = cluster size = K splits = column groups of the tile; tile width BP_BN = 8 * BP_CL hidden units (every rank
+// finishes 8)
+constexpr int BP_CL = 4;
+constexpr int BP_BN = 8 * BP_CL;
 constexpr int BP_A_BYTES = BM * BK * 4;       // 16 KB: 128 rows x 32 fp32 of dG
+constexpr int BP_B_BYTES = BK * BP_BN * 4;    // 32 k-rows x BP_BN columns of W_hh (MN-major, 32-column slabs)
 constexpr int BP_STAGES = 8;
-template <int CL>
-struct BpCfg {
-  static constexpr int BN = 8 * CL;
-  static constexpr int B_BYTES = BK * BN * 4;   // 32 k-rows x BN columns of W_hh (MN-major, 32-column slabs)
-  static constexpr int STAGE = BP_A_BYTES + B_BYTES;
-  static constexpr int SMEM = BP_STAGES * STAGE + 1024 + 256;
-};
+constexpr int BP_STAGE = BP_A_BYTES + BP_B_BYTES;
+constexpr int BP_SMEM = BP_STAGES * BP_STAGE + 1024 + 256;
 
 __device__ __forceinline__ void bp_cluster_sync() {
   asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
@@ -54,17 +55,15 @@ struct BpttArgs {
   float* dG_out;                  // [B, 4H] gate pre-activation gradients of step t - 1
 };
 
-template <int BP_CL>
 __global__ void __launch_bounds__(NTHREADS, 1)
 bptt_step_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, BpttArgs a) {
-  constexpr int BP_BN = BpCfg<BP_CL>::BN, BP_STAGE = BpCfg<BP_CL>::STAGE;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
   uint64_t* full = reinterpret_cast<uint64_t*>(smem + BP_STAGES * BP_STAGE);
   uint64_t* empty = full + BP_STAGES;
   uint64_t* tmem_full = empty + BP_STAGES;
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tmem_full + 1);
-  uint8_t* part = smem;                       // [dest rank 8][chunk 2][row 128][16 B]: aliases the ring after tmem_full
+  uint8_t* part = smem;                       // [dest rank 4][chunk 2][row 128][16 B]: aliases the ring after tmem_full
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const uint32_t ks = bp_cluster_rank();      // K split of this CTA = the column group it finishes
@@ -439,13 +438,7 @@ int bptt_step_tc(const float* dG_t, const float* W_hh, const float* acts_prev, c
   using namespace tc;
   *handled = false;
   if (option("GIC_BPTT_FUSED", 1) == 0) return GIC_OK;
-  // Cluster size: 8 CTAs x 64 columns would need 16 co-resident clusters of 8 at c2, and a B200 fits 15
-  // (cudaOccupancyMaxActiveClusters; two waves: 2.585 ms per step against 2.503 with clusters of 4), so 4 x 32 columns
-  // is the default.
-  int CL = 4;
-  if (option("GIC_BPTT_CL", 0) == 8) CL = 8;
-  const int BP_BN = 8 * CL;
-  if (B <= 0 || t < 1 || (H % BP_BN) || ((4 * H) % (BK * CL))) return GIC_OK;
+  if (B <= 0 || t < 1 || (H % BP_BN) || ((4 * H) % (BK * BP_CL))) return GIC_OK;
   const void* ptrs[] = {dG_t, W_hh, acts_prev, c_prev, c_cur, dh_top, dc_rec, dG_out};
   for (const void* p : ptrs)
     if (!aligned16(p)) return GIC_OK;
@@ -455,30 +448,22 @@ int bptt_step_tc(const float* dG_t, const float* W_hh, const float* acts_prev, c
   if (!make_map(&tb, W_hh, 4 * H, H, H, 32, BK, rn, true)) return GIC_OK;
   static bool attr = false;
   if (!attr) {
-    cudaFuncSetAttribute(bptt_step_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, BpCfg<8>::SMEM);
-    cudaFuncSetAttribute(bptt_step_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, BpCfg<4>::SMEM);
+    cudaFuncSetAttribute(bptt_step_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, BP_SMEM);
     attr = true;
   }
   BpttArgs a;
   a.B = B; a.H = H; a.L = L; a.t = t; a.acts = acts_prev; a.c_prev = c_prev; a.c_cur = c_cur; a.dh_top = dh_top;
   a.dc_rec = dc_rec; a.dG_out = dG_out;
   cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(cdiv(B, BM) * (H / BP_BN) * CL, 1, 1);
+  cfg.gridDim = dim3(cdiv(B, BM) * (H / BP_BN) * BP_CL, 1, 1);
   cfg.blockDim = dim3(NTHREADS, 1, 1);
-  cfg.dynamicSmemBytes = (CL == 8) ? BpCfg<8>::SMEM : BpCfg<4>::SMEM;
+  cfg.dynamicSmemBytes = BP_SMEM;
   cfg.stream = stream;
   cudaLaunchAttribute at[1];
   at[0].id = cudaLaunchAttributeClusterDimension;
-  at[0].val.clusterDim.x = CL; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
+  at[0].val.clusterDim.x = BP_CL; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
   cfg.attrs = at; cfg.numAttrs = 1;
-  static int shown = 0;
-  if (!shown && option("GIC_BPTT_DEBUG", 0)) {
-    shown = 1;
-    int nc = -1;
-    if (CL == 8) cudaOccupancyMaxActiveClusters(&nc, bptt_step_kernel<8>, &cfg); else cudaOccupancyMaxActiveClusters(&nc, bptt_step_kernel<4>, &cfg);
-    fprintf(stderr, "bptt_step_kernel<%d>: grid %d CTAs, max co-resident clusters %d\n", CL, cfg.gridDim.x, nc);
-  }
-  cudaError_t e = (CL == 8) ? cudaLaunchKernelEx(&cfg, bptt_step_kernel<8>, ta, tb, a) : cudaLaunchKernelEx(&cfg, bptt_step_kernel<4>, ta, tb, a);
+  cudaError_t e = cudaLaunchKernelEx(&cfg, bptt_step_kernel, ta, tb, a);
   if (e != cudaSuccess) { set_error("bptt_step_kernel launch: %s", cudaGetErrorString(e)); return GIC_ERR_CUDA; }
   int rc = check_launch("bptt_step_kernel");
   if (rc == GIC_OK) *handled = true;

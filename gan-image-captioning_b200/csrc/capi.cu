@@ -27,10 +27,7 @@ int bn_bwd(const float*, const float*, int, int, const float*, const float*, con
            cudaStream_t);
 int lstm_cell_fwd(const float*, const float*, int, int, float*, float*, float*, float*, int, int, cudaStream_t);
 int lstm_cell_bwd(const float*, const float*, const float*, const float*, long long, const float*, float*, int, int,
-                  float*, cudaStream_t, void* dgates_bf = nullptr);
-// gemm_dispatch.cu
-int gemm_dz(int, int, int, int, const float*, int, const float*, int, const float*, const float*, float, float*, int,
-            cudaStream_t, bool*);
+                  float*, cudaStream_t);
 // attn.cu
 int attn_fwd(const float*, const float*, const float*, const float*, int, int, int, int, float*, float*, cudaStream_t);
 int attn_bwd_step(const float*, const float*, const float*, const float*, const float*, const float*, int, int, int, int,
@@ -277,7 +274,7 @@ static int decode_fwd(int mode, const float* features, const float* W_emb, const
 //   dlogits[B*L*V] | dHtop[B*L*H] | dG[layers][L][B][4H] | dh_rec[layers][B][H] | dc_rec[layers][B][H]
 //   | dxin[B][H] | dX[L][B][E] | dot[B*L] | bf16 copies for GIC_GEMM_BF16: dz[B*L][Vp], htop[B*L][H], W_out[V][H]
 struct DecodeBwdWs {
-  size_t dlogits, dhtop, dG, dhrec, dcrec, dxin, dX, dot, dz_bf, htop_bf, wout_bf, dG_bf, whh_bf, wih_bf, xs_bf, hs_bf, total;
+  size_t dlogits, dhtop, dG, dhrec, dcrec, dxin, dX, dot, dz_bf, htop_bf, wout_bf, total;
   int Vp;
   DecodeBwdWs(int B, int L, int V, int E, int H, int layers) {
     const size_t BH = (size_t)B * H;
@@ -293,14 +290,7 @@ struct DecodeBwdWs {
     dz_bf = dot + a4((size_t)B * L);
     htop_bf = dz_bf + a4((size_t)B * L * Vp / 2);
     wout_bf = htop_bf + a4(((size_t)B * L * H + 1) / 2);
-    // bf16 operands of the recurrent backward (GIC_GEMM_BF16, single layer): dG[L*B,4H], W_hh[4H,H], W_ih[4H,E], xs[L*B,E],
-    // hs[(L+1)*B,H]
-    dG_bf = wout_bf + a4(((size_t)V * H + 1) / 2);
-    whh_bf = dG_bf + a4((size_t)L * BH * 4 / 2);
-    wih_bf = whh_bf + a4((size_t)4 * H * H / 2);
-    xs_bf = wih_bf + a4(((size_t)4 * H * E + 1) / 2);
-    hs_bf = xs_bf + a4(((size_t)L * B * E + 1) / 2);
-    total = hs_bf + a4(((size_t)(L + 1) * BH + 1) / 2);
+    total = wout_bf + a4(((size_t)V * H + 1) / 2);
   }
 };
 
@@ -389,10 +379,7 @@ static int decode_bwd(int mode, const float* dout, const float* demb, const floa
         GIC_TRY(gemm_bf16(false, false, BL, H, V, 1.f, dz_bf, w.Vp, wout_bf, H, 0.f, ws + w.dhtop, H, nullptr, s));
         vocab_done = true;
       }
-      bool fused = false;
-      if (!vocab_done)
-      GIC_TRY(gemm_dz(mode, BL, V, De, demb, De, W_e, V, out, ws + w.dot, T, ws + w.dlogits, V, s, &fused));
-      if (!fused && !vocab_done) {
+      if (!vocab_done) {
         GIC_TRY(gemm(mode, false, false, BL, V, De, 1.f, demb, De, W_e, V, 0.f, ws + w.dlogits, V, nullptr, s));
         GIC_TRY(softmax_bwd_dot(out, ws + w.dlogits, ws + w.dot, T, BL, V, ws + w.dlogits, s));
       }
@@ -409,23 +396,9 @@ static int decode_bwd(int mode, const float* dout, const float* demb, const floa
     GIC_TRY(record_vocab_grads_event(s));
     GIC_TRY(gemm(mode, false, false, BL, H, V, 1.f, dlogits, V, W_out, H, 0.f, ws + w.dhtop, H, nullptr, s));
   }
-  // GIC_GEMM_BF16, single layer, no attention: the recurrent backward's contractions (dh_rec = dG W_hh per step, dW_ih,
-  // dW_hh, dX over all steps) read bf16 operands -- they are bound by per-SM operand ingest, so half the bytes is close
-  // to half the time.  dG is written in both precisions by the cell kernel (fp32 for the bias gradients).
-  // Measured at c2: the GEMM class gets ~50 us shorter, the four conversions cost ~25 us and the step time does not move
-  // (the BPTT GEMMs are launch / stream-K-epilogue bound, not ingest bound) -> opt-in only (GIC_REC_BF16=1).
-  const int rec_env = option("GIC_REC_BF16", 0);
-  const bool rec_bf = rec_env && (mode == GEMM_BF16) && layers == 1 && !at && (H % 8 == 0) && (E % 8 == 0);
-  void* dG_bf = rec_bf ? (void*)(ws + w.dG_bf) : nullptr;
-  if (rec_bf) {
-    GIC_TRY(f32_to_bf16(W_hh[0], 4 * H, H, H, ws + w.whh_bf, H, s));
-    GIC_TRY(f32_to_bf16(W_ih[0], 4 * H, E, E, ws + w.wih_bf, E, s));
-    GIC_TRY(f32_to_bf16(saved + sv.xs, L * B, E, E, ws + w.xs_bf, E, s));
-    GIC_TRY(f32_to_bf16(saved + sv.hs(0), L * B, H, H, ws + w.hs_bf, H, s));
-  }
   // 3. BPTT through (h, c)
   cudaMemsetAsync(ws + w.dhrec, 0, (size_t)2 * layers * a4(BH) * sizeof(float), s);   // dh_rec and dc_rec
-  const bool bptt_fusable = (mode == GEMM_TF32 || mode == GEMM_BF16) && layers == 1 && !at && !rec_bf;
+  const bool bptt_fusable = (mode == GEMM_TF32 || mode == GEMM_BF16) && layers == 1 && !at;
   bool bptt_fused_prev = false;
   bool bptt_done = false;
   if (bptt_fusable && L >= 2) {
@@ -435,7 +408,7 @@ static int decode_bwd(int mode, const float* dout, const float* demb, const floa
     const int t = L - 1;
     GIC_TRY(lstm_cell_bwd(saved + sv.acts(0) + (size_t)t * BH * 4, saved + sv.cs(0) + (size_t)t * BH,
                           saved + sv.cs(0) + (size_t)(t + 1) * BH, ws + w.dhtop + (size_t)t * H, (long long)L * H, ws + w.dhrec,
-                          ws + w.dcrec, B, H, ws + w.dG + (size_t)t * BH * 4, s, nullptr));
+                          ws + w.dcrec, B, H, ws + w.dG + (size_t)t * BH * 4, s));
     GIC_TRY(bptt_persistent_tc(ws + w.dG, W_hh[0], saved + sv.acts(0), saved + sv.cs(0), ws + w.dhtop, ws + w.dcrec,
                                reinterpret_cast<unsigned int*>(ws + w.dhrec), B, H, L, s, &bptt_done));
     bptt_fused_prev = !bptt_done;      // not handled: the loop below continues from the cell backward already done
@@ -448,24 +421,20 @@ static int decode_bwd(int mode, const float* dout, const float* demb, const floa
       float* dG_lt = ws + w.dG + (size_t)l * dG_stride + (size_t)t * BH * 4;
       float* dhrec = ws + w.dhrec + (size_t)l * a4(BH);
       float* dcrec = ws + w.dcrec + (size_t)l * a4(BH);
-      void* dG_bf_t = rec_bf ? (void*)(reinterpret_cast<unsigned short*>(dG_bf) + (size_t)t * BH * 4) : nullptr;
       if (!bptt_fused_prev)      // else dG of this step (and dc) came out of the fused kernel launched for step t + 1
         GIC_TRY(lstm_cell_bwd(saved + sv.acts(l) + (size_t)t * BH * 4, saved + sv.cs(l) + (size_t)t * BH,
-                              saved + sv.cs(l) + (size_t)(t + 1) * BH, dh_in, stride, dhrec, dcrec, B, H, dG_lt, s, dG_bf_t));
+                              saved + sv.cs(l) + (size_t)(t + 1) * BH, dh_in, stride, dhrec, dcrec, B, H, dG_lt, s));
       bptt_fused_prev = false;
       // recurrent gradient for step t-1: dh_rec = dgates W_hh    ([B,4H] x [4H,H])
       if (t > 0) {
-        if (rec_bf) GIC_TRY(gemm_bf16(false, false, B, H, 4 * H, 1.f, dG_bf_t, 4 * H, ws + w.whh_bf, H, 0.f, dhrec, H, nullptr, s));
-        else {
-          // tensor-core modes, one layer, no attention: contraction (split-K over a cluster, DSMEM reduction) and the cell
-          // backward of step t - 1 in ONE kernel (bptt_tcgen05.cu)
-          if (bptt_fusable)
-            GIC_TRY(bptt_step_tc(dG_lt, W_hh[0], saved + sv.acts(0) + (size_t)(t - 1) * BH * 4, saved + sv.cs(0) + (size_t)(t - 1) * BH,
-                                 saved + sv.cs(0) + (size_t)t * BH, ws + w.dhtop, dcrec, ws + w.dG + (size_t)(t - 1) * BH * 4, B, H, L, t,
-                                 s, &bptt_fused_prev));
-          if (!bptt_fused_prev)
-            GIC_TRY(gemm(mode, false, false, B, H, 4 * H, 1.f, dG_lt, 4 * H, W_hh[l], H, 0.f, dhrec, H, nullptr, s));
-        }
+        // tensor-core modes, one layer, no attention: contraction (split-K over a cluster, DSMEM reduction) and the cell
+        // backward of step t - 1 in ONE kernel (bptt_tcgen05.cu)
+        if (bptt_fusable)
+          GIC_TRY(bptt_step_tc(dG_lt, W_hh[0], saved + sv.acts(0) + (size_t)(t - 1) * BH * 4, saved + sv.cs(0) + (size_t)(t - 1) * BH,
+                               saved + sv.cs(0) + (size_t)t * BH, ws + w.dhtop, dcrec, ws + w.dG + (size_t)(t - 1) * BH * 4, B, H, L, t,
+                               s, &bptt_fused_prev));
+        if (!bptt_fused_prev)
+          GIC_TRY(gemm(mode, false, false, B, H, 4 * H, 1.f, dG_lt, 4 * H, W_hh[l], H, 0.f, dhrec, H, nullptr, s));
       }
       if (at && l == 0) {
         // attention: dx'_t = dG_t W_ih (per step: dq_t feeds the recurrent gradient), then the attention backward
@@ -487,8 +456,7 @@ static int decode_bwd(int mode, const float* dout, const float* demb, const floa
   // They need dG only, and dW_emb is 40 % of the generator's gradient bytes: formed BEFORE the weight-gradient GEMMs, its
   // all-reduce (gic_set_embed_grads_event) runs underneath them instead of in the exposed tail of the step.
   if (!at) {
-    if (rec_bf) GIC_TRY(gemm_bf16(false, false, L * B, E, 4 * H, 1.f, dG_bf, 4 * H, ws + w.wih_bf, E, 0.f, ws + w.dX, E, nullptr, s));
-    else GIC_TRY(gemm(mode, false, false, L * B, E, 4 * H, 1.f, ws + w.dG, 4 * H, W_ih[0], E, 0.f, ws + w.dX, E, nullptr, s));
+    GIC_TRY(gemm(mode, false, false, L * B, E, 4 * H, 1.f, ws + w.dG, 4 * H, W_ih[0], E, 0.f, ws + w.dX, E, nullptr, s));
     if (!accumulate) cudaMemsetAsync(dW_emb, 0, (size_t)V * E * sizeof(float), s);
     GIC_TRY(embed_scatter(ws + w.dX, fed, B, L, E, V, dW_emb, dfeat, s));
     GIC_TRY(record_embed_grads_event(s));
@@ -498,13 +466,8 @@ static int decode_bwd(int mode, const float* dout, const float* demb, const floa
     const float* dG_l = ws + w.dG + (size_t)l * dG_stride;           // [L*B, 4H]
     const int In = (l == 0) ? E : H;
     const float* xin = (l == 0) ? saved + sv.xs : saved + sv.hs(l - 1) + BH;   // inputs of step t, t-major
-    if (rec_bf) {
-      GIC_TRY(gemm_bf16(true, false, 4 * H, In, L * B, 1.f, dG_bf, 4 * H, ws + w.xs_bf, In, beta, dW_ih[l], In, nullptr, s));
-      GIC_TRY(gemm_bf16(true, false, 4 * H, H, L * B, 1.f, dG_bf, 4 * H, ws + w.hs_bf, H, beta, dW_hh[l], H, nullptr, s));
-    } else {
-      GIC_TRY(gemm(mode, true, false, 4 * H, In, L * B, 1.f, dG_l, 4 * H, xin, In, beta, dW_ih[l], In, nullptr, s));
-      GIC_TRY(gemm(mode, true, false, 4 * H, H, L * B, 1.f, dG_l, 4 * H, saved + sv.hs(l), H, beta, dW_hh[l], H, nullptr, s));
-    }
+    GIC_TRY(gemm(mode, true, false, 4 * H, In, L * B, 1.f, dG_l, 4 * H, xin, In, beta, dW_ih[l], In, nullptr, s));
+    GIC_TRY(gemm(mode, true, false, 4 * H, H, L * B, 1.f, dG_l, 4 * H, saved + sv.hs(l), H, beta, dW_hh[l], H, nullptr, s));
     // both biases enter the same pre-activation (src/generator.py:61), so their gradients are the same column sums
     GIC_TRY(colsum_f32(dG_l, L * B, 4 * H, 4 * H, 1.f, accumulate != 0, db_ih[l], s));
     if (!accumulate) cudaMemcpyAsync(db_hh[l], db_ih[l], (size_t)4 * H * sizeof(float), cudaMemcpyDeviceToDevice, s);

@@ -159,8 +159,7 @@ __global__ void lstm_cell_fwd_kernel(const float* __restrict__ gates, const floa
 __global__ void lstm_cell_bwd_kernel(const float* __restrict__ acts, const float* __restrict__ c_prev,
                                      const float* __restrict__ c_cur, const float* __restrict__ dh_in,
                                      long long dh_stride, const float* __restrict__ dh_rec,
-                                     float* __restrict__ dc_rec, int B, int H, float* __restrict__ dgates,
-                                     unsigned short* __restrict__ dgates_bf /*bf16 copy for GIC_GEMM_BF16, or null*/) {
+                                     float* __restrict__ dc_rec, int B, int H, float* __restrict__ dgates) {
   const int idx = blockIdx.x * blockDim.x + threadIdx.x;
   if (idx >= B * H) return;
   const int b = idx / H, j = idx % H;
@@ -174,11 +173,6 @@ __global__ void lstm_cell_bwd_kernel(const float* __restrict__ acts, const float
   const float di = dc * g_ * i_ * (1.f - i_), df = dc * c_prev[idx] * f_ * (1.f - f_);
   const float dgg = dc * i_ * (1.f - g_ * g_), dout = dh * tc * o_ * (1.f - o_);
   dg[j] = di; dg[H + j] = df; dg[2 * H + j] = dgg; dg[3 * H + j] = dout;
-  if (dgates_bf) {
-    auto bf = [](float x) { unsigned int u = __float_as_uint(x); u += 0x7fffu + ((u >> 16) & 1u); return (unsigned short)(u >> 16); };
-    unsigned short* db = dgates_bf + (size_t)b * 4 * H;
-    db[j] = bf(di); db[H + j] = bf(df); db[2 * H + j] = bf(dgg); db[3 * H + j] = bf(dout);
-  }
   dc_rec[idx] = dc * f_;
 }
 
@@ -928,10 +922,9 @@ int lstm_cell_fwd(const float* gates, const float* c_prev, int B, int H, float* 
 }
 int lstm_cell_bwd(const float* acts, const float* c_prev, const float* c_cur, const float* dh_in,
                   long long dh_stride, const float* dh_rec, float* dc_rec, int B, int H, float* dgates,
-                  cudaStream_t s, void* dgates_bf) {
+                  cudaStream_t s) {
   lstm_cell_bwd_kernel<<<cdiv((long long)B * H, 256), 256, 0, s>>>(acts, c_prev, c_cur, dh_in, dh_stride,
-                                                                  dh_rec, dc_rec, B, H, dgates,
-                                                                  reinterpret_cast<unsigned short*>(dgates_bf));
+                                                                  dh_rec, dc_rec, B, H, dgates);
   return check_launch("lstm_cell_bwd_kernel");
 }
 

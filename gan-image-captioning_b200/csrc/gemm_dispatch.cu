@@ -38,22 +38,8 @@ int gemm_tc(int mode, bool transA, bool transB, int M, int N, int K, float alpha
             bool* handled);
 
 int gemm_tc_persistent(bool transA, bool transB, int M, int N, int K, float alpha, const float* A, int lda,
-                       const float* B, int ldb, float beta, float* C, int ldc, const float* bias, int epi,
-                       const float* aux, const float* rowv, float scalar, cudaStream_t stream, bool* handled);
-
-// dz[M,N] = T * p .* (demb[M,K] * W[K,N] - dot[:,None]): the D-embedding input gradient fused with the tempered
-// softmax backward (tensor-core mode; the dense d(probs) never exists).  handled = false -> caller uses the unfused path.
-int gemm_dz(int mode, int M, int N, int K, const float* demb, int lda, const float* W, int ldb, const float* p,
-            const float* dot, float T, float* dz, int ldc, cudaStream_t stream, bool* handled) {
-  *handled = false;
-  if (mode != GEMM_TF32) return GIC_OK;
-  // The register/LSU epilogue cannot keep enough bytes of p in flight (measured 1.16 ms at c2, profiles/README.md);
-  // until the aux tile is TMA-prefetched the unfused pair (GEMM with TMA store + streaming softmax backward) is used.
-  if (option("GIC_FUSED_DZ", 0) != 1) return GIC_OK;
-  ProfScope prof(PROF_GEMM, 2.0 * M * N * K, stream);
-  return gemm_tc_persistent(false, false, M, N, K, 1.f, demb, lda, W, ldb, 0.f, dz, ldc, nullptr, 1, p, dot, T, stream,
-                            handled);
-}
+                       const float* B, int ldb, float beta, float* C, int ldc, const float* bias, cudaStream_t stream,
+                       bool* handled);
 
 int gemm_tc_bf16(bool transA, bool transB, int M, int N, int K, float alpha, const void* A, int lda, const void* B,
                  int ldb, float beta, float* C, int ldc, const float* bias, cudaStream_t stream, bool* handled);
@@ -113,8 +99,7 @@ int gemm(int mode, bool transA, bool transB, int M, int N, int K, float alpha, c
     bool handled = false;
     int rc = GIC_OK;
     if (mode == GEMM_TF32) {
-      rc = gemm_tc_persistent(transA, transB, M, N, K, alpha, A, lda, B, ldb, beta, C, ldc, bias, 0, nullptr, nullptr, 0.f,
-                              stream, &handled);
+      rc = gemm_tc_persistent(transA, transB, M, N, K, alpha, A, lda, B, ldb, beta, C, ldc, bias, stream, &handled);
       if (rc != GIC_OK) return rc;
       if (handled) return GIC_OK;
     }

@@ -6,8 +6,8 @@
 //   * schedule = data-parallel rounds over whole output tiles + a stream-K tail: the tiles that do not fill a
 //     round are cut along K into equal shares per CTA and combined with fp32 reductions (red.global.add) into the
 //     zero-initialised / beta = 1 output
-//   * epilogue: TMEM -> registers -> per-warp smem transpose -> 128-byte coalesced global accesses, with a
-//     pluggable functor: plain store (alpha/beta/bias), reduction, or the fused softmax-backward of the decoder
+//   * epilogue: TMEM -> registers -> per-warp smem staging -> TMA store (plain stores of whole 32 x 32 blocks) or
+//     128-byte coalesced global accesses (alpha/beta/bias stores, stream-K reductions)
 //   * K-major and MN-major operands through the UMMA descriptor "major" bits (no transposes in the backward pass)
 // Warp roles (192 threads): warp 0 = TMA producer, warp 1 = TMEM allocator + MMA issuer, warps 2..5 = epilogue.
 #include "tcgen05_common.cuh"
@@ -15,18 +15,11 @@
 namespace gic {
 namespace tc {
 
-enum : int { EPI_STORE = 0, EPI_DZ = 1 };
-
 struct EpiArgs {
   float alpha, beta;
   float* C;
   int ldc;
   const float* bias;   // [N] or nullptr
-  const float* aux;    // EPI_DZ: p[M, ldc]
-  const float* rowv;   // EPI_DZ: dot[M]
-  float scalar;        // EPI_DZ: temperature
-  const float* scalar_dev;   // EPI_DZ: temperature read at run time when non-null (CUDA-graph replay)
-  int dbg;             // profiling experiments only (GIC_GEMM_DBG): 1 = skip the global stores of the epilogue
   int vec_red;         // C is 16-byte aligned with ldc % 4 == 0: stream-K shares use red.global.add.v4.f32
   int tma_store;       // tmC is valid: full-width chunks of plain stores leave through cp.async.bulk.tensor
 };
@@ -85,7 +78,7 @@ __device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
 
 // DT: 0 = fp32 operands fed as TF32 (k-block = 32 elements), 1 = bf16 operands (k-block = 64 elements); both are 128-byte
 // rows in shared memory, so tile sizes, the ring and the K-major descriptors are identical.
-template <int BN, bool A_MN, bool B_MN, int EPI, int DT = 0>
+template <int BN, bool A_MN, bool B_MN, int DT = 0>
 __global__ void __launch_bounds__(NTHREADS, 1)
 gemm_p_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
               const __grid_constant__ CUtensorMap tmC, int M, int N, int K, int tiles_n, int tiles, int dp_tiles,
@@ -208,7 +201,7 @@ gemm_p_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
       const int m0 = (tile / tiles_n) * BM, n0 = (tile % tiles_n) * BN;
       const bool partial = (kb_hi - kb_lo) < nkb;            // stream-K share: reduce into C
       const bool first = (kb_lo == 0);
-      const bool bias_smem = (EPI == EPI_STORE) && ea.tma_store && ea.beta == 0.f && ea.bias != nullptr;   // kernel-uniform
+      const bool bias_smem = ea.tma_store && ea.beta == 0.f && ea.bias != nullptr;   // kernel-uniform
       if (bias_smem) {
         // the tile's bias slice goes to shared memory while the tile's MMAs still run (a global load per block inside
         // the drain loop was a dependent L2 round trip per 32 columns: 73 us instead of 45 on the EW GEMM of the step)
@@ -238,8 +231,8 @@ gemm_p_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
           __syncwarp();
           if (lane == 0) mbar_arrive(&tmem_empty[acc]);
         }
-        if (n0 + c0 >= N || rows <= 0 || ea.dbg == 1) continue;   // warp-uniform
-        if (EPI == EPI_STORE && ea.tma_store && !partial && ea.beta == 0.f && W == 32) {
+        if (n0 + c0 >= N || rows <= 0) continue;             // warp-uniform
+        if (ea.tma_store && !partial && ea.beta == 0.f && W == 32) {
           // TMA store: the warp's 32 x 32 block goes to a 128B-swizzled 4 KB staging tile (lane = row, 16-byte chunk
           // c at physical chunk c ^ (row & 7): conflict-free STS.128), then one bulk tensor store (clipped at M, N)
           if (lane == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");   // staging tile free again
@@ -265,21 +258,9 @@ gemm_p_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
           }
           continue;
         }
-        if (EPI == EPI_STORE && ea.tma_store) {              // generic path below reuses the staging tile
+        if (ea.tma_store) {                                  // generic path below reuses the staging tile
           if (lane == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
           __syncwarp();
-        }
-        if (ea.dbg == 3) {      // experiment: v1-style direct stores, one row per lane (no smem staging)
-          const int m = m_base + lane;
-          if (m < M) {
-            float* crow = ea.C + (size_t)m * ea.ldc + n0 + c0;
-#pragma unroll
-            for (int j = 0; j < 32; j += 4)
-              if (j < W && n0 + c0 + j + 3 < N)
-                *reinterpret_cast<float4*>(crow + j) = make_float4(__uint_as_float(r[j]), __uint_as_float(r[j + 1]),
-                                                                   __uint_as_float(r[j + 2]), __uint_as_float(r[j + 3]));
-          }
-          continue;
         }
 #pragma unroll
         for (int j = 0; j < 32; ++j)
@@ -288,27 +269,9 @@ gemm_p_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
         const int n = n0 + c0 + lane;
         const bool n_ok = (lane < W) && (n < N);
         float bv = 0.f;
-        if (EPI == EPI_STORE && ea.bias != nullptr && n_ok && first) bv = ea.bias[n];
+        if (ea.bias != nullptr && n_ok && first) bv = ea.bias[n];
         float* cptr = ea.C + (size_t)m_base * ea.ldc + n;
-        if (EPI == EPI_DZ) {
-          // loads of p first (8 rows in flight), then the stores: p and dz may not alias but the compiler cannot know
-          const float* pptr = ea.aux + (size_t)m_base * ea.ldc + n;
-          const float tscal = ea.scalar_dev ? __ldg(ea.scalar_dev) : ea.scalar;
-#pragma unroll
-          for (int r0 = 0; r0 < 32; r0 += 8) {
-            float pv[8], dv[8];
-#pragma unroll
-            for (int i = 0; i < 8; ++i) {
-              const bool ok = (r0 + i < rows) && n_ok;
-              pv[i] = ok ? __ldg(pptr + (size_t)(r0 + i) * ea.ldc) : 0.f;
-              dv[i] = (r0 + i < rows) ? __ldg(ea.rowv + m_base + r0 + i) : 0.f;
-            }
-#pragma unroll
-            for (int i = 0; i < 8; ++i)
-              if ((r0 + i < rows) && n_ok)
-                cptr[(size_t)(r0 + i) * ea.ldc] = tscal * pv[i] * (stg[(r0 + i) * 33 + lane] - dv[i]);
-          }
-        } else if (partial) {
+        if (partial) {
           if (ea.vec_red) {
             // 16-byte vector reductions: lane = (row lane/8, 4 columns starting at 4*(lane%8)), 4 rows per instruction
             const int cg = (lane & 7) * 4, rsub = lane >> 3;
@@ -343,11 +306,6 @@ gemm_p_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
 #pragma unroll
           for (int i = 0; i < 32; ++i)
             if ((i < rows) && n_ok) cptr[(size_t)i * ea.ldc] = ea.alpha * stg[i * 33 + lane] + bv + ea.beta * cv[i];
-        } else if (ea.dbg == 2) {   // experiment: smem staging only, a single store per chunk
-          float acc2 = 0.f;
-#pragma unroll 8
-          for (int rr = 0; rr < 32; ++rr) acc2 += stg[rr * 33 + lane];
-          if (n_ok && rows > 0) cptr[0] = acc2;
         } else {
 #pragma unroll 8
           for (int rr = 0; rr < 32; ++rr) {
@@ -358,7 +316,7 @@ gemm_p_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
       }
       ++seg;
     }
-    if (EPI == EPI_STORE && ea.tma_store && lane == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
+    if (ea.tma_store && lane == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
   }
   tcgen05_fence_before();
   __syncthreads();
@@ -368,16 +326,16 @@ gemm_p_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
   }
 }
 
-template <int BN, bool A_MN, bool B_MN, int EPI, int DT = 0>
+template <int BN, bool A_MN, bool B_MN, int DT = 0>
 static int launch_p(const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap& tcm, int M, int N, int K, int tiles_n, int tiles,
                     int dp_tiles, int grid, const EpiArgs& ea, cudaStream_t s) {
   using S = PCfg<BN>;
   static bool attr = false;
   if (!attr) {
-    cudaFuncSetAttribute(gemm_p_kernel<BN, A_MN, B_MN, EPI, DT>, cudaFuncAttributeMaxDynamicSharedMemorySize, S::TOTAL);
+    cudaFuncSetAttribute(gemm_p_kernel<BN, A_MN, B_MN, DT>, cudaFuncAttributeMaxDynamicSharedMemorySize, S::TOTAL);
     attr = true;
   }
-  gemm_p_kernel<BN, A_MN, B_MN, EPI, DT><<<grid, NTHREADS, S::TOTAL, s>>>(ta, tb, tcm, M, N, K, tiles_n, tiles, dp_tiles, ea);
+  gemm_p_kernel<BN, A_MN, B_MN, DT><<<grid, NTHREADS, S::TOTAL, s>>>(ta, tb, tcm, M, N, K, tiles_n, tiles, dp_tiles, ea);
   return check_launch("gemm_p_kernel");
 }
 
@@ -407,25 +365,19 @@ static int choose_bn(int M, int N, int K, bool b_mn, bool allow_sk) {
 
 }  // namespace tc
 
-static bool use_v1() {
-  return option("GIC_GEMM_V1", 0) == 1;
-}
-
-// Persistent GEMM entry.  handled = false (nothing launched) when the operands do not meet TMA's constraints.
-// epi: 0 = C = alpha*op(A)*op(B) + beta*C + bias;  1 = C = scalar * aux .* (op(A)*op(B) - rowv[:,None]) (softmax bwd)
+// Persistent GEMM entry: C = alpha*op(A)*op(B) + beta*C + bias.  handled = false (nothing launched) when the operands do
+// not meet TMA's constraints or the shape is left to the other kernels.
 int gemm_tc_persistent(bool transA, bool transB, int M, int N, int K, float alpha, const float* A, int lda,
-                       const float* B, int ldb, float beta, float* C, int ldc, const float* bias, int epi,
-                       const float* aux, const float* rowv, float scalar, cudaStream_t stream, bool* handled) {
-  extern const float* temperature_device();
+                       const float* B, int ldb, float beta, float* C, int ldc, const float* bias, cudaStream_t stream,
+                       bool* handled) {
   using namespace tc;
   *handled = false;
-  if (use_v1() && epi == EPI_STORE) return GIC_OK;
   if (M <= 0 || N <= 0 || K <= 0) return GIC_OK;
   if (!aligned16(A) || !aligned16(B) || (lda % 4) || (ldb % 4)) return GIC_OK;
-  if (epi == EPI_STORE && ((long long)M * N < 64 * 64 || K < 32)) return GIC_OK;
+  if ((long long)M * N < 64 * 64 || K < 32) return GIC_OK;
   const bool rn = tf32_round_in_tma();
   const bool a_mn = transA, b_mn = !transB;
-  const bool allow_sk = (epi == EPI_STORE) && (beta == 0.f || beta == 1.f);
+  const bool allow_sk = (beta == 0.f || beta == 1.f);
   int BN = choose_bn(M, N, K, b_mn, allow_sk);
   { const int f = option("GIC_GEMM_BN", 0); if (f == 64 || f == 128 || f == 192 || f == 256 || (!b_mn && (f == 144 || f == 240))) BN = f; }   // tuning
   CUtensorMap ta, tb;
@@ -440,8 +392,7 @@ int gemm_tc_persistent(bool transA, bool transB, int M, int N, int K, float alph
   const int G = num_sms();
   const int tiles_n = cdiv(N, BN), tiles_m = cdiv(M, BM), tiles = tiles_n * tiles_m, nkb = cdiv(K, BK);
   int dp_tiles = tiles;
-  const int sk_env = option("GIC_SK", 1), dbg_env = option("GIC_GEMM_DBG", 0);
-  if (allow_sk && sk_env) {
+  if (allow_sk && option("GIC_SK", 1)) {
     // stream-K only when whole tiles cannot occupy half the machine (long-K / small-MN shapes of the backward pass):
     // every CTA gets an equal share of the (tile, k-block) iteration space.  fp32 reductions into L2 cost ~5 ps per
     // element, so a tail of partial tiles after full data-parallel rounds does not pay off.
@@ -449,9 +400,8 @@ int gemm_tc_persistent(bool transA, bool transB, int M, int N, int K, float alph
   }
   // Long-K shapes that need no stream-K (dW_out, dhtop of the generator backward) measure ~20% faster on the
   // one-tile-per-CTA kernel of gemm_tcgen05.cu (profiles/README.md, "GEMM A/B"): leave them to it.
-  if (epi == EPI_STORE && dp_tiles == tiles && nkb >= 128 && dbg_env != 7) return GIC_OK;
-  int grid = (dp_tiles < tiles) ? G : min(tiles, G);
-  if (dbg_env == 6 && dp_tiles == tiles) grid = tiles;      // experiment: one tile per CTA, hardware-scheduled
+  if (dp_tiles == tiles && nkb >= 128) return GIC_OK;
+  const int grid = (dp_tiles < tiles) ? G : min(tiles, G);
   if (dp_tiles < tiles && beta == 0.f) {
     // zero the rows that hold stream-K tiles (a superset: data-parallel tiles in those rows are stored afterwards)
     const int row0 = (dp_tiles / tiles_n) * BM;
@@ -460,41 +410,30 @@ int gemm_tc_persistent(bool transA, bool transB, int M, int N, int K, float alph
     if (e != cudaSuccess) { set_error("memset2D: %s", cudaGetErrorString(e)); return GIC_ERR_CUDA; }
   }
   EpiArgs ea;
-  ea.alpha = alpha; ea.beta = beta; ea.C = C; ea.ldc = ldc; ea.bias = bias; ea.aux = aux; ea.rowv = rowv; ea.scalar = scalar; ea.scalar_dev = (epi == EPI_DZ) ? temperature_device() : nullptr; ea.dbg = dbg_env;
+  ea.alpha = alpha; ea.beta = beta; ea.C = C; ea.ldc = ldc; ea.bias = bias;
   CUtensorMap tcm;
   ea.vec_red = (aligned16(C) && (ldc % 4) == 0 && (!bias || aligned16(bias))) ? 1 : 0;
   ea.tma_store = 0;
-  if (epi == EPI_STORE && beta == 0.f && aligned16(C) && (ldc % 4) == 0 && (!bias || aligned16(bias)) && dbg_env != 5)
+  if (beta == 0.f && aligned16(C) && (ldc % 4) == 0 && (!bias || aligned16(bias)))
     ea.tma_store = make_map(&tcm, C, M, N, ldc, 32, 32, false, false) ? 1 : 0;
   if (!ea.tma_store) tcm = ta;                       // unused placeholder
   int rc = GIC_OK;
-#define GIC_P(BN_, EPI_)                                                                                            \
+#define GIC_P(BN_)                                                                                                  \
   do {                                                                                                              \
-    if (!a_mn && !b_mn) rc = launch_p<BN_, false, false, EPI_>(ta, tb, tcm, M, N, K, tiles_n, tiles, dp_tiles, grid, ea, stream); \
-    else if (a_mn && !b_mn) rc = launch_p<BN_, true, false, EPI_>(ta, tb, tcm, M, N, K, tiles_n, tiles, dp_tiles, grid, ea, stream); \
+    if (!a_mn && !b_mn) rc = launch_p<BN_, false, false>(ta, tb, tcm, M, N, K, tiles_n, tiles, dp_tiles, grid, ea, stream); \
+    else if (a_mn && !b_mn) rc = launch_p<BN_, true, false>(ta, tb, tcm, M, N, K, tiles_n, tiles, dp_tiles, grid, ea, stream); \
     else if constexpr ((BN_ % 32) == 0) {                                                                           \
-      if (!a_mn) rc = launch_p<BN_, false, true, EPI_>(ta, tb, tcm, M, N, K, tiles_n, tiles, dp_tiles, grid, ea, stream);  \
-      else rc = launch_p<BN_, true, true, EPI_>(ta, tb, tcm, M, N, K, tiles_n, tiles, dp_tiles, grid, ea, stream);         \
+      if (!a_mn) rc = launch_p<BN_, false, true>(ta, tb, tcm, M, N, K, tiles_n, tiles, dp_tiles, grid, ea, stream);  \
+      else rc = launch_p<BN_, true, true>(ta, tb, tcm, M, N, K, tiles_n, tiles, dp_tiles, grid, ea, stream);         \
     }                                                                                                               \
   } while (0)
-  if (epi == EPI_DZ) {
-    // A = demb [M, K] K-major, B = W_e [K, N] N-major
-    if (a_mn || !b_mn) { set_error("gemm_tc_persistent: dz epilogue expects A[M,K], B[K,N]"); return GIC_ERR_UNSUPPORTED; }
-    switch (BN) {
-      case 64: rc = launch_p<64, false, true, EPI_DZ>(ta, tb, tcm, M, N, K, tiles_n, tiles, dp_tiles, grid, ea, stream); break;
-      case 128: rc = launch_p<128, false, true, EPI_DZ>(ta, tb, tcm, M, N, K, tiles_n, tiles, dp_tiles, grid, ea, stream); break;
-      case 192: rc = launch_p<192, false, true, EPI_DZ>(ta, tb, tcm, M, N, K, tiles_n, tiles, dp_tiles, grid, ea, stream); break;
-      default: rc = launch_p<256, false, true, EPI_DZ>(ta, tb, tcm, M, N, K, tiles_n, tiles, dp_tiles, grid, ea, stream); break;
-    }
-  } else {
-    switch (BN) {
-      case 64: GIC_P(64, EPI_STORE); break;
-      case 128: GIC_P(128, EPI_STORE); break;
-      case 144: GIC_P(144, EPI_STORE); break;
-      case 192: GIC_P(192, EPI_STORE); break;
-      case 240: GIC_P(240, EPI_STORE); break;
-      default: GIC_P(256, EPI_STORE); break;
-    }
+  switch (BN) {
+    case 64: GIC_P(64); break;
+    case 128: GIC_P(128); break;
+    case 144: GIC_P(144); break;
+    case 192: GIC_P(192); break;
+    case 240: GIC_P(240); break;
+    default: GIC_P(256); break;
   }
 #undef GIC_P
   if (rc == GIC_OK) *handled = true;
@@ -556,8 +495,7 @@ int gemm_tc_bf16(bool transA, bool transB, int M, int N, int K, float alpha, con
     if (e != cudaSuccess) { set_error("memset2D: %s", cudaGetErrorString(e)); return GIC_ERR_CUDA; }
   }
   EpiArgs ea;
-  ea.alpha = alpha; ea.beta = beta; ea.C = C; ea.ldc = ldc; ea.bias = bias; ea.aux = nullptr; ea.rowv = nullptr;
-  ea.scalar = 0.f; ea.scalar_dev = nullptr; ea.dbg = 0;
+  ea.alpha = alpha; ea.beta = beta; ea.C = C; ea.ldc = ldc; ea.bias = bias;
   ea.vec_red = (aligned16(C) && (ldc % 4) == 0 && (!bias || aligned16(bias))) ? 1 : 0;
   CUtensorMap tcm;
   ea.tma_store = 0;
@@ -567,10 +505,10 @@ int gemm_tc_bf16(bool transA, bool transB, int M, int N, int K, float alpha, con
   int rc = GIC_OK;
 #define GIC_PB(BN_)                                                                                                  \
   do {                                                                                                              \
-    if (!a_mn && !b_mn) rc = launch_p<BN_, false, false, EPI_STORE, 1>(ta, tb, tcm, M, N, K, tiles_n, tiles, dp_tiles, grid, ea, stream); \
-    else if (a_mn && !b_mn) rc = launch_p<BN_, true, false, EPI_STORE, 1>(ta, tb, tcm, M, N, K, tiles_n, tiles, dp_tiles, grid, ea, stream); \
-    else if (!a_mn) rc = launch_p<BN_, false, true, EPI_STORE, 1>(ta, tb, tcm, M, N, K, tiles_n, tiles, dp_tiles, grid, ea, stream); \
-    else rc = launch_p<BN_, true, true, EPI_STORE, 1>(ta, tb, tcm, M, N, K, tiles_n, tiles, dp_tiles, grid, ea, stream); \
+    if (!a_mn && !b_mn) rc = launch_p<BN_, false, false, 1>(ta, tb, tcm, M, N, K, tiles_n, tiles, dp_tiles, grid, ea, stream); \
+    else if (a_mn && !b_mn) rc = launch_p<BN_, true, false, 1>(ta, tb, tcm, M, N, K, tiles_n, tiles, dp_tiles, grid, ea, stream); \
+    else if (!a_mn) rc = launch_p<BN_, false, true, 1>(ta, tb, tcm, M, N, K, tiles_n, tiles, dp_tiles, grid, ea, stream); \
+    else rc = launch_p<BN_, true, true, 1>(ta, tb, tcm, M, N, K, tiles_n, tiles, dp_tiles, grid, ea, stream); \
   } while (0)
   switch (BN) {
     case 64: GIC_PB(64); break;

@@ -180,186 +180,6 @@ lstm_step_tf32_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_cons
   }
 }
 
-
-// ---------------------------------------------------------------------------------------------------------
-// Split-K variant over a 4-CTA thread-block cluster.  The decode-step kernels are bound by how fast ONE SM can ingest
-// operands through TMA (~44 B/clk, profiles/README.md), so the way to shorten the main loop is fewer bytes per SM: a
-// cluster of four CTAs shares one 128-row x 32-unit tile (128 accumulator columns, gate-interleaved) and each CTA runs a
-// quarter of the k-blocks: 8 x 32 KB instead of 32 x 20 KB at c2.  The four partial tiles meet over distributed shared
-// memory: every CTA stages its partial in shared memory grouped by destination rank, the cluster synchronises, and CTA r
-// adds the four partials (rank order: deterministic) of units 8r .. 8r+7 and applies the cell update to them.
-// ---------------------------------------------------------------------------------------------------------
-constexpr int SK_CL = 4;                 // cluster size = K splits
-constexpr int SK_U = 32;                 // hidden units per cluster tile
-constexpr int SK_STAGE = BM * BK * 4 + 4 * SK_U * BK * 4;      // 16 KB + 16 KB
-constexpr int SK_STAGES = 6;
-constexpr int SK_SMEM = SK_STAGES * SK_STAGE + 1024 + 256;
-
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-  asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ float4 ld_dsmem_f4(uint32_t local_addr, uint32_t rank) {
-  uint32_t ra;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(ra) : "r"(local_addr), "r"(rank));
-  float4 v;
-  asm volatile("ld.shared::cluster.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(ra) : "memory");
-  return v;
-}
-
-__global__ void __launch_bounds__(NTHREADS, 1)
-lstm_step_splitk_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ CUtensorMap tmH,
-                        const __grid_constant__ CUtensorMap tmWih, const __grid_constant__ CUtensorMap tmWhh, int B,
-                        int H, int In, const float* __restrict__ b_ih, const float* __restrict__ b_hh,
-                        const float* __restrict__ c_prev, float* __restrict__ acts, float* __restrict__ c_out,
-                        float* __restrict__ h_out, float* __restrict__ htop, int L, int t) {
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
-  uint64_t* full = reinterpret_cast<uint64_t*>(smem + SK_STAGES * SK_STAGE);
-  uint64_t* empty = full + SK_STAGES;
-  uint64_t* tmem_full = empty + SK_STAGES;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tmem_full + 1);
-  uint8_t* part = smem;                    // [dest rank 4][row 128][8 chunks of 16 B, XOR-swizzled by row & 7]: aliases the ring
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int ks = blockIdx.x % SK_CL;       // cluster rank = K split = the quarter of the tile's units this CTA finishes
-  const int j0 = (blockIdx.x / SK_CL) * SK_U, m0 = blockIdx.y * BM;
-  const int nkb1 = (In + BK - 1) / BK, nkb2 = (H + BK - 1) / BK, nkb = nkb1 + nkb2;
-  const int kb_lo = ks * (nkb / SK_CL), kb_hi = kb_lo + nkb / SK_CL;
-  constexpr uint32_t TMEM_COLS = 4 * SK_U;
-
-  if (warp == 0 && lane == 0) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&tmX) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&tmWih) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&tmH) : "memory");
-    asm volatile("prefetch.tensormap [%0];" ::"l"(&tmWhh) : "memory");
-    for (int s = 0; s < SK_STAGES; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], 1); }
-    mbar_init(tmem_full, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "n"(TMEM_COLS));
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-  }
-  tcgen05_fence_before();
-  __syncthreads();
-  tcgen05_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-
-  if (warp == 0) {
-    if (lane == 0) {
-      for (int kb = kb_lo, it = 0; kb < kb_hi; ++kb, ++it) {
-        const int s = it % SK_STAGES;
-        const uint32_t ph = (it / SK_STAGES) & 1;
-        mbar_wait(&empty[s], ph ^ 1);
-        uint8_t* sa = smem + s * SK_STAGE;
-        uint8_t* sb = sa + BM * BK * 4;
-        mbar_expect_tx(&full[s], SK_STAGE);
-        const bool first = kb < nkb1;
-        const int k0 = (first ? kb : kb - nkb1) * BK;
-        tma_load_2d(sa, first ? &tmX : &tmH, &full[s], k0, m0);
-#pragma unroll
-        for (int g = 0; g < 4; ++g) tma_load_2d(sb + g * (SK_U * 128), first ? &tmWih : &tmWhh, &full[s], k0, g * H + j0);
-      }
-    }
-  } else if (warp == 1) {
-    if (lane == 0) {
-      constexpr uint32_t idesc = make_idesc(0, 0, 4 * SK_U);
-      for (int kb = kb_lo, it = 0; kb < kb_hi; ++kb, ++it) {
-        const int s = it % SK_STAGES;
-        const uint32_t ph = (it / SK_STAGES) & 1;
-        mbar_wait(&full[s], ph);
-        tcgen05_fence_after();
-        const uint32_t sa = smem_u32(smem + s * SK_STAGE);
-        const uint32_t sb = sa + BM * BK * 4;
-#pragma unroll
-        for (int k = 0; k < BK / UMMA_K; ++k)
-          umma_tf32(tmem_base, make_desc(sa + k * 32, 16, 1024, 2), make_desc(sb + k * 32, 16, 1024, 2), idesc,
-                    (it > 0 || k > 0) ? 1u : 0u);
-        umma_commit(&empty[s]);
-      }
-      umma_commit(tmem_full);
-    }
-  } else {
-    // stage this CTA's partial tile, grouped by the rank that will finish each unit
-    mbar_wait(tmem_full, 0);
-    tcgen05_fence_after();
-    const int q = warp & 3;
-    const int row = q * 32 + lane;
-    const uint32_t lane_addr = tmem_base + ((uint32_t)(q * 32) << 16);
-    const int sw = row & 7;
-#pragma unroll
-    for (int g = 0; g < 4; ++g) {
-      uint32_t r[32];
-      tmem_ld32(lane_addr + g * SK_U, r);              // gate g, units 0..31 of the tile
-#pragma unroll
-      for (int rr = 0; rr < SK_CL; ++rr) {             // units 8rr .. 8rr+7 belong to rank rr: chunks 2g, 2g+1 of its row
-        uint8_t* dst = part + rr * (BM * 128) + row * 128;
-        *reinterpret_cast<float4*>(dst + (((2 * g) ^ sw) << 4)) =
-            make_float4(__uint_as_float(r[8 * rr + 0]), __uint_as_float(r[8 * rr + 1]), __uint_as_float(r[8 * rr + 2]), __uint_as_float(r[8 * rr + 3]));
-        *reinterpret_cast<float4*>(dst + (((2 * g + 1) ^ sw) << 4)) =
-            make_float4(__uint_as_float(r[8 * rr + 4]), __uint_as_float(r[8 * rr + 5]), __uint_as_float(r[8 * rr + 6]), __uint_as_float(r[8 * rr + 7]));
-      }
-    }
-  }
-  __syncwarp();
-  cluster_sync_all();                                  // every CTA's partial is in its shared memory
-
-  if (warp >= 2) {
-    const int q = warp & 3;
-    const int row = q * 32 + lane;
-    const int b = m0 + row;
-    const int sw = row & 7;
-    const uint32_t my = smem_u32(part + ks * (BM * 128) + row * 128);
-    float pre[32];                                     // [gate 4][unit 8] pre-activations of this rank's units
-#pragma unroll
-    for (int i = 0; i < 32; ++i) pre[i] = 0.f;
-#pragma unroll
-    for (int src = 0; src < SK_CL; ++src) {            // fixed order: the sum does not depend on scheduling
-#pragma unroll
-      for (int c = 0; c < 8; ++c) {
-        const float4 v = ld_dsmem_f4(my + ((c ^ sw) << 4), (uint32_t)src);
-        pre[4 * c + 0] += v.x; pre[4 * c + 1] += v.y; pre[4 * c + 2] += v.z; pre[4 * c + 3] += v.w;
-      }
-    }
-    if (b < B) {
-      const int j = j0 + 8 * ks;
-      float cp[8], ai[8], af[8], ag[8], ao[8], cn[8], hn[8];
-      *reinterpret_cast<float4*>(cp) = *reinterpret_cast<const float4*>(c_prev + (size_t)b * H + j);
-      *reinterpret_cast<float4*>(cp + 4) = *reinterpret_cast<const float4*>(c_prev + (size_t)b * H + j + 4);
-#pragma unroll
-      for (int e = 0; e < 8; ++e) {
-        const float pi = pre[0 * 8 + e] + b_ih[0 * H + j + e] + b_hh[0 * H + j + e];
-        const float pf = pre[1 * 8 + e] + b_ih[1 * H + j + e] + b_hh[1 * H + j + e];
-        const float pg = pre[2 * 8 + e] + b_ih[2 * H + j + e] + b_hh[2 * H + j + e];
-        const float po = pre[3 * 8 + e] + b_ih[3 * H + j + e] + b_hh[3 * H + j + e];
-        ai[e] = sigmoidf_acc(pi); af[e] = sigmoidf_acc(pf); ag[e] = tanhf(pg); ao[e] = sigmoidf_acc(po);
-        cn[e] = af[e] * cp[e] + ai[e] * ag[e];
-        hn[e] = ao[e] * tanhf(cn[e]);
-      }
-      auto st8 = [](float* dst, const float* v) {
-        *reinterpret_cast<float4*>(dst) = make_float4(v[0], v[1], v[2], v[3]);
-        *reinterpret_cast<float4*>(dst + 4) = make_float4(v[4], v[5], v[6], v[7]);
-      };
-      if (acts) {
-        float* arow = acts + (size_t)b * 4 * H + j;
-        st8(arow, ai); st8(arow + H, af); st8(arow + 2 * H, ag); st8(arow + 3 * H, ao);
-      }
-      st8(c_out + (size_t)b * H + j, cn);
-      st8(h_out + (size_t)b * H + j, hn);
-      if (htop) st8(htop + ((size_t)b * L + t) * H + j, hn);
-    }
-  }
-  __syncwarp();
-  cluster_sync_all();                                  // peers have read this CTA's partial: its shared memory may go
-  tcgen05_fence_before();
-  __syncthreads();
-  if (warp == 1) {
-    tcgen05_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(TMEM_COLS));
-  }
-}
-
 }  // namespace tc
 
 // One LSTM layer / time step on the tensor cores.  handled = false (nothing launched) when the shape does not fit
@@ -392,40 +212,6 @@ int lstm_step_tc(const float* x, int In, const float* h_prev, const float* W_ih,
     attr = true;
   }
   ProfScope prof(PROF_GEMM_DECODE, 2.0 * B * 4 * H * (In + H), stream);
-  // split-K over 4-CTA clusters when the k-blocks divide by 4 and the clusters give at least half the SMs a CTA
-  {
-    // Measured at c2 (bench32*.log): 23.3 us per launch against 22.0 us for the one-CTA-per-tile kernel, decode 0.822 vs
-    // 0.799 ms -- the two cluster barriers, the TMEM -> shared staging and the DSMEM reads cost more than the shorter
-    // main loop saves.  Opt-in (option GIC_LSTM_SPLITK = 1).
-    const int sk_env = option("GIC_LSTM_SPLITK", 0) == 1;
-    const int nkb = cdiv(In, BK) + cdiv(H, BK);
-    if (sk_env && (H % SK_U) == 0 && (In % BK) == 0 && (H % BK) == 0 && (nkb % SK_CL) == 0 && nkb / SK_CL >= 2 &&
-        (H / SK_U) * SK_CL * mt * 2 >= num_sms() && !option_is_set("GIC_LSTM_U")) {
-      CUtensorMap swi, swh;
-      if (make_map(&swi, W_ih, 4 * H, In, In, BK, SK_U, rn, false) && make_map(&swh, W_hh, 4 * H, H, H, BK, SK_U, rn, false)) {
-        static bool sk_attr = false;
-        if (!sk_attr) {
-          cudaFuncSetAttribute(lstm_step_splitk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SK_SMEM);
-          sk_attr = true;
-        }
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3((H / SK_U) * SK_CL, mt, 1);
-        cfg.blockDim = dim3(NTHREADS, 1, 1);
-        cfg.dynamicSmemBytes = SK_SMEM;
-        cfg.stream = stream;
-        cudaLaunchAttribute at[1];
-        at[0].id = cudaLaunchAttributeClusterDimension;
-        at[0].val.clusterDim.x = SK_CL; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-        cfg.attrs = at; cfg.numAttrs = 1;
-        cudaError_t e = cudaLaunchKernelEx(&cfg, lstm_step_splitk_kernel, tx, th, swi, swh, B, H, In, b_ih, b_hh, c_prev, acts,
-                                           c_out, h_out, htop, L, t);
-        if (e != cudaSuccess) { set_error("lstm_step_splitk_kernel launch: %s", cudaGetErrorString(e)); return GIC_ERR_CUDA; }
-        int rc = check_launch("lstm_step_splitk_kernel");
-        if (rc == GIC_OK) *handled = true;
-        return rc;
-      }
-    }
-  }
   dim3 grid(H / U, mt);
   cudaError_t le;
 #define GIC_LSTM(U_) le = launch_pdl(lstm_step_tf32_kernel<U_>, grid, dim3(NTHREADS), LstmCfg<U_>::SMEM, stream, tx, th, twi, twh, B, H, In, b_ih, b_hh, c_prev, acts, c_out, h_out, htop, L, t)

@@ -104,8 +104,6 @@ class GANInstructor:
         # opt-in (args.sync_bn / GIC_SYNC_BN=1): the reference is single-GPU, per-shard statistics are the documented default
         self.sync_bn = bool(getattr(args, "sync_bn", 0)) or os.environ.get("GIC_SYNC_BN", "0") == "1"
         self.overlap = os.environ.get("GIC_NO_OVERLAP", "0") != "1"
-        self.d_priority = os.environ.get("GIC_D_PRIORITY", "0") == "1"
-        self._hp = None
         self.world, self.rank = 1, 0
         if torch.distributed.is_available() and torch.distributed.is_initialized():
             self.world = torch.distributed.get_world_size()
@@ -471,29 +469,12 @@ class GANInstructor:
                                         P(g(disc.feature2out.bias)), P(g(disc.out2logits.weight)),
                                         P(g(disc.out2logits.bias)), P(dinp), want_param, acc, stream), "gic_disc_bwd")
 
-        # The seed of d_loss w.r.t. D(real) does not depend on D(fake) (every divergence except rsgan), and neither does
-        # anything else in backward(real), so it CAN run on the side stream right behind forward(real), underneath the
-        # decode loop.  Measured (profiles/step_timeline.py): the decode kernels need nearly every SM (126-128 CTAs of
-        # ~200 KB shared memory), so whatever runs beside them stalls them almost one for one: decode 989 -> 1232 us, the
-        # phase after the losses 1346 -> 1150 us, step 2.62 -> 2.67 ms.  Opt-in only (GIC_EARLY_REAL=1).
-        early_real = train and self.overlap and loss_type != "rsgan" and os.environ.get("GIC_EARLY_REAL", "0") == "1"
-        real_bwd_done = None
         if side is not None:
             side.wait_stream(main)
             with torch.cuda.stream(side):
                 (d_real,), saved_r = disc_fwd_raw(lib, mode, None, captions, B, L, V, De, R, fsz, nfl, *dW, [k0], drop_p,
                                                   dev)
                 self._mark("side: D(real) forward done")
-                if early_real:
-                    nR = B * R
-                    seed_real = self._buf("seed_real", nR)
-                    _lib.check(lib.gic_gan_loss_fwd_bwd(_lib.LOSS_TYPES[loss_type], P(d_real), P(d_real), P(d_real), nR,
-                                                        P(self._buf("loss_scratch", 2)), P(seed_real), None, None,
-                                                        side.cuda_stream), "gic_gan_loss_fwd_bwd")
-                    disc_bwd(seed_real, k0, None, captions, saved_r, 1, 0, None, bws, side.cuda_stream)
-                    real_bwd_done = torch.cuda.Event()
-                    real_bwd_done.record(side)
-                    self._mark("side: D backward(real) done")
         else:
             (d_real,), saved_r = disc_fwd_raw(lib, mode, None, captions, B, L, V, De, R, fsz, nfl, *dW, [k0], drop_p, dev)
         # -- step-0 input (:144-147)
@@ -619,25 +600,13 @@ class GANInstructor:
                     gen_chain(bws2, side.cuda_stream)
                     gen_done.record(side)
                 g_bucketed = self._gen_backward_early_bucket(_bwd)
-            # GIC_D_PRIORITY=1 (experiment): the D chain on a high-priority stream, so that it finishes ahead of the
-            # generator chain and its gradient all-reduce runs under the generator chain's tail
-            dst = main
-            if self.d_priority:
-                if self._hp is None:
-                    self._hp = torch.cuda.Stream(device=self.device, priority=-1)
-                dst = self._hp
-                dst.wait_stream(main)
-            with torch.cuda.stream(dst):
-                ds = dst.cuda_stream
-                if real_bwd_done is None:
-                    disc_bwd(seeds[0], k0, None, captions, saved_r, 1, 0, None, bws, ds)
-                    self._mark("D chain: backward(real) done")
-                else:
-                    dst.wait_event(real_bwd_done)         # fake accumulates onto real's parameter gradients
-                disc_bwd(seeds[1], k1, probs, None, saved_f, 1, 1, None, bws, ds)
-                self._mark("D chain: backward(fake) done")
-                d_sq = self._allreduce(fd.grad, 0, self._sq_d)
-                self._mark("D chain: gradients all-reduced")
+            # the D chain on main: backward(real), then backward(fake) accumulated onto its parameter gradients
+            disc_bwd(seeds[0], k0, None, captions, saved_r, 1, 0, None, bws, main.cuda_stream)
+            self._mark("D chain: backward(real) done")
+            disc_bwd(seeds[1], k1, probs, None, saved_f, 1, 1, None, bws, main.cuda_stream)
+            self._mark("D chain: backward(fake) done")
+            d_sq = self._allreduce(fd.grad, 0, self._sq_d)
+            self._mark("D chain: gradients all-reduced")
             with torch.cuda.stream(side):
                 self._mark("G chain: backward done")
                 self._gen_allreduce_rest(g_bucketed)
@@ -645,12 +614,9 @@ class GANInstructor:
                 g_sq = self._peer is not None and self.world > 1 and not self.skip_allreduce and self._peer.owns(fg.grad)
                 out["g_sqnorm"] = self._clip_adam(fg, a.gen_lr, update, 3, self._sq_g.sum().reshape(1) if g_sq else None)
                 self._mark("G chain: clip + Adam done")
-            with torch.cuda.stream(dst):
-                dst.wait_event(gen_done)
-                out["d_sqnorm"] = self._clip_adam(fd, a.disc_lr, update, 1, self._sq_d if d_sq else None)
-                self._mark("D chain: clip + Adam done")
-            if dst is not main:
-                main.wait_stream(dst)
+            main.wait_event(gen_done)
+            out["d_sqnorm"] = self._clip_adam(fd, a.disc_lr, update, 1, self._sq_d if d_sq else None)
+            self._mark("D chain: clip + Adam done")
             main.wait_stream(side)
             self._mark("end")
         else:

@@ -326,7 +326,7 @@ gic_ctx_t* gic_ctx_create(void);
 gic_ctx_t* gic_ctx_set_current(gic_ctx_t* ctx);
 void gic_ctx_destroy(gic_ctx_t* ctx);
 /* A/B and tuning switches of the CURRENT context (which kernel variant a launch path takes: GIC_DECODE_STEP, GIC_FUSED_SAMPLE,
- * GIC_GEMM_2CTA, GIC_CONV_MMA, GIC_BPTT_PERSISTENT, GIC_BPTT_FUSED, GIC_FUSED_DZ_BF16, GIC_LSTM_SPLITK, GIC_PDL, ...; the
+ * GIC_GEMM_2CTA, GIC_CONV_MMA, GIC_BPTT_PERSISTENT, GIC_BPTT_FUSED, GIC_FUSED_DZ_BF16, GIC_PDL, ...; the
  * full table is in DESIGN.md).  They are integers held by the context; a switch nobody set is looked up in the process
  * environment under the same name ONCE per context -- the first time a launch path asks -- and remembered, so no launch
  * path calls getenv twice and a running job cannot be re-routed by a later setenv.

@@ -23,6 +23,6 @@ def bench(M, N, K, lda, ldb, ldc, tB=1, beta=0.0, iters=100):
     us = e0.elapsed_time(e1) * 1e3 / iters
     print(f"M{M} N{N} K{K} lda{lda} ldb{ldb} ldc{ldc} tB{tB} beta{beta}: {us:8.2f} us  {2.0*M*N*K/us/1e6:7.1f} TF/s", flush=True)
 
-print("V1 =", os.environ.get("GIC_GEMM_V1", "0"), "SK =", os.environ.get("GIC_SK"), "DBG =", os.environ.get("GIC_GEMM_DBG"))
+print("SK =", os.environ.get("GIC_SK"))
 bench(18944, 1024, 1024, 1024, 1024, 1024)   # 148 x 4 tiles of 128 x 256: exactly 4 rounds
 bench(18944, 1024, 4096, 4096, 4096, 1024)

@@ -1,4 +1,4 @@
-"""Tile-width sweep of the persistent TF32 GEMM on one shape (option GIC_GEMM_BN), with and without the epilogue's stores."""
+"""Tile-width sweep of the persistent TF32 GEMM on one shape (option GIC_GEMM_BN)."""
 import os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -14,20 +14,18 @@ def bench(mode, tA, tB, M, N, K, iters=100):
     C = torch.zeros(M, N, device=dev)
     s = L.stream()
     for bn in (0, 128, 192, 240, 256):
-        row = []
-        for dbg in (0, 1):
-            L.set_option("GIC_GEMM_DBG", dbg); L.set_option("GIC_GEMM_BN", bn)
-            def run():
-                L.check(lib.gic_gemm(mode, tA, tB, M, N, K, 1.0, L.ptr(A), A.shape[1], L.ptr(B), B.shape[1], 0.0, L.ptr(C), N, None, s), "gemm")
-            for _ in range(5): run()
-            torch.cuda.synchronize()
-            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            e0.record()
-            for _ in range(iters): run()
-            e1.record(); torch.cuda.synchronize()
-            row.append(e0.elapsed_time(e1) * 1e3 / iters)
-        print(f"mode {mode} tA{tA} tB{tB} {M}x{N}x{K} BN {bn or 'auto':>4}: {row[0]:7.1f} us with stores | {row[1]:7.1f} us without", flush=True)
-    L.clear_option("GIC_GEMM_DBG"); L.clear_option("GIC_GEMM_BN")
+        L.set_option("GIC_GEMM_BN", bn)
+        def run():
+            L.check(lib.gic_gemm(mode, tA, tB, M, N, K, 1.0, L.ptr(A), A.shape[1], L.ptr(B), B.shape[1], 0.0, L.ptr(C), N, None, s), "gemm")
+        for _ in range(5): run()
+        torch.cuda.synchronize()
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record()
+        for _ in range(iters): run()
+        e1.record(); torch.cuda.synchronize()
+        us = e0.elapsed_time(e1) * 1e3 / iters
+        print(f"mode {mode} tA{tA} tB{tB} {M}x{N}x{K} BN {bn or 'auto':>4}: {us:7.1f} us", flush=True)
+    L.clear_option("GIC_GEMM_BN")
 
 
 bench(1, 0, 1, 10000, 2048, 512)

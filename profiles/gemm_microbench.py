@@ -39,7 +39,6 @@ def bench(mode, tA, tB, M, N, K, iters=200, beta=0.0):
 
 
 if __name__ == "__main__":
-    print("GIC_GEMM_V1 =", os.environ.get("GIC_GEMM_V1", "0"), flush=True)
     if len(sys.argv) > 1 and sys.argv[1] == "short":
         bench(1, 0, 0, 16384, 900, 900, beta=1.0)
         bench(1, 1, 0, 10000, 512, 5120)
