@@ -172,6 +172,12 @@ def _declare(L):
     L.gic_decode_beam_workspace_floats.restype = Z
     L.gic_decode_beam_workspace_floats.argtypes = [I] * 7
     L.gic_decode_beam.argtypes = [I, P, P, P, P, P, P, P, P, I, I, I, I, I, I, I, C.c_int64, F, P, P, P, P, P, P]
+    L.gic_vocab_target_logp_workspace_floats.restype = Z
+    L.gic_vocab_target_logp_workspace_floats.argtypes = [I] * 2
+    L.gic_vocab_target_logp.argtypes = [I, P, P, P, P, I, I, I, P, P, P, P, P]
+    L.gic_score_captions_workspace_floats.restype = Z
+    L.gic_score_captions_workspace_floats.argtypes = [I] * 6
+    L.gic_score_captions.argtypes = [I, P, P, P, P, P, P, P, P, P, P, I, I, I, I, I, I, P, P, P, P, P]
     for name in header_symbols():      # every declared entry point must be exported
         getattr(L, name)
 

@@ -9,6 +9,9 @@
 //   beam_merge_kernel  per image: the image's K best (parent, token) candidates, scores / frozen flags / lengths, the
 //                      (parent, token) trace, the parents' (h, c) of every layer gathered into the next state, x = embed[tok]
 //   beam_finalize_kernel per image: backtrack, PAD after EOS, sort by score / length^length_penalty
+//   score_rows_kernel  per caption (teacher-forced scoring, K = 1): lse, logp of the row's target, argmax == target, the
+//                      caption's sum of logp.  With targets[M] the producers also write part_tgt[Mpad], the biased logit
+//                      of column targets[m]; only the slice owning that column writes it.
 // Producers:
 //   vocab_topk_kernel  (tensor-core modes) one CTA per (128-row block, vocabulary slice); TMA ring for h and W_out,
 //                      tcgen05.mma kind::tf32 into a double-buffered TMEM accumulator (tile j's epilogue runs under tile
@@ -36,6 +39,8 @@ struct TKArgs {
   const float* bias;
   float2* part_ms;
   float2* part_cand;
+  const int64_t* targets;   // TGT instantiations only
+  float* part_tgt;
 };
 
 __device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
@@ -68,7 +73,7 @@ __device__ __forceinline__ void ms_combine(float& M, float& S, float m, float s)
   else S += s * expf(m - M);
 }
 
-template <int KMAX>
+template <int KMAX, bool TGT>
 __global__ void __launch_bounds__(TK_THREADS, 1)
 vocab_topk_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, TKArgs a) {
   extern __shared__ uint8_t smem_raw[];
@@ -158,6 +163,11 @@ vocab_topk_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
 #pragma unroll
     for (int i = 0; i < KMAX; ++i) { tv[i] = -INFINITY; ti[i] = 0x7fffffff; }
     float m_run = -INFINITY, s_run = 0.f;
+    int tgt = -1;                                // TGT: the row's target column when it is inside [0, N)
+    if (TGT && m < a.M) {
+      const int64_t t64 = a.targets[m];
+      if (t64 >= 0 && t64 < a.N) tgt = (int)t64;
+    }
     for (int j = 0; j < nt; ++j) {
       const int buf = j & 1;
       mbar_wait(&tfull[buf], (j >> 1) & 1);
@@ -192,6 +202,12 @@ vocab_topk_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
             z[4 * k + 0] = z[4 * k + 1] = z[4 * k + 2] = z[4 * k + 3] = -INFINITY;
           }
           cm = fmaxf(cm, fmaxf(fmaxf(z[4 * k + 0], z[4 * k + 1]), fmaxf(z[4 * k + 2], z[4 * k + 3])));
+        }
+        if (TGT && (unsigned)(tgt - nb) < 16u) {   // this thread owns the target column: no other CTA or thread writes it
+          float zt = 0.f;
+#pragma unroll
+          for (int e = 0; e < 16; ++e) zt = (nb + e == tgt) ? z[e] : zt;
+          a.part_tgt[m] = zt;
         }
         if (cm > -INFINITY) {
           const float m_new = fmaxf(m_run, cm);
@@ -253,9 +269,10 @@ vocab_topk_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
 // ---------------------------------------------------------------------------------------------------------
 constexpr int RT_THREADS = 256;
 
-template <int KMAX>
+template <int KMAX, bool TGT>
 __global__ void __launch_bounds__(RT_THREADS)
-row_topk_kernel(const float* __restrict__ logits, int V, int topk, float2* part_ms, float2* part_cand) {
+row_topk_kernel(const float* __restrict__ logits, int V, int topk, float2* part_ms, float2* part_cand,
+                const int64_t* targets, float* part_tgt) {
   using namespace tc;
   __shared__ float2 s_list[RT_THREADS * KMAX];
   __shared__ float2 s_ms[RT_THREADS / 32];
@@ -288,6 +305,10 @@ row_topk_kernel(const float* __restrict__ logits, int V, int topk, float2* part_
     float Mb = -INFINITY, Sb = 0.f;
     for (int i = 0; i < RT_THREADS / 32; ++i) ms_combine(Mb, Sb, s_ms[i].x, s_ms[i].y);
     part_ms[m] = make_float2(Mb, Sb);
+    if (TGT) {
+      const int64_t tg = targets[m];
+      if (tg >= 0 && tg < V) part_tgt[m] = row[tg];
+    }
   }
   // K rounds: every thread offers the head of its list, the block's best is emitted and its owner advances
   int head = 0;
@@ -387,6 +408,51 @@ topk_rows_kernel(const float2* part_ms, const float2* part_cand, int slices, int
   }
 }
 
+// gic_vocab_target_logp / gic_score_captions: block b takes the rows b L .. b L + L - 1 (one warp per row), then sums the
+// caption's logp in increasing t.  Rows t >= lengths[b] (clamped to [0, L]) get logp 0 and correct 0; a target outside
+// [0, V) gets logp NaN.  No atomics: two calls give the same bits.
+constexpr int SR_WARPS = 8;
+__global__ void __launch_bounds__(SR_WARPS * 32)
+score_rows_kernel(const float2* part_ms, const float2* part_cand, const float* part_tgt, int slices, int Mpad, int V,
+                  const int64_t* targets, int L, const int32_t* lengths, float* logp, float* lse_out, int64_t* argmax_out,
+                  uint8_t* correct, float* caption_logp) {
+  const int b = blockIdx.x, lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  const int n = lengths ? min(max(lengths[b], 0), L) : L;
+  for (int t = w; t < L; t += blockDim.x / 32) {
+    const int m = b * L + t;
+    const float lse = row_lse(part_ms, slices, Mpad, m, lane);
+    // argmax: the best of the slices' first candidates (higher logit, then lower column)
+    float bv = -INFINITY;
+    int bc = 0x7fffffff;
+    for (int s = lane; s < slices; s += 32) {
+      const float2 c = part_cand[(size_t)s * Mpad + m];
+      if (tc::cand_before(c.x, __float_as_int(c.y), bv, bc)) { bv = c.x; bc = __float_as_int(c.y); }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      const float ov = __shfl_xor_sync(0xffffffffu, bv, o);
+      const int oc = __shfl_xor_sync(0xffffffffu, bc, o);
+      if (tc::cand_before(ov, oc, bv, bc)) { bv = ov; bc = oc; }
+    }
+    if (lane == 0) {
+      if (bc < 0 || bc >= V) bc = 0;                 // no finite logit in the row: stay in bounds
+      const int64_t tg = targets[m];
+      const bool in = tg >= 0 && tg < V, live = t < n;
+      logp[m] = live ? (in ? part_tgt[m] - lse : __int_as_float(0x7fc00000)) : 0.f;
+      if (lse_out) lse_out[m] = lse;
+      if (argmax_out) argmax_out[m] = bc;
+      if (correct) correct[m] = (live && in && bc == tg) ? 1 : 0;
+    }
+  }
+  if (!caption_logp) return;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    float sum = 0.f;
+    for (int t = 0; t < L; ++t) sum += logp[(size_t)b * L + t];
+    caption_logp[b] = sum;
+  }
+}
+
 constexpr int BEAM_MAX_LAYERS = 8;
 struct BeamState {
   float* hA[BEAM_MAX_LAYERS]; float* cA[BEAM_MAX_LAYERS];       // state the next step reads (gathered by the merge)
@@ -477,6 +543,25 @@ __global__ void beam_init_kernel(const float* features, BeamState st) {
   if (threadIdx.x == 0) { st.score[r] = (k == 0) ? 0.f : -INFINITY; st.fin[r] = 0; st.len[r] = st.L; }
 }
 
+// teacher forcing: x[t][b] = features[b] at t = 0, embed[captions[b, t - 1]] after (an id outside [0, V) feeds row 0, as
+// Decoder.sample's forced_ids do)
+__global__ void teacher_inputs_kernel(const float* features, const int64_t* captions, const float* embed, int B, int L, int E,
+                                      int V, float* x) {
+  const int r = blockIdx.x, t = r / B, b = r - t * B;
+  const float* src = features + (size_t)b * E;
+  if (t > 0) {
+    int64_t id = captions[(size_t)b * L + t - 1];
+    if (id < 0 || id >= V) id = 0;
+    src = embed + (size_t)id * E;
+  }
+  for (int u = threadIdx.x; u < E; u += blockDim.x) x[(size_t)r * E + u] = __ldg(src + u);
+}
+int teacher_inputs(const float* features, const int64_t* captions, const float* embed, int B, int L, int E, int V, float* x,
+                   cudaStream_t s) {
+  teacher_inputs_kernel<<<B * L, 128, 0, s>>>(features, captions, embed, B, L, E, V, x);
+  return check_launch("teacher_inputs_kernel");
+}
+
 // one warp per image: rank by score / length^length_penalty (ties -> lower slot), backtrack the trace
 __global__ void beam_finalize_kernel(BeamState st, float length_penalty, int64_t* ids, float* scores, int32_t* lengths) {
   const int b = blockIdx.x, k = threadIdx.x, K = st.K;
@@ -520,20 +605,22 @@ struct TopkWs {
 };
 size_t vocab_topk_ws_floats(int M, int V, int K) { return TopkWs(M, V, K).total; }
 
-template <int KMAX>
+template <int KMAX, bool TGT = false>
 static int launch_tk(const CUtensorMap& ta, const CUtensorMap& tb, const tc::TKArgs& a, dim3 grid, cudaStream_t s) {
   static bool attr = false;
   if (!attr) {
-    cudaFuncSetAttribute(tc::vocab_topk_kernel<KMAX>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::TK_SMEM);
+    cudaFuncSetAttribute(tc::vocab_topk_kernel<KMAX, TGT>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::TK_SMEM);
     attr = true;
   }
-  tc::vocab_topk_kernel<KMAX><<<grid, tc::TK_THREADS, tc::TK_SMEM, s>>>(ta, tb, a);
+  tc::vocab_topk_kernel<KMAX, TGT><<<grid, tc::TK_THREADS, tc::TK_SMEM, s>>>(ta, tb, a);
   return check_launch("vocab_topk_kernel");
 }
 
 // Per-slice (m, s) and top-K candidates of the rows of h[M, H] W_out^T + b_out into ws; *slices = how many slices.
-int vocab_topk_partials(int mode, const float* h, const float* W_out, const float* b_out, int M, int V, int H, int K,
-                        float* ws, cudaStream_t s, int* slices) {
+// targets[M] (K = 1 only, else NULL): also the logit of column targets[m] into part_tgt[m].
+static int vocab_topk_partials(int mode, const float* h, const float* W_out, const float* b_out, int M, int V, int H, int K,
+                               float* ws, cudaStream_t s, int* slices, const int64_t* targets = nullptr,
+                               float* part_tgt = nullptr) {
   using namespace tc;
   const TopkWs w(M, V, K);
   float2* part_ms = reinterpret_cast<float2*>(ws + w.ms);
@@ -550,9 +637,10 @@ int vocab_topk_partials(int mode, const float* h, const float* W_out, const floa
     if (make_map(&ta, h, M, H, H, BK, BM, rn, false) && make_map(&tb, W_out, V, H, H, BK, TK_BN, rn, false)) {
       TKArgs a;
       a.M = M; a.N = V; a.K = H; a.tiles_n = tiles_n; a.tiles_per_slice = tps; a.Mpad = w.Mpad; a.topk = K;
-      a.bias = b_out; a.part_ms = part_ms; a.part_cand = part_cand;
+      a.bias = b_out; a.part_ms = part_ms; a.part_cand = part_cand; a.targets = targets; a.part_tgt = part_tgt;
       const dim3 grid(ns, tiles_m);
       *slices = ns;
+      if (targets) return launch_tk<1, true>(ta, tb, a, grid, s);
       if (K <= 4) return launch_tk<4>(ta, tb, a, grid, s);
       if (K <= 8) return launch_tk<8>(ta, tb, a, grid, s);
       return launch_tk<16>(ta, tb, a, grid, s);
@@ -561,9 +649,10 @@ int vocab_topk_partials(int mode, const float* h, const float* W_out, const floa
   float* logits = ws + w.logits;
   GIC_TRY(gemm(mode, false, true, M, V, H, 1.f, h, H, W_out, H, 0.f, logits, V, b_out, s, PROF_GEMM_DECODE));
   *slices = 1;
-  if (K <= 4) row_topk_kernel<4><<<M, RT_THREADS, 0, s>>>(logits, V, K, part_ms, part_cand);
-  else if (K <= 8) row_topk_kernel<8><<<M, RT_THREADS, 0, s>>>(logits, V, K, part_ms, part_cand);
-  else row_topk_kernel<16><<<M, RT_THREADS, 0, s>>>(logits, V, K, part_ms, part_cand);
+  if (targets) row_topk_kernel<1, true><<<M, RT_THREADS, 0, s>>>(logits, V, K, part_ms, part_cand, targets, part_tgt);
+  else if (K <= 4) row_topk_kernel<4, false><<<M, RT_THREADS, 0, s>>>(logits, V, K, part_ms, part_cand, nullptr, nullptr);
+  else if (K <= 8) row_topk_kernel<8, false><<<M, RT_THREADS, 0, s>>>(logits, V, K, part_ms, part_cand, nullptr, nullptr);
+  else row_topk_kernel<16, false><<<M, RT_THREADS, 0, s>>>(logits, V, K, part_ms, part_cand, nullptr, nullptr);
   return check_launch("row_topk_kernel");
 }
 
@@ -575,6 +664,27 @@ int vocab_topk(int mode, const float* h, const float* W_out, const float* b_out,
   topk_rows_kernel<<<M, TR_THREADS, 0, s>>>(reinterpret_cast<const float2*>(ws + w.ms), reinterpret_cast<const float2*>(ws + w.cand),
                                             slices, w.Mpad, K, V, logp, tokens, lse);
   return check_launch("topk_rows_kernel");
+}
+
+// workspace of the target-logit producer (floats): the candidate producers' at K = 1 | part_tgt[Mpad]
+struct TargetWs {
+  TopkWs tk;
+  size_t tgt, total;
+  TargetWs(int M, int V) : tk(M, V, 1) { tgt = tk.total; total = tgt + a4((size_t)tk.Mpad); }
+};
+size_t vocab_target_ws_floats(int M, int V) { return TargetWs(M, V).total; }
+
+// Rows m = b L + t of h[M = B L, H] against targets[M] (score_rows_kernel; L = 1 scores independent rows).
+int vocab_target_scores(int mode, const float* h, const float* W_out, const float* b_out, const int64_t* targets, int M, int V,
+                        int H, int L, const int32_t* lengths, float* logp, float* lse, int64_t* argmax, uint8_t* correct,
+                        float* caption_logp, float* ws, cudaStream_t s) {
+  const TargetWs w(M, V);
+  int slices = 1;
+  GIC_TRY(vocab_topk_partials(mode, h, W_out, b_out, M, V, H, 1, ws, s, &slices, targets, ws + w.tgt));
+  score_rows_kernel<<<M / L, 32 * (L < SR_WARPS ? L : SR_WARPS), 0, s>>>(
+      reinterpret_cast<const float2*>(ws + w.tk.ms), reinterpret_cast<const float2*>(ws + w.tk.cand), ws + w.tgt, slices,
+      w.tk.Mpad, V, targets, L, lengths, logp, lse, argmax, correct, caption_logp);
+  return check_launch("score_rows_kernel");
 }
 
 // lstm_cell_fwd / lstm_step_tc live in decode.cu / lstm_tcgen05.cu

@@ -58,6 +58,12 @@ int decode_beam(int mode, const float* features, const float* W_emb, const float
                 const float* const* b_ih, const float* const* b_hh, const float* W_out, const float* b_out, int B, int K,
                 int L, int V, int E, int H, int layers, int64_t eos, float length_penalty, int64_t* ids, float* scores,
                 int32_t* lengths, int32_t* trace, float* ws, cudaStream_t s);
+size_t vocab_target_ws_floats(int M, int V);
+int vocab_target_scores(int mode, const float* h, const float* W_out, const float* b_out, const int64_t* targets, int M, int V,
+                        int H, int L, const int32_t* lengths, float* logp, float* lse, int64_t* argmax, uint8_t* correct,
+                        float* caption_logp, float* ws, cudaStream_t s);
+int teacher_inputs(const float* features, const int64_t* captions, const float* embed, int B, int L, int E, int V, float* x,
+                   cudaStream_t s);
 // disc.cu
 size_t disc_saved_floats(int, int, int, int, int);
 size_t disc_fwd_workspace_floats(int);
@@ -142,6 +148,32 @@ struct DecodeSaved {
   size_t acts(int l) const { return acts0 + (size_t)l * per_layer; }
 };
 
+// One time step of the LSTM stack.  Layer 0 reads x[B,E], layer l > 0 the h that layer l - 1 just wrote.  Tensor-core modes
+// run lstm_step_tc (both contractions + the cell update in one tcgen05 kernel); where it declines, and in exact fp32, two
+// GEMMs into gates[B,4H] and lstm_cell_fwd.  acts may be NULL; the top layer also writes htop[B,L,H] at step t unless NULL.
+struct LstmLayerIO { const float* h_prev; const float* c_prev; float* h_new; float* c_new; float* acts; };
+static int lstm_stack_step(int mode, const float* x, const LstmLayerIO* io, int layers, const float* const* W_ih,
+                           const float* const* W_hh, const float* const* b_ih, const float* const* b_hh, int B, int E, int H,
+                           float* htop, float* gates, int L, int t, cudaStream_t s) {
+  for (int l = 0; l < layers; ++l) {
+    const float* xin = (l == 0) ? x : io[l - 1].h_new;
+    const int In = (l == 0) ? E : H;
+    const LstmLayerIO& y = io[l];
+    float* ht = (l == layers - 1) ? htop : nullptr;
+    bool fused = false;
+    if (mode == GEMM_TF32 || mode == GEMM_BF16)
+      GIC_TRY(lstm_step_tc(xin, In, y.h_prev, W_ih[l], W_hh[l], b_ih[l], b_hh[l], y.c_prev, B, H, y.acts, y.c_new, y.h_new, ht,
+                           L, t, s, &fused));
+    if (!fused) {
+      // gates = x W_ih^T + b_ih + h W_hh^T + b_hh          (src/generator.py:61)
+      GIC_TRY(gemm(mode, false, true, B, 4 * H, In, 1.f, xin, In, W_ih[l], In, 0.f, gates, 4 * H, b_ih[l], s));
+      GIC_TRY(gemm(mode, false, true, B, 4 * H, H, 1.f, y.h_prev, H, W_hh[l], H, 1.f, gates, 4 * H, b_hh[l], s));
+      GIC_TRY(lstm_cell_fwd(gates, y.c_prev, B, H, y.acts, y.c_new, y.h_new, ht, L, t, s));
+    }
+  }
+  return GIC_OK;
+}
+
 // pretrain: 0 = Gumbel-softmax (u[L,B,V], out = soft captions), 1 = pretrain (out = logits, greedy), 2 = inverse-CDF
 // categorical sampling (EXTENSION: u[L,B], out = logits or NULL, logp[B,L] or NULL)
 static int decode_fwd(int mode, const float* features, const float* W_emb, const float* const* W_ih,
@@ -222,26 +254,12 @@ static int decode_fwd(int mode, const float* features, const float* W_emb, const
       GIC_TRY(attn_fwd(at->saved + al.Ak, at->saved + al.Av, q_t, at->w_e, B, at->P, at->Da, E,
                        saved + sv.xs + (size_t)t * BE, at->saved + al.alpha + (size_t)t * B * at->P, s));
     }
-    for (int l = 0; l < layers; ++l) {
-      const float* xin = (l == 0) ? saved + sv.xs + (size_t)t * BE : saved + sv.hs(l - 1) + (size_t)(t + 1) * BH;
-      const int In = (l == 0) ? E : H;
-      const float* hprev = saved + sv.hs(l) + (size_t)t * BH;
-      float* acts_t = saved + sv.acts(l) + (size_t)t * BH * 4;
-      const float* c_prev = saved + sv.cs(l) + (size_t)t * BH;
-      float* c_new = saved + sv.cs(l) + (size_t)(t + 1) * BH;
-      float* h_new = saved + sv.hs(l) + (size_t)(t + 1) * BH;
-      float* htop = (l == layers - 1) ? saved + sv.htop : nullptr;
-      bool fused = false;
-      if (mode == GEMM_TF32 || mode == GEMM_BF16)   // tensor-core modes: both contractions + the cell update in one tcgen05 kernel
-        GIC_TRY(lstm_step_tc(xin, In, hprev, W_ih[l], W_hh[l], b_ih[l], b_hh[l], c_prev, B, H, acts_t, c_new, h_new,
-                             htop, L, t, s, &fused));
-      if (!fused) {
-        // gates = x W_ih^T + b_ih + h W_hh^T + b_hh          (src/generator.py:61)
-        GIC_TRY(gemm(mode, false, true, B, 4 * H, In, 1.f, xin, In, W_ih[l], In, 0.f, gates, 4 * H, b_ih[l], s));
-        GIC_TRY(gemm(mode, false, true, B, 4 * H, H, 1.f, hprev, H, W_hh[l], H, 1.f, gates, 4 * H, b_hh[l], s));
-        GIC_TRY(lstm_cell_fwd(gates, c_prev, B, H, acts_t, c_new, h_new, htop, L, t, s));
-      }
-    }
+    LstmLayerIO io[8];
+    for (int l = 0; l < layers; ++l)
+      io[l] = {saved + sv.hs(l) + (size_t)t * BH, saved + sv.cs(l) + (size_t)t * BH, saved + sv.hs(l) + (size_t)(t + 1) * BH,
+               saved + sv.cs(l) + (size_t)(t + 1) * BH, saved + sv.acts(l) + (size_t)t * BH * 4};
+    GIC_TRY(lstm_stack_step(mode, saved + sv.xs + (size_t)t * BE, io, layers, W_ih, W_hh, b_ih, b_hh, B, E, H, saved + sv.htop,
+                            gates, L, t, s));
     const float* htop_t = saved + sv.hs(layers - 1) + (size_t)(t + 1) * BH;
     float* x_next = (t + 1 < L) ? saved + sv.xs + (size_t)(t + 1) * BE : nullptr;
     if (pretrain == 0 && (mode == GEMM_TF32 || mode == GEMM_BF16)) {
@@ -268,6 +286,50 @@ static int decode_fwd(int mode, const float* features, const float* W_emb, const
     }
   }
   return GIC_OK;
+}
+
+// teacher-forced scoring workspace (floats): x[L][B][E] | per layer: h[2][B][H] (ping-pong), c[B][H] (updated in place)
+// | gates[B][4H] | htop[B][L][H] | target-logit producer
+struct ScoreWs {
+  size_t x, state, per_layer, gates, htop, prod, total;
+  ScoreWs(int B, int L, int V, int E, int H, int layers) {
+    const size_t BH = a4((size_t)B * H);
+    x = 0;
+    state = a4((size_t)L * B * E);
+    per_layer = 3 * BH;
+    gates = state + (size_t)layers * per_layer;
+    htop = gates + a4((size_t)B * 4 * H);
+    prod = htop + a4((size_t)B * L * H);
+    total = prod + vocab_target_ws_floats(B * L, V);
+  }
+};
+
+// Teacher-forced log-likelihood of captions[B,L] (gic_score_captions): the LSTM stack over the forced inputs with the
+// kernels decode_fwd runs (so the hidden states are Decoder.sample(pretrain=True, forced_ids)'s), then ONE projection of
+// all B L rows with the target pick, and one consumer.  No host sync.
+static int score_captions(int mode, const float* features, const int64_t* captions, const int32_t* lengths, const float* W_emb,
+                          const float* const* W_ih, const float* const* W_hh, const float* const* b_ih, const float* const* b_hh,
+                          const float* W_out, const float* b_out, int B, int L, int V, int E, int H, int layers, float* logp,
+                          float* caption_logp, uint8_t* correct, float* ws, cudaStream_t s) {
+  const ScoreWs w(B, L, V, E, H, layers);
+  const size_t BH = a4((size_t)B * H);
+  GIC_TRY(teacher_inputs(features, captions, W_emb, B, L, E, V, ws + w.x, s));
+  for (int l = 0; l < layers; ++l) {
+    float* st = ws + w.state + (size_t)l * w.per_layer;
+    cudaMemsetAsync(st, 0, (size_t)B * H * sizeof(float), s);                    // h of step -1
+    cudaMemsetAsync(st + 2 * BH, 0, (size_t)B * H * sizeof(float), s);          // c
+  }
+  for (int t = 0; t < L; ++t) {
+    LstmLayerIO io[8];
+    for (int l = 0; l < layers; ++l) {
+      float* st = ws + w.state + (size_t)l * w.per_layer;
+      io[l] = {st + (t & 1) * BH, st + 2 * BH, st + ((t + 1) & 1) * BH, st + 2 * BH, nullptr};
+    }
+    GIC_TRY(lstm_stack_step(mode, ws + w.x + (size_t)t * B * E, io, layers, W_ih, W_hh, b_ih, b_hh, B, E, H, ws + w.htop,
+                            ws + w.gates, L, t, s));
+  }
+  return vocab_target_scores(mode, ws + w.htop, W_out, b_out, captions, B * L, V, H, L, lengths, logp, nullptr, nullptr,
+                             correct, caption_logp, ws + w.prod, s);
 }
 
 // backward workspace (floats):
@@ -858,6 +920,35 @@ int gic_decode_beam(int mode, const float* features, const float* W_emb, const f
     GIC_REQUIRE(W_ih[l] && W_hh[l] && b_ih[l] && b_hh[l], GIC_ERR_NULL, "decode_beam: NULL weight of layer %d", l);
   return decode_beam(mode, features, W_emb, W_ih, W_hh, b_ih, b_hh, W_out, b_out, B, K, L, V, E, H, layers, eos_id,
                      length_penalty, ids, scores, lengths, trace, workspace, S(stream));
+}
+
+size_t gic_vocab_target_logp_workspace_floats(int M, int V) { return vocab_target_ws_floats(M, V); }
+int gic_vocab_target_logp(int mode, const float* h, const float* W_out, const float* b_out, const int64_t* targets, int M, int V,
+                          int H, float* logp, float* lse, int64_t* argmax, float* workspace, gic_stream_t stream) {
+  GIC_TRY(require_device());
+  GIC_REQUIRE(M >= 0 && V >= 1 && H >= 1, GIC_ERR_SHAPE, "vocab_target_logp: bad shape M=%d V=%d H=%d", M, V, H);
+  if (M == 0) return GIC_OK;
+  GIC_REQUIRE(h && W_out && b_out && targets && logp && workspace, GIC_ERR_NULL, "vocab_target_logp: NULL pointer");
+  return vocab_target_scores(mode, h, W_out, b_out, targets, M, V, H, 1, nullptr, logp, lse, argmax, nullptr, nullptr,
+                             workspace, S(stream));
+}
+size_t gic_score_captions_workspace_floats(int B, int L, int V, int E, int H, int layers) {
+  return ScoreWs(B, L, V, E, H, layers).total;
+}
+int gic_score_captions(int mode, const float* features, const int64_t* captions, const int32_t* lengths, const float* W_emb,
+                       const float* const* W_ih, const float* const* W_hh, const float* const* b_ih, const float* const* b_hh,
+                       const float* W_out, const float* b_out, int B, int L, int V, int E, int H, int layers, float* logp,
+                       float* caption_logp, uint8_t* correct, float* workspace, gic_stream_t stream) {
+  GIC_TRY(require_device());
+  GIC_REQUIRE(B >= 0 && L >= 1 && V >= 1 && E >= 1 && H >= 1 && layers >= 1 && layers <= 8, GIC_ERR_SHAPE,
+              "score_captions: bad shape B=%d L=%d V=%d E=%d H=%d layers=%d", B, L, V, E, H, layers);
+  if (B == 0) return GIC_OK;
+  GIC_REQUIRE(features && captions && W_emb && W_ih && W_hh && b_ih && b_hh && W_out && b_out && logp && caption_logp &&
+                  workspace, GIC_ERR_NULL, "score_captions: NULL pointer");
+  for (int l = 0; l < layers; ++l)
+    GIC_REQUIRE(W_ih[l] && W_hh[l] && b_ih[l] && b_hh[l], GIC_ERR_NULL, "score_captions: NULL weight of layer %d", l);
+  return score_captions(mode, features, captions, lengths, W_emb, W_ih, W_hh, b_ih, b_hh, W_out, b_out, B, L, V, E, H, layers,
+                        logp, caption_logp, correct, workspace, S(stream));
 }
 
 size_t gic_disc_saved_floats(int N, int L, int De, int R, int F) { return disc_saved_floats(N, L, De, R, F); }

@@ -263,6 +263,39 @@ def decode_beam(dec, features, beam_size, max_caption_len, length_penalty=0.0, e
     return ids, scores, lengths
 
 
+def score_captions(dec, features, captions, lengths=None, mode=None):
+    """gic_score_captions over the decoder's weights -> (logp[B,L], caption_logp[B], correct[B,L] uint8).  No
+    host sync: ids outside [0, V) are not checked here (they give NaN, see Decoder.score)."""
+    _lib.require_cuda()
+    lib = _lib.lib()
+    mode = gic_b200.get_gemm_mode() if mode is None else mode
+    features = _f32c(features)
+    captions = captions.detach().to(features.device).contiguous().long()
+    B, E = features.shape
+    if captions.dim() != 2 or captions.shape[0] != B:
+        raise ValueError("captions must have shape [B, L] with B = %d" % B)
+    L = captions.shape[1]
+    if lengths is not None:
+        lengths = torch.as_tensor(lengths, device=features.device).to(torch.int32).contiguous()
+        if tuple(lengths.shape) != (B,):
+            raise ValueError("lengths must have shape [B] = [%d]" % B)
+    V, H = dec.linear.weight.shape
+    layers = dec.lstm.num_layers
+    dev = features.device
+    lp = [_f32c(w) for w in dec.lstm_params()]
+    W_ih, W_hh, b_ih, b_hh = lp[0::4], lp[1::4], lp[2::4], lp[3::4]
+    W_emb, W_out, b_out = _f32c(dec.embed.weight), _f32c(dec.linear.weight), _f32c(dec.linear.bias)
+    logp = torch.empty(B, L, device=dev)
+    total = torch.empty(B, device=dev)
+    corr = torch.empty(B, L, dtype=torch.uint8, device=dev)
+    ws = torch.empty(lib.gic_score_captions_workspace_floats(B, L, V, E, H, layers), device=dev)
+    _lib.check(lib.gic_score_captions(mode, _lib.ptr(features), _lib.ptr(captions), _lib.ptr(lengths), _lib.ptr(W_emb),
+                                      _lib.ptr_array(W_ih), _lib.ptr_array(W_hh), _lib.ptr_array(b_ih), _lib.ptr_array(b_hh),
+                                      _lib.ptr(W_out), _lib.ptr(b_out), B, L, V, E, H, layers, _lib.ptr(logp),
+                                      _lib.ptr(total), _lib.ptr(corr), _lib.ptr(ws), _lib.stream()), "gic_score_captions")
+    return logp, total, corr
+
+
 class Decoder(nn.Module):
     """LSTM caption decoder (src/generator.py:27-96).  ``embed``/``lstm``/``linear`` are parameter
     containers with the reference's state_dict keys; ``sample`` runs on the B200 kernels."""
@@ -327,6 +360,22 @@ class Decoder(nn.Module):
         if self.attention:
             raise NotImplementedError("beam search is implemented for the plain LSTM decoder, not the attention cell")
         return decode_beam(self, features, beam_size, max_caption_len, length_penalty, eos_id)
+
+    @torch.no_grad()
+    def score(self, features, captions, lengths=None):
+        """Teacher-forced log-likelihood of given captions (EXTENSION; oracle/ref_score.py teacher_forced_logp defines it)
+        -> (logp[B,L], caption_logp[B], correct[B,L] bool).  Step 0's input is features[B,E], as in sample; position t
+        predicts captions[:, t], which is fed to step t + 1.  logp[b, t] = log_softmax(h W_out^T + b_out)[captions[b, t]]
+        for t < lengths[b] (clamped to [0, L]; None: all L positions) and 0 after; caption_logp[b] is their sum; correct
+        marks the positions whose target is the argmax (ties -> lower token, as sample(pretrain=True) picks).  Raises
+        ValueError when an id lies outside [0, V); that check is one host read."""
+        if self.attention:
+            raise NotImplementedError("caption scoring is implemented for the plain LSTM decoder, not the attention cell")
+        V = self.linear.out_features
+        if captions.numel() and bool(((captions < 0) | (captions >= V)).any()):
+            raise ValueError("caption ids must lie in [0, %d)" % V)
+        logp, total, corr = score_captions(self, features, captions, lengths)
+        return logp, total, corr.bool()
 
     def add_gumbel(self, o_t, eps=1e-10, gpu=0):
         """Kept for interface parity (src/generator.py:84-96); the hot path fuses this into the sampler."""

@@ -11,6 +11,7 @@ Data parallel: one process per GPU, each rank owns B/world rows; the only exchan
 (sum) of the flat G and D gradient buffers before the clip (SURVEY.md section 8e)."""
 from __future__ import annotations
 
+import math
 import os
 from typing import Optional
 
@@ -20,7 +21,8 @@ import torch.nn as nn
 import gic_b200
 from . import _lib, parallel
 from .discriminator import Discriminator, disc_fwd_raw
-from .generator import Generator, bn_running_update, encoder_eval
+from .generator import Generator, bn_running_update, encoder_eval, score_captions
+from .tasks import END
 from .utils import get_fixed_temperature, get_losses
 
 
@@ -754,19 +756,71 @@ class GANInstructor:
         Inference only: parameters, gradients, optimizer state, step counters, temperature and the library's random stream
         are left as they were."""
         _lib.require_cuda()
-        dev = self.device
+        dec = self.gen.decoder
+        if not self.cgan and batch_size is None:
+            if pooled is None:
+                raise ValueError("unconditional generation needs batch_size")
+            batch_size = pooled.shape[0]
+        feats = self._start_features(pooled, batch_size)
+        return dec.beam_search(feats, beam_size=beam_size, max_caption_len=max_caption_len, length_penalty=length_penalty)
+
+    def _start_features(self, pooled, batch_size):
+        """Step-0 input of inference: the eval-mode encoder projection of pooled (conditional), or embed.weight[1]."""
         dec = self.gen.decoder
         if self.cgan:
             if pooled is None:
                 raise ValueError("conditional generation needs the pooled image features")
-            feats = encoder_eval(self.gen.encoder, pooled.to(dev).float(), gic_b200.get_gemm_mode())
-        else:
-            if batch_size is None:
-                if pooled is None:
-                    raise ValueError("unconditional generation needs batch_size")
-                batch_size = pooled.shape[0]
-            feats = dec.embed.weight[1].expand(int(batch_size), dec.embed.weight.shape[1]).contiguous()
-        return dec.beam_search(feats, beam_size=beam_size, max_caption_len=max_caption_len, length_penalty=length_penalty)
+            return encoder_eval(self.gen.encoder, pooled.to(self.device).float(), gic_b200.get_gemm_mode())
+        return dec.embed.weight[1].expand(int(batch_size), dec.embed.weight.shape[1]).contiguous()
+
+    # ---- EXTENSION: teacher-forced caption scoring (held-out NLL / perplexity of the generator) ------------------------
+    @_in_ctx
+    @torch.no_grad()
+    def score(self, captions, pooled=None, lengths=None):
+        """Decoder.score of captions[B,L] -> (logp[B,L], caption_logp[B], correct[B,L] bool), from the step-0 input
+        generate uses (eval-mode encoder projection of pooled, or embed.weight[1] when unconditional).  Leaves parameters,
+        gradients, optimizer state, step counters, temperature and the library's random stream as they were."""
+        _lib.require_cuda()
+        captions = captions.to(self.device)
+        feats = self._start_features(pooled, captions.shape[0])
+        return self.gen.decoder.score(feats, captions, lengths)
+
+    @_in_ctx
+    @torch.no_grad()
+    def evaluate_nll(self, batches):
+        """Generator NLL of held-out captions (NLL-gen) over an iterable of (pooled_or_None, captions) or
+        (pooled_or_None, captions, lengths) batches.  Without lengths a caption counts through its first <E>, or all L
+        positions when it has none.  Sums stay on the device; one host read at the end.  Returns dict(nll = -sum logp /
+        tokens, perplexity = exp(nll), token_accuracy = argmax hits / tokens, tokens, captions).  Raises ValueError when an
+        id lies outside [0, V).  Leaves the instructor's state as score does."""
+        _lib.require_cuda()
+        dev = self.device
+        dec = self.gen.decoder
+        if dec.attention:
+            raise NotImplementedError("caption scoring is implemented for the plain LSTM decoder, not the attention cell")
+        V = dec.linear.out_features
+        sums = torch.zeros(4, dtype=torch.float64, device=dev)      # sum logp, tokens, argmax hits, ids outside [0, V)
+        n_captions = 0
+        for batch in batches:
+            pooled, captions = batch[0], batch[1]
+            lengths = batch[2] if len(batch) > 2 else None
+            captions = captions.to(dev).long()
+            B, L = captions.shape
+            if lengths is None:
+                eos = captions == END
+                lengths = torch.where(eos.any(1), eos.int().argmax(1) + 1, torch.full_like(captions[:, 0], L))
+            lengths = torch.as_tensor(lengths, device=dev).to(torch.int32)
+            feats = self._start_features(pooled, B)
+            _, total, corr = score_captions(dec, feats, captions, lengths)
+            sums += torch.stack([total.double().sum(), lengths.clamp(0, L).double().sum(), corr.double().sum(),
+                                 ((captions < 0) | (captions >= V)).double().sum()])
+            n_captions += B
+        lp, tokens, hits, bad = sums.tolist()
+        if bad:
+            raise ValueError("caption ids must lie in [0, %d)" % V)
+        nll = -lp / tokens if tokens else float("nan")
+        return dict(nll=nll, perplexity=math.exp(nll) if tokens else float("nan"),
+                    token_accuracy=hits / tokens if tokens else float("nan"), tokens=int(tokens), captions=n_captions)
 
     # ---- generator pre-training step (src/training.py:53-95; SURVEY.md 8f rank 1) -------------------------------
     @_in_ctx

@@ -273,6 +273,32 @@ int gic_decode_beam(int mode, const float* features, const float* W_emb, const f
                     int32_t* lengths /*[B,K]*/, int32_t* trace /*[L,B,K,2] (parent, token) or NULL*/,
                     float* workspace, gic_stream_t stream);
 
+/* ---- teacher-forced caption scoring (EXTENSION, parity unpinned by reference: oracle/ref_score.py teacher_forced_logp
+ * defines it).
+ * gic_vocab_target_logp: per row of h[M,H], with z = h W_out^T + b_out: logp[m] = z[targets[m]] - logsumexp(z), lse[m] =
+ *   logsumexp(z) and argmax[m] = the column of the largest z (ties -> lower column, the rule of Decoder.sample(pretrain=True)).
+ *   A target outside [0, V) gives logp NaN and is never read.  lse and argmax may be NULL.  Nothing of size V is written in
+ *   the tensor-core modes.  workspace: gic_vocab_target_logp_workspace_floats(M, V).
+ * gic_score_captions: the log-likelihood of given captions under Decoder.sample's LSTM (any number of layers).  Step 0's
+ *   input is features[B,E], h = c = 0; position t predicts captions[b, t], which is step t + 1's input (an id outside [0, V)
+ *   feeds embed row 0, as forced_ids do in gic_decode_sample_fwd).  logp[b, t] = log_softmax(h_top W_out^T + b_out)
+ *   [captions[b, t]] for t < lengths[b], and 0 for t >= lengths[b]; lengths are clamped to [0, L] and NULL means L for every
+ *   caption.  A target outside [0, V) at t < lengths[b] gives NaN.  caption_logp[b] = sum of logp[b, :] in increasing t;
+ *   correct[b, t] (may be NULL) = 1 where t < lengths[b] and captions[b, t] is the argmax (ties -> lower column).  All B L
+ *   positions are projected in one call, no host sync (the call can be captured into a CUDA graph), and two calls give the
+ *   same bits.  workspace: gic_score_captions_workspace_floats(B, L, V, E, H, layers).
+ *   GIC_ERR_SHAPE: L < 1, V, E or H < 1, layers outside 1..8.  B = 0 (M = 0) is a no-op. */
+size_t gic_vocab_target_logp_workspace_floats(int M, int V);
+int gic_vocab_target_logp(int mode, const float* h /*[M,H]*/, const float* W_out, const float* b_out,
+                          const int64_t* targets /*[M]*/, int M, int V, int H, float* logp /*[M]*/,
+                          float* lse /*[M] or NULL*/, int64_t* argmax /*[M] or NULL*/, float* workspace, gic_stream_t stream);
+size_t gic_score_captions_workspace_floats(int B, int L, int V, int E, int H, int layers);
+int gic_score_captions(int mode, const float* features, const int64_t* captions /*[B,L]*/, const int32_t* lengths /*[B] or NULL*/,
+                       const float* W_emb, const float* const* W_ih, const float* const* W_hh, const float* const* b_ih,
+                       const float* const* b_hh, const float* W_out, const float* b_out, int B, int L, int V, int E, int H,
+                       int layers, float* logp /*[B,L]*/, float* caption_logp /*[B]*/, uint8_t* correct /*[B,L] or NULL*/,
+                       float* workspace, gic_stream_t stream);
+
 /* ---- B1 (EXTENSION, parity unpinned by reference): additive attention over the CNN feature grid in the decode step.
  * The reference feeds one pooled vector at step 0 (src/generator.py:19-25,58) and has no attention.  Definition:
  *   once per image: Ak = grid W_k^T [B,P,Da], Av = grid W_v^T [B,P,E];  every step: q = h_{t-1} W_q^T,
