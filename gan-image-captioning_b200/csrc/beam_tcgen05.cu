@@ -588,8 +588,6 @@ __global__ void beam_finalize_kernel(BeamState st, float length_penalty, int64_t
 // ---------------------------------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------------------------------
-static size_t a4(size_t x) { return (x + 3) & ~(size_t)3; }
-
 // workspace of the candidate producers (floats): part_ms | part_cand | logits[M, V] (exact-fp32 / unaligned path)
 struct TopkWs {
   size_t ms, cand, logits, total;

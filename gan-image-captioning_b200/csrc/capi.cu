@@ -42,7 +42,6 @@ int bptt_persistent_tc(float* dG, const float* W_hh, const float* acts, const fl
                        unsigned int* counter, int B, int H, int L, cudaStream_t stream, bool* handled);
 // vocab_sample_tcgen05.cu: fused decode step (projection + sample of step t, recurrent contraction and cell of step t + 1)
 bool decode_step_plan(int B, int V, int H);
-size_t decode_step_scratch_floats(int B, int V, int H);
 int decode_step_tc(const float* hs_t1, const float* W_out, const float* b_out, const float* W_hh, const float* EW, float* R, unsigned int* rec_done, const float* u_t, float T,
                    const float* T_dev, int B, int V, int H, int L, int t, int last, float* out, int64_t* ids,
                    const int64_t* forced, const float* embed, int E, float* x_next, const float* c_prev, float* c_out,
@@ -65,9 +64,6 @@ int vocab_target_scores(int mode, const float* h, const float* W_out, const floa
 int teacher_inputs(const float* features, const int64_t* captions, const float* embed, int B, int L, int E, int V, float* x,
                    cudaStream_t s);
 // disc.cu
-size_t disc_saved_floats(int, int, int, int, int);
-size_t disc_fwd_workspace_floats(int);
-size_t disc_bwd_workspace_floats(int, int, int, int, int);
 int scale_inplace(float*, size_t, float, cudaStream_t);
 // loss_optim.cu
 int gan_loss(int, const float*, const float*, const float*, int, float*, float*, float*, float*, cudaStream_t);
@@ -92,7 +88,6 @@ int pack_captions(const int32_t*, const int32_t*, int, int, int64_t*, int32_t*, 
 const float* temperature_device();
 void disc_set_prepared(const float*);
 int disc_prepare(int, const float*, const float*, const float*, int, const float*, const float*, int, float*, cudaStream_t);
-size_t disc_fwd_workspace_floats(int);
 const char* last_error();
 unsigned long long launch_count();
 unsigned long long kernel_launches(const char*);
@@ -112,8 +107,6 @@ int disc_bwd_entry(int mode, const float* dlogits, const uint8_t* keep, float dr
                    float* ws, float* dW_e, float* const* dcw, float* const* dcb, float* dW_h, float* db_h,
                    float* dW_f, float* db_f, float* dW_o, float* db_o, float* dinp, int want_param, int accumulate,
                    cudaStream_t s);
-
-static size_t a4(size_t x) { return (x + 3) & ~(size_t)3; }
 
 // attention saved layout (floats): Ak[B,P,Da] | Av[B,P,E] | q[L,B,Da] | alpha[L,B,P]
 // attention backward workspace:    dAk[B,P,Da] | dAv[B,P,E] | dq[L,B,Da] | ds[L,B,P]
@@ -174,6 +167,20 @@ static int lstm_stack_step(int mode, const float* x, const LstmLayerIO* io, int 
   return GIC_OK;
 }
 
+// forward workspace of the decode (floats):
+//   gates[B][4H] | logits[B][V] | vs_scratch (fused projection + sampler: barrier counters + row statistics)
+//   | u_slice[B][V] (uniforms of one step: u == NULL, unfused path)
+//   | fused decode step: EW[V][4H] (embed W_ih^T + b_ih + b_hh) | R[B][4H] | rec_done (64 u32 counters) | bsum[4H] (b_ih + b_hh)
+struct DecodeFwdWs {
+  size_t gates, logits, vs_scratch, u_slice, EW, R, rec_done, bsum, total;
+  DecodeFwdWs(int B, int V, int H) {
+    const size_t G4 = (size_t)4 * H;
+    gates = 0; logits = a4(B * G4); vs_scratch = logits + a4((size_t)B * V);
+    u_slice = vs_scratch + a4(vocab_sample_scratch_floats(B, V)); EW = u_slice + a4((size_t)B * V);
+    R = EW + V * G4; rec_done = R + B * G4; bsum = rec_done + 64; total = bsum + G4;
+  }
+};
+
 // pretrain: 0 = Gumbel-softmax (u[L,B,V], out = soft captions), 1 = pretrain (out = logits, greedy), 2 = inverse-CDF
 // categorical sampling (EXTENSION: u[L,B], out = logits or NULL, logp[B,L] or NULL)
 static int decode_fwd(int mode, const float* features, const float* W_emb, const float* const* W_ih,
@@ -190,11 +197,12 @@ static int decode_fwd(int mode, const float* features, const float* W_emb, const
   // pretrain == 0 with u == NULL: the Gumbel uniforms are drawn by the library (Philox state of gic_set_rng; the fused
   // kernel draws its tile on the fly, the separate sampler reads a [B,V] slice filled by the same generator)
   const DecodeSaved sv(B, L, E, H, layers);
+  const DecodeFwdWs w(B, V, H);
   const size_t BH = (size_t)B * H, BE = (size_t)B * E;
-  float* gates = ws;                         // [B,4H]
-  float* logits = ws + a4(4 * BH);           // [B,V]
-  float* vs_scratch = logits + a4((size_t)B * V);   // fused projection + sampler: barrier counters + row statistics
-  float* u_slice = vs_scratch + a4(vocab_sample_scratch_floats(B, V));   // [B,V] uniforms of one step (u == NULL, unfused path)
+  float* gates = ws + w.gates;
+  float* logits = ws + w.logits;
+  float* vs_scratch = ws + w.vs_scratch;
+  float* u_slice = ws + w.u_slice;
   cudaMemcpyAsync(saved + sv.xs, features, BE * sizeof(float), cudaMemcpyDeviceToDevice, s);
   for (int l = 0; l < layers; ++l) {
     cudaMemsetAsync(saved + sv.hs(l), 0, BH * sizeof(float), s);
@@ -216,11 +224,10 @@ static int decode_fwd(int mode, const float* features, const float* W_emb, const
     // it runs as extra tiles of step t's projection / sample launch, and the token-dependent half is a row of
     // EW = embed W_ih^T [V, 4H], rebuilt once per decode (the weights change every optimizer step), added in the cell
     // tail of the CTA that sampled the token.  Step 0 (input = features, h = 0) is the stand-alone LSTM kernel.
-    float* ds = u_slice + a4((size_t)B * V);
-    float* EW = ds;
-    float* R = EW + (size_t)V * 4 * H;
-    unsigned int* rec_done = reinterpret_cast<unsigned int*>(R + (size_t)B * 4 * H);
-    float* bsum = R + (size_t)B * 4 * H + 64;
+    float* EW = ws + w.EW;
+    float* R = ws + w.R;
+    unsigned int* rec_done = reinterpret_cast<unsigned int*>(ws + w.rec_done);
+    float* bsum = ws + w.bsum;
     bool ok0 = false;
     GIC_TRY(lstm_step_tc(saved + sv.xs, E, saved + sv.hs(0), W_ih[0], W_hh[0], b_ih[0], b_hh[0], saved + sv.cs(0), B, H,
                          saved + sv.acts(0), saved + sv.cs(0) + BH, saved + sv.hs(0) + BH, saved + sv.htop, L, 0, s, &ok0));
@@ -797,10 +804,7 @@ int gic_sample_cdf_step(const float* logits, const float* u, int B, int V, int L
 }
 
 size_t gic_decode_saved_floats(int B, int L, int E, int H, int layers) { return DecodeSaved(B, L, E, H, layers).total; }
-size_t gic_decode_fwd_workspace_floats(int B, int V, int H) {
-  return a4((size_t)4 * B * H) + 2 * a4((size_t)B * V) + a4(vocab_sample_scratch_floats(B, V)) +
-         a4(decode_step_scratch_floats(B, V, H));
-}
+size_t gic_decode_fwd_workspace_floats(int B, int V, int H) { return DecodeFwdWs(B, V, H).total; }
 size_t gic_decode_bwd_workspace_floats(int B, int L, int V, int E, int H, int layers) {
   return DecodeBwdWs(B, L, V, E, H, layers).total;
 }
@@ -841,13 +845,7 @@ int gic_decode_sample_bwd_factored(int mode, const float* demb, const float* emb
                     accumulate, S(stream));
 }
 
-size_t gic_disc_bwd_demb_offset_floats(int N, int L, int De, int R, int F) {
-  (void)L; (void)De;
-  const size_t rows = (size_t)N * R;
-  const size_t Fp = (size_t)((F + 63) / 64) * 64;
-  const size_t dh = a4(rows * F) > a4(rows * Fp / 2) ? a4(rows * F) : a4(rows * Fp / 2);
-  return a4((size_t)F + 1) + dh + a4(rows * F) + 2 * a4(F);
-}
+size_t gic_disc_bwd_demb_offset_floats(int N, int L, int De, int R, int F) { return DiscBwdWs(N, L, De, R, F).demb; }
 
 int gic_decode_sample_cdf_fwd(int mode, const float* features, const float* W_emb, const float* const* W_ih,
                               const float* const* W_hh, const float* const* b_ih, const float* const* b_hh,
@@ -951,11 +949,9 @@ int gic_score_captions(int mode, const float* features, const int64_t* captions,
                         logp, caption_logp, correct, workspace, S(stream));
 }
 
-size_t gic_disc_saved_floats(int N, int L, int De, int R, int F) { return disc_saved_floats(N, L, De, R, F); }
-size_t gic_disc_fwd_workspace_floats(int F) { return disc_fwd_workspace_floats(F); }
-size_t gic_disc_bwd_workspace_floats(int N, int L, int De, int R, int F) {
-  return disc_bwd_workspace_floats(N, L, De, R, F);
-}
+size_t gic_disc_saved_floats(int N, int L, int De, int R, int F) { return DiscSaved(N, L, De, R, F).total; }
+size_t gic_disc_fwd_workspace_floats(int F) { return DiscFwdWs(F).total; }
+size_t gic_disc_bwd_workspace_floats(int N, int L, int De, int R, int F) { return DiscBwdWs(N, L, De, R, F).total; }
 
 int gic_disc_fwd(int mode, const float* inp_soft, const int64_t* ids, int N, int L, int V, int De, int R,
                  int n_groups, const int* filter_sizes, const int* num_filters, const float* W_e,
@@ -1008,7 +1004,7 @@ int gic_clip_adam_dyn(float* p, const float* g, float* m, float* v, size_t n, co
 
 void gic_set_temperature_device(const float* t_dev) { set_temperature_device(t_dev); }
 
-size_t gic_disc_prepared_floats(int F) { return disc_fwd_workspace_floats(F); }
+size_t gic_disc_prepared_floats(int F) { return DiscFwdWs(F).total; }
 int gic_disc_prepare(int mode, const float* W_h, const float* W_f, const float* b_f, int Hd, const float* W_o,
                      const float* b_o, int F, float* prepared, gic_stream_t stream) {
   GIC_TRY(require_device());

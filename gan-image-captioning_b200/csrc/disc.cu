@@ -899,30 +899,6 @@ struct DiscDims {
   size_t rows() const { return (size_t)N * R; }
 };
 
-static size_t align4(size_t x) { return (x + 3) & ~(size_t)3; }
-
-// saved-for-backward layout (floats): emb[N*L*De] | pooled[N*R*F] | hpre[N*R*F] | arg(u8)[N*R*F]
-// pitch (elements) of the bf16 copies used by GIC_GEMM_BF16: rows of 128-byte multiples (TMA fetches whole lines)
-static inline int bf_pitch(int F) { return ((F + 63) / 64) * 64; }
-
-// saved-for-backward layout (floats): emb[N*L*De] | pooled[N*R*F] | hpre[N*R*F] | arg(u8)[N*R*F] | pooled_bf(bf16)[N*R*Fp]
-size_t disc_saved_floats(int N, int L, int De, int R, int F) {
-  const size_t rows = (size_t)N * R;
-  return align4((size_t)N * L * De) + 2 * align4(rows * F) + align4((rows * F + 3) / 4) + align4(rows * bf_pitch(F) / 2);
-}
-// forward workspace: weff[F+1]
-// forward workspace: weff[F+1] | W_h_bf(bf16)[F*Fp]
-size_t disc_fwd_workspace_floats(int F) { return align4((size_t)F + 1) + align4((size_t)F * bf_pitch(F) / 2); }
-// backward workspace: weff[F+1] | dh[rows*F] | dx[rows*F] | s[F] | dbh[F] | demb[N*L*De]
-size_t disc_bwd_workspace_floats(int N, int L, int De, int R, int F) {
-  const size_t rows = (size_t)N * R;
-  // weff | dh (fp32 [rows,F], or bf16 [rows,Fp] in GIC_GEMM_BF16 mode) | dx | s | dbh | demb | W_h_bf(bf16)[F*Fp]
-  const size_t dh = align4(rows * F) > align4(rows * bf_pitch(F) / 2) ? align4(rows * F) : align4(rows * bf_pitch(F) / 2);
-  // ... | W_h_bf | dxg[rows*F] (dh W_h, written with beta = 0; the consumers add it to the direct term in dx)
-  return align4((size_t)F + 1) + dh + align4(rows * F) + 2 * align4(F) + align4((size_t)N * L * De) +
-         align4((size_t)F * bf_pitch(F) / 2) + align4(rows * F);
-}
-
 int disc_fill_groups(ConvGroups& g, int ngroups, const int* fs, const int* nf, const float* const* cw,
                      const float* const* cb, float* const* dcw, float* const* dcb, int es) {
   GIC_REQUIRE(ngroups >= 1 && ngroups <= MAX_GROUPS, GIC_ERR_SHAPE, "disc: 1..%d filter groups supported", MAX_GROUPS);
@@ -940,7 +916,7 @@ int disc_fill_groups(ConvGroups& g, int ngroups, const int* fs, const int* nf, c
 }
 
 // Derived weights shared by every discriminator call of one step (collapsed head, bf16 copy of highway.weight):
-// layout = the forward workspace, weff[F+1] | W_h_bf(bf16)[F*Fp].  While a prepared blob is registered the forward /
+// layout = the forward workspace (DiscFwdWs).  While a prepared blob is registered the forward /
 // backward read it instead of recomputing (one adversarial step makes 2 forward and 3 backward calls on the same
 // pre-update weights, SURVEY.md Q1).
 void disc_set_prepared(const float* prep) { ctx().prepared = prep; }
@@ -950,10 +926,11 @@ int disc_prepare(int mode, const float* W_h, const float* W_f, const float* b_f,
                  const float* b_o, int F, float* prep, cudaStream_t s) {
   GIC_REQUIRE(W_h && W_f && b_f && W_o && b_o && prep, GIC_ERR_NULL, "disc_prepare: NULL pointer");
   GIC_REQUIRE(F >= 1 && Hd >= 1, GIC_ERR_SHAPE, "disc_prepare: bad shape");
-  head_collapse_kernel<<<cdiv(F + 1, 32), 256, 0, s>>>(W_f, b_f, W_o, b_o, F, Hd, prep);
+  const DiscFwdWs w(F);
+  head_collapse_kernel<<<cdiv(F + 1, 32), 256, 0, s>>>(W_f, b_f, W_o, b_o, F, Hd, prep + w.weff);
   GIC_TRY(check_launch("head_collapse_kernel"));
   if (mode == GEMM_BF16 && (F % 4 == 0)) {
-    unsigned short* W_h_bf = reinterpret_cast<unsigned short*>(prep + align4((size_t)F + 1));
+    unsigned short* W_h_bf = reinterpret_cast<unsigned short*>(prep + w.W_h_bf);
     GIC_TRY(f32_to_bf16(W_h, F, F, F, W_h_bf, bf_pitch(F), s));
   }
   return GIC_OK;
@@ -964,16 +941,19 @@ int disc_forward(int mode, const float* inp_soft, const int64_t* ids, const Disc
                  const float* W_o, const float* b_o, int n_heads, const uint8_t* const* keep, float drop_p,
                  float* const* logits, float* saved, float* ws, cudaStream_t s) {
   const size_t rows = d.rows();
-  float* emb = saved;
-  float* pooled = emb + align4((size_t)d.N * d.L * d.De);
-  float* hpre = pooled + align4(rows * d.F);
-  uint8_t* arg = reinterpret_cast<uint8_t*>(hpre + align4(rows * d.F));
+  const DiscSaved sv(d.N, d.L, d.De, d.R, d.F);
+  const DiscFwdWs w(d.F);
+  float* emb = saved + sv.emb;
+  float* pooled = saved + sv.pooled;
+  float* hpre = saved + sv.hpre;
+  uint8_t* arg = reinterpret_cast<uint8_t*>(saved + sv.arg);
   const bool bf = (mode == GEMM_BF16) && (d.F % 4 == 0);
   const int Fp = bf_pitch(d.F);
-  unsigned short* pooled_bf = reinterpret_cast<unsigned short*>(reinterpret_cast<float*>(arg) + align4((rows * d.F + 3) / 4));
+  unsigned short* pooled_bf = reinterpret_cast<unsigned short*>(saved + sv.pooled_bf);
   const float* prep = g_prepared;
-  const float* weff = prep ? prep : ws;
-  const unsigned short* W_h_bf = reinterpret_cast<const unsigned short*>(weff + align4((size_t)d.F + 1));
+  const float* derived = prep ? prep : ws;          // the prepared blob has the forward workspace's layout
+  const float* weff = derived + w.weff;
+  const unsigned short* W_h_bf = reinterpret_cast<const unsigned short*>(derived + w.W_h_bf);
   if (d.N == 0) return GIC_OK;
   // 1. embedding
   if (inp_soft) {
@@ -1045,7 +1025,7 @@ int disc_forward(int mode, const float* inp_soft, const int64_t* ids, const Disc
   }
   // 4. collapsed head
   if (!prep) {
-    head_collapse_kernel<<<cdiv(d.F + 1, 32), 256, 0, s>>>(W_f, b_f, W_o, b_o, d.F, d.Hd, ws);
+    head_collapse_kernel<<<cdiv(d.F + 1, 32), 256, 0, s>>>(W_f, b_f, W_o, b_o, d.F, d.Hd, ws + w.weff);
     GIC_TRY(check_launch("head_collapse_kernel"));
   }
   HeadPtrs hp;
@@ -1079,32 +1059,33 @@ int disc_backward(int mode, const float* dlogit, const uint8_t* keep, float drop
                   float* db_o, float* dinp, int want_param, int accumulate, cudaStream_t s) {
   const size_t rows = d.rows();
   if (d.N == 0) return GIC_OK;
-  const float* emb = saved;
-  const float* pooled = emb + align4((size_t)d.N * d.L * d.De);
-  const float* hpre = pooled + align4(rows * d.F);
-  const uint8_t* arg = reinterpret_cast<const uint8_t*>(hpre + align4(rows * d.F));
+  const DiscSaved sv(d.N, d.L, d.De, d.R, d.F);
+  const DiscBwdWs w(d.N, d.L, d.De, d.R, d.F);
+  const DiscFwdWs pw(d.F);                          // layout of the prepared blob
+  const float* emb = saved + sv.emb;
+  const float* pooled = saved + sv.pooled;
+  const float* hpre = saved + sv.hpre;
+  const uint8_t* arg = reinterpret_cast<const uint8_t*>(saved + sv.arg);
   const bool bf = (mode == GEMM_BF16) && (d.F % 4 == 0) && (!keep || (reinterpret_cast<uintptr_t>(keep) & 3u) == 0);
   const int Fp = bf_pitch(d.F);
-  const unsigned short* pooled_bf =
-      reinterpret_cast<const unsigned short*>(reinterpret_cast<const float*>(arg) + align4((rows * d.F + 3) / 4));
+  const unsigned short* pooled_bf = reinterpret_cast<const unsigned short*>(saved + sv.pooled_bf);
   const float* prep = g_prepared;
-  const float* weff = prep ? prep : ws;
-  float* dh = ws + align4((size_t)d.F + 1);
-  const size_t dh_floats = align4(rows * d.F) > align4(rows * Fp / 2) ? align4(rows * d.F) : align4(rows * Fp / 2);
-  float* dx = dh + dh_floats;
-  float* sacc = dx + align4(rows * d.F);
-  float* dbh = sacc + align4(d.F);
-  float* demb = dbh + align4(d.F);
-  unsigned short* W_h_bf_ws = reinterpret_cast<unsigned short*>(demb + align4((size_t)d.N * d.L * d.De));
-  const unsigned short* W_h_bf = prep ? reinterpret_cast<const unsigned short*>(prep + align4((size_t)d.F + 1)) : W_h_bf_ws;
-  float* dxg = reinterpret_cast<float*>(W_h_bf_ws) + align4((size_t)d.F * Fp / 2);
+  const float* weff = prep ? prep + pw.weff : ws + w.weff;
+  float* dh = ws + w.dh;
+  float* dx = ws + w.dx;
+  float* sacc = ws + w.s;
+  float* dbh = ws + w.dbh;
+  float* demb = ws + w.demb;
+  unsigned short* W_h_bf_ws = reinterpret_cast<unsigned short*>(ws + w.W_h_bf);
+  const unsigned short* W_h_bf = prep ? reinterpret_cast<const unsigned short*>(prep + pw.W_h_bf) : W_h_bf_ws;
+  float* dxg = ws + w.dxg;
   const float beta = accumulate ? 1.f : 0.f;
 
   if (!prep) {
-    head_collapse_kernel<<<cdiv(d.F + 1, 32), 256, 0, s>>>(W_f, b_f, W_o, b_o, d.F, d.Hd, ws);
+    head_collapse_kernel<<<cdiv(d.F + 1, 32), 256, 0, s>>>(W_f, b_f, W_o, b_o, d.F, d.Hd, ws + w.weff);
     GIC_TRY(check_launch("head_collapse_kernel"));
   }
-  cudaMemsetAsync(sacc, 0, 2 * align4(d.F) * sizeof(float), s);
+  cudaMemsetAsync(sacc, 0, (w.demb - w.s) * sizeof(float), s);      // s and dbh
   if ((d.F % 4 == 0) && (!keep || (reinterpret_cast<uintptr_t>(keep) & 3u) == 0)) {
     const int colb = cdiv(d.F / 4, 256);
     int per_sm = 3;           // measured (ncu, c2): 3 -> 51 us, 4 -> 55, 6 -> 61, 8 -> 69, 2 -> 52, 1 -> 69

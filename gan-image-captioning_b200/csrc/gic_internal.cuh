@@ -29,6 +29,8 @@ int check_launch(const char* what);
 
 static inline int cdiv(long long a, long long b) { return (int)((a + b - 1) / b); }
 static inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
+// float count rounded up to a multiple of 4: every region of a caller-allocated buffer starts 16-byte aligned
+static inline size_t a4(size_t x) { return (x + 3) & ~(size_t)3; }
 
 int num_sms();
 
@@ -106,6 +108,36 @@ int vocab_sample_tc(const float* htop, int lda, const float* W_out, const float*
 // dz (bf16) = T p (demb W_e - dot) and db_out = colsum(dz) in one streaming tcgen05 kernel (dz_fused_tcgen05.cu)
 int dz_fused_tc(const float* demb, int K, const float* W_e, const float* p, const float* dot, float T, const float* T_dev,
                 int M, int V, void* dz_bf, int Vp, float* db_out, int accumulate, cudaStream_t stream, bool* handled);
+
+// ---- discriminator buffers (disc.cu).  Each struct is the one definition of a buffer's layout: the fields are region
+// offsets in floats, `total` is the size the gic_disc_*_floats queries return.
+// pitch (elements) of the bf16 copies used by GIC_GEMM_BF16: rows of 128-byte multiples (TMA fetches whole lines)
+static inline int bf_pitch(int F) { return ((F + 63) / 64) * 64; }
+// saved for backward: emb[N*L*De] | pooled[N*R*F] | hpre[N*R*F] | arg(u8)[N*R*F] | pooled_bf(bf16)[N*R*Fp]
+struct DiscSaved {
+  size_t emb, pooled, hpre, arg, pooled_bf, total;
+  DiscSaved(int N, int L, int De, int R, int F) {
+    const size_t rows = (size_t)N * R;
+    emb = 0; pooled = a4((size_t)N * L * De); hpre = pooled + a4(rows * F); arg = hpre + a4(rows * F);
+    pooled_bf = arg + a4((rows * F + 3) / 4); total = pooled_bf + a4(rows * bf_pitch(F) / 2);
+  }
+};
+// forward workspace, also the layout of the prepared blob: weff[F+1] (collapsed head) | W_h_bf(bf16)[F*Fp]
+struct DiscFwdWs {
+  size_t weff, W_h_bf, total;
+  explicit DiscFwdWs(int F) { weff = 0; W_h_bf = a4((size_t)F + 1); total = W_h_bf + a4((size_t)F * bf_pitch(F) / 2); }
+};
+// backward workspace: weff[F+1] | dh | dx[rows*F] | s[F] | dbh[F] | demb[N*L*De] | W_h_bf(bf16)[F*Fp] | dxg[rows*F]
+//   dh is fp32 [rows,F], or bf16 [rows,Fp] in GIC_GEMM_BF16 mode; dxg = dh W_h (beta = 0), added to dx by the conv / pool backward
+struct DiscBwdWs {
+  size_t weff, dh, dx, s, dbh, demb, W_h_bf, dxg, total;
+  DiscBwdWs(int N, int L, int De, int R, int F) {
+    const size_t rows = (size_t)N * R, dh_f32 = a4(rows * F), dh_bf16 = a4(rows * bf_pitch(F) / 2);
+    weff = 0; dh = a4((size_t)F + 1); dx = dh + (dh_f32 > dh_bf16 ? dh_f32 : dh_bf16); s = dx + a4(rows * F);
+    dbh = s + a4(F); demb = dbh + a4(F); W_h_bf = demb + a4((size_t)N * L * De);
+    dxg = W_h_bf + a4((size_t)F * bf_pitch(F) / 2); total = dxg + a4(rows * F);
+  }
+};
 
 // out[N] (+)= scale * sum_rows A[M,N]
 int colsum_f32(const float* A, int M, int N, int lda, float scale, bool accumulate, float* out,

@@ -777,21 +777,69 @@ extern "C" void gic_vs_stamps_table(int ncta) {
   }
 }
 
-// scratch (floats) for B rows and V columns: two buffers part[tiles_n][Mpad] float2 (sized for the narrowest tile) that
-// alternate between steps
-static size_t vs_part_floats(int B, int V) {
-  const size_t Mpad = (size_t)cdiv(B, tc::BM) * tc::BM;
-  return 2 * Mpad * (size_t)cdiv(V, 128);
+// Scratch of vocab_sample_kernel (floats): part[0] | part[1] | tokpub | 4 spare.  part[t & 1] holds the (m, s) row
+// statistics of step t, float2 [tiles_n][Mpad] sized for the narrowest tile; the two buffers alternate between steps.
+// tokpub is int2 [Mpad].  [0, zeroed) is cleared before step 0.
+struct VSScratch {
+  size_t part[2], tokpub, zeroed, total;
+  VSScratch(int B, int V) {
+    const size_t Mpad = (size_t)cdiv(B, tc::BM) * tc::BM;
+    part[0] = 0; part[1] = 2 * Mpad * (size_t)cdiv(V, 128);
+    tokpub = 2 * part[1]; zeroed = tokpub + 2 * Mpad; total = zeroed + 4;
+  }
+};
+size_t vocab_sample_scratch_floats(int B, int V) { return VSScratch(B, V).total; }
+
+// Launch of vocab_sample_kernel at column-tile width BN, shared by its two roles (vocab_sample_tc, decode_step_tc): the
+// h / W_out / u / out tensor maps, the VSArgs fields both roles set, the scratch carve-up (zeroed at t == 0) and the
+// BN dispatch.  `a` arrives with the role's rec / cell fields set; tw is the W_hh map of the rec tiles (null in the plain
+// role, which has none: ta is passed in its place).  handled stays false when TMA rejects an operand.
+static int launch_vocab_sample(int BN, const float* h, int lda, const float* W_out, const float* b_out, const float* u_t,
+                               float T, const float* T_dev, int B, int V, int H, int L, int t, float* out, int64_t* ids,
+                               const int64_t* forced, const float* embed, int E, float* x_next, float* scratch,
+                               long long* stamps, const CUtensorMap* tw, tc::VSArgs& a, cudaStream_t stream, bool* handled) {
+  extern RngState rng_state();
+  using namespace tc;
+  const int tiles_m = cdiv(B, BM), tiles_n = cdiv(V, BN);
+  const bool rn = tf32_round_in_tma();
+  CUtensorMap ta, tb, tu, tp;
+  bool ok = make_map(&ta, h, B, H, lda, BK, BM, rn, false) && make_map(&tb, W_out, V, H, H, BK, BN, rn, false) &&
+            make_map(&tu, u_t ? u_t : out, B, V, V, 32, BM, false, false) &&
+            make_map(&tp, out + (size_t)t * V, B, V, L * V, 32, 32, false, false);
+  if (!ok) return GIC_OK;
+  if (!tw) tw = &ta;
+  const VSScratch sc(B, V);
+  a.M = B; a.N = V; a.K = H; a.tiles_n = tiles_n; a.Mpad = tiles_m * BM;
+  a.bias = b_out; a.T = T; a.T_dev = T_dev;
+  a.part = reinterpret_cast<float2*>(scratch + sc.part[t & 1]);
+  a.part_next = reinterpret_cast<float2*>(scratch + sc.part[(t + 1) & 1]);
+  a.ids = ids; a.forced = forced; a.L = L; a.t = t; a.embed = embed; a.E = E; a.x_next = x_next;
+  a.stamps = stamps;
+  a.use_rng = (u_t == nullptr) ? 1 : 0;
+  a.rng = rng_state();
+  a.tokpub = reinterpret_cast<int2*>(scratch + sc.tokpub);
+  if (t == 0) {
+    cudaError_t e = cudaMemsetAsync(scratch, 0, sc.zeroed * sizeof(float), stream);   // statistics "not ready", token tags 0
+    if (e != cudaSuccess) { set_error("vocab_sample memset: %s", cudaGetErrorString(e)); return GIC_ERR_CUDA; }
+  }
+  int rc;
+  const int grid = a.n_rec + tiles_m * tiles_n;
+  switch (BN) {
+    case 128: rc = launch_vs<128>(ta, tb, tu, tp, *tw, a, grid, stream); break;
+    case 160: rc = launch_vs<160>(ta, tb, tu, tp, *tw, a, grid, stream); break;
+    case 192: rc = launch_vs<192>(ta, tb, tu, tp, *tw, a, grid, stream); break;
+    case 224: rc = launch_vs<224>(ta, tb, tu, tp, *tw, a, grid, stream); break;
+    default: rc = launch_vs<256>(ta, tb, tu, tp, *tw, a, grid, stream); break;
+  }
+  if (rc == GIC_OK) *handled = true;
+  return rc;
 }
-static size_t vs_tok_floats(int B) { return 2 * (size_t)cdiv(B, tc::BM) * tc::BM; }
-size_t vocab_sample_scratch_floats(int B, int V) { return 2 * vs_part_floats(B, V) + vs_tok_floats(B) + 4; }
 
 // One fused decode step on the tensor cores.  handled = false (nothing launched) when the shape does not fit the
 // co-resident grid or TMA's alignment rules; the caller then runs the separate projection + sampler kernels.
 int vocab_sample_tc(const float* htop, int lda, const float* W_out, const float* b_out, const float* u_t, float T,
                     const float* T_dev, int B, int V, int H, int L, int t, float* out, int64_t* ids, const int64_t* forced,
                     const float* embed, int E, float* x_next, float* scratch, cudaStream_t stream, bool* handled) {
-  extern RngState rng_state();
   using namespace tc;
   *handled = false;
   if (option("GIC_FUSED_SAMPLE", 1) == 0) return GIC_OK;
@@ -807,42 +855,10 @@ int vocab_sample_tc(const float* htop, int lda, const float* W_out, const float*
   for (int i = 0; kBN[i]; ++i)
     if ((long long)tiles_m * cdiv(V, kBN[i]) <= G) { BN = kBN[i]; break; }
   if (!BN) return GIC_OK;
-  const int tiles_n = cdiv(V, BN);
-  const bool rn = tf32_round_in_tma();
-  CUtensorMap ta, tb, tu, tp;
-  bool ok = make_map(&ta, htop, B, H, lda, BK, BM, rn, false) && make_map(&tb, W_out, V, H, H, BK, BN, rn, false) &&
-            make_map(&tu, u_t ? u_t : out, B, V, V, 32, BM, false, false) &&
-            make_map(&tp, out + (size_t)t * V, B, V, L * V, 32, 32, false, false);
-  if (!ok) return GIC_OK;
-  VSArgs a;
-  a.M = B; a.N = V; a.K = H; a.tiles_n = tiles_n; a.Mpad = tiles_m * BM;
-  a.bias = b_out; a.T = T; a.T_dev = T_dev;
-  const size_t pf = vs_part_floats(B, V);
-  a.part = reinterpret_cast<float2*>(scratch + (size_t)(t & 1) * pf);
-  a.part_next = reinterpret_cast<float2*>(scratch + (size_t)((t + 1) & 1) * pf);
-  a.ids = ids; a.forced = forced; a.L = L; a.t = t; a.embed = embed; a.E = E; a.x_next = x_next;
-  a.stamps = vs_stamps_buffer();
-  a.use_rng = (u_t == nullptr) ? 1 : 0;
-  a.rng = rng_state();
-  a.n_rec = 0; a.rec_tiles_n = 1; a.RBN = 16; a.G4 = 0; a.R = nullptr; a.rec_done = nullptr; a.rec_expect = 0u; a.do_cell = 0;
-  a.EW = nullptr; a.c_prev = nullptr; a.c_out = nullptr; a.h_out = nullptr; a.acts = nullptr;
-  a.htop = nullptr;
-  a.tokpub = reinterpret_cast<int2*>(scratch + 2 * pf);
-  if (t == 0) {
-    cudaError_t e = cudaMemsetAsync(scratch, 0, (2 * pf + vs_tok_floats(B)) * sizeof(float), stream);   // statistics "not ready", token tags 0
-    if (e != cudaSuccess) { set_error("vocab_sample memset: %s", cudaGetErrorString(e)); return GIC_ERR_CUDA; }
-  }
-  int rc;
-  const int grid = tiles_m * tiles_n;
-  switch (BN) {
-    case 128: rc = launch_vs<128>(ta, tb, tu, tp, ta, a, grid, stream); break;
-    case 160: rc = launch_vs<160>(ta, tb, tu, tp, ta, a, grid, stream); break;
-    case 192: rc = launch_vs<192>(ta, tb, tu, tp, ta, a, grid, stream); break;
-    case 224: rc = launch_vs<224>(ta, tb, tu, tp, ta, a, grid, stream); break;
-    default: rc = launch_vs<256>(ta, tb, tu, tp, ta, a, grid, stream); break;
-  }
-  if (rc == GIC_OK) *handled = true;
-  return rc;
+  VSArgs a = {};                // no rec tiles, no cell tail
+  a.rec_tiles_n = 1; a.RBN = 16;
+  return launch_vocab_sample(BN, htop, lda, W_out, b_out, u_t, T, T_dev, B, V, H, L, t, out, ids, forced, embed, E, x_next,
+                             scratch, vs_stamps_buffer(), nullptr, a, stream, handled);
 }
 
 // ---------------------------------------------------------------------------------------------------------
@@ -856,7 +872,7 @@ int vocab_sample_tc(const float* htop, int lda, const float* W_out, const float*
 // decode_step_plan says whether the shape fits (co-resident grid: projection tiles + at least ceil(4H / 256) rec tiles per
 // row block <= SMs); the caller falls back to lstm_step_tc + vocab_sample_tc otherwise.
 // ---------------------------------------------------------------------------------------------------------
-struct DecodeStepPlan { int BN, tiles_m, tiles_n, rec_tiles_n, RBN; };
+struct DecodeStepPlan { int BN, tiles_m, rec_tiles_n, RBN; };
 
 static bool decode_step_plan_impl(int B, int V, int H, DecodeStepPlan* p) {
   using namespace tc;
@@ -873,7 +889,7 @@ static bool decode_step_plan_impl(int B, int V, int H, DecodeStepPlan* p) {
     if (per > G4 / 32) per = G4 / 32;                            // no narrower than 32 columns
     int RBN = ((cdiv(G4, per) + 15) / 16) * 16;
     if (RBN > 256) RBN = 256;
-    p->BN = kBN[i]; p->tiles_m = tiles_m; p->tiles_n = cdiv(V, kBN[i]); p->RBN = RBN; p->rec_tiles_n = cdiv(G4, RBN);
+    p->BN = kBN[i]; p->tiles_m = tiles_m; p->RBN = RBN; p->rec_tiles_n = cdiv(G4, RBN);
     return true;
   }
   return false;
@@ -883,15 +899,10 @@ bool decode_step_plan(int B, int V, int H) {
   DecodeStepPlan p;
   return decode_step_plan_impl(B, V, H, &p);
 }
-size_t decode_step_scratch_floats(int B, int V, int H) {          // EW | R | rec_done counters | b_ih + b_hh
-  return ((size_t)V * 4 * H + (size_t)B * 4 * H + 64 + (size_t)4 * H + 3) & ~(size_t)3;
-}
-
 int decode_step_tc(const float* hs_t1, const float* W_out, const float* b_out, const float* W_hh, const float* EW, float* R, unsigned int* rec_done, const float* u_t, float T,
                    const float* T_dev, int B, int V, int H, int L, int t, int last, float* out, int64_t* ids,
                    const int64_t* forced, const float* embed, int E, float* x_next, const float* c_prev, float* c_out,
                    float* h_out, float* acts, float* htop, float* scratch, cudaStream_t stream, bool* handled) {
-  extern RngState rng_state();
   using namespace tc;
   *handled = false;
   DecodeStepPlan pl;
@@ -900,47 +911,18 @@ int decode_step_tc(const float* hs_t1, const float* W_out, const float* b_out, c
   for (const void* p : ptrs)
     if (!aligned16(p)) return GIC_OK;
   if (((size_t)L * V) % 4) return GIC_OK;
-  const bool rn = tf32_round_in_tma();
-  CUtensorMap ta, tb, tu, tp, tw;
-  bool ok = make_map(&ta, hs_t1, B, H, H, BK, BM, rn, false) && make_map(&tb, W_out, V, H, H, BK, pl.BN, rn, false) &&
-            make_map(&tu, u_t ? u_t : out, B, V, V, 32, BM, false, false) &&
-            make_map(&tp, out + (size_t)t * V, B, V, L * V, 32, 32, false, false) &&
-            make_map(&tw, W_hh, 4 * H, H, H, BK, pl.RBN, rn, false);
-  if (!ok) return GIC_OK;
-  VSArgs a;
-  a.M = B; a.N = V; a.K = H; a.tiles_n = pl.tiles_n; a.Mpad = pl.tiles_m * BM;
-  a.bias = b_out; a.T = T; a.T_dev = T_dev;
-  const size_t pf = vs_part_floats(B, V);
-  a.part = reinterpret_cast<float2*>(scratch + (size_t)(t & 1) * pf);
-  a.part_next = reinterpret_cast<float2*>(scratch + (size_t)((t + 1) & 1) * pf);
-  a.ids = ids; a.forced = forced; a.L = L; a.t = t; a.embed = embed; a.E = E; a.x_next = x_next;
-  a.stamps = nullptr;
-  if (long long* sb = vs_stamps_buffer()) {       // debug timeline of ONE step (GIC_VS_STAMPS=1, GIC_VS_STAMPS_T=t; default L - 2)
-    if (t == option("GIC_VS_STAMPS_T", L - 2)) a.stamps = sb;
-  }
-  a.use_rng = (u_t == nullptr) ? 1 : 0;
-  a.rng = rng_state();
+  CUtensorMap tw;
+  if (!make_map(&tw, W_hh, 4 * H, H, H, BK, pl.RBN, tf32_round_in_tma(), false)) return GIC_OK;
+  VSArgs a = {};
   a.n_rec = last ? 0 : pl.tiles_m * pl.rec_tiles_n;
   a.rec_tiles_n = pl.rec_tiles_n; a.RBN = pl.RBN; a.G4 = 4 * H; a.R = R; a.rec_done = rec_done;
   a.rec_expect = (unsigned int)(t + 1) * (unsigned int)pl.rec_tiles_n;
   a.do_cell = last ? 0 : 1;
   a.EW = EW; a.c_prev = c_prev; a.c_out = c_out; a.h_out = h_out; a.acts = acts; a.htop = htop;
-  a.tokpub = reinterpret_cast<int2*>(scratch + 2 * pf);
-  if (t == 0) {
-    cudaError_t e = cudaMemsetAsync(scratch, 0, (2 * pf + vs_tok_floats(B)) * sizeof(float), stream);   // statistics "not ready", token tags 0
-    if (e != cudaSuccess) { set_error("decode_step memset: %s", cudaGetErrorString(e)); return GIC_ERR_CUDA; }
-  }
-  int rc;
-  const int grid = a.n_rec + pl.tiles_m * pl.tiles_n;
-  switch (pl.BN) {
-    case 128: rc = launch_vs<128>(ta, tb, tu, tp, tw, a, grid, stream); break;
-    case 160: rc = launch_vs<160>(ta, tb, tu, tp, tw, a, grid, stream); break;
-    case 192: rc = launch_vs<192>(ta, tb, tu, tp, tw, a, grid, stream); break;
-    case 224: rc = launch_vs<224>(ta, tb, tu, tp, tw, a, grid, stream); break;
-    default: rc = launch_vs<256>(ta, tb, tu, tp, tw, a, grid, stream); break;
-  }
-  if (rc == GIC_OK) *handled = true;
-  return rc;
+  long long* stamps = vs_stamps_buffer();     // debug timeline of ONE step (GIC_VS_STAMPS=1, GIC_VS_STAMPS_T=t; default L - 2)
+  if (stamps && t != option("GIC_VS_STAMPS_T", L - 2)) stamps = nullptr;
+  return launch_vocab_sample(pl.BN, hs_t1, H, W_out, b_out, u_t, T, T_dev, B, V, H, L, t, out, ids, forced, embed, E, x_next,
+                             scratch, stamps, &tw, a, stream, handled);
 }
 
 }  // namespace gic
