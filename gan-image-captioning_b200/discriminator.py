@@ -17,11 +17,11 @@ def _f32c(t):
 
 
 def disc_weights(disc):
-    """Flat tuple of the discriminator's tensors in the order the C ABI takes them."""
-    cw = [c.weight for c in disc.convs]
-    cb = [c.bias for c in disc.convs]
-    return (disc.embeddings.weight, disc.highway.weight, disc.highway.bias, disc.feature2out.weight,
-            disc.feature2out.bias, disc.out2logits.weight, disc.out2logits.bias, *cw, *cb)
+    """The discriminator's tensors in the order disc_fwd_raw / disc_bwd_raw take them: (W_e, conv weights, conv biases,
+    W_h, b_h, W_f, b_f, W_o, b_o), the conv tensors as per-filter-group lists."""
+    return (disc.embeddings.weight, [c.weight for c in disc.convs], [c.bias for c in disc.convs], disc.highway.weight,
+            disc.highway.bias, disc.feature2out.weight, disc.feature2out.bias, disc.out2logits.weight,
+            disc.out2logits.bias)
 
 
 def disc_fwd_raw(lib, mode, inp_soft, ids, N, L, V, De, R, fsz, nfl, W_e, cw, cb, W_h, b_h, W_f, b_f, W_o, b_o, keeps,
@@ -38,6 +38,20 @@ def disc_fwd_raw(lib, mode, inp_soft, ids, N, L, V, De, R, fsz, nfl, W_e, cw, cb
                                 float(drop_p), _lib.ptr_array(logits), _lib.ptr(saved), _lib.ptr(ws), _lib.stream()),
                "gic_disc_fwd")
     return logits, saved
+
+
+def disc_bwd_raw(mode, dlogits, keep, drop_p, inp_soft, ids, N, L, V, De, R, fsz, nfl, W, saved, ws, dW, dinp, want_param,
+                 accumulate, stream):
+    """gic_disc_bwd of one head.  W: disc_weights() order; dW: gradient outputs in the same structure (written when
+    want_param, added to when accumulate); dinp: d loss / d inp_soft or None."""
+    W_e, cw, cb, W_h, _, W_f, b_f, W_o, b_o = W
+    dW_e, dcw, dcb, dW_h, db_h, dW_f, db_f, dW_o, db_o = dW
+    P, PA = _lib.ptr, _lib.ptr_array
+    _lib.check(_lib.lib().gic_disc_bwd(mode, P(dlogits), P(keep), drop_p, P(inp_soft), P(ids), N, L, V, De, R, len(fsz),
+                                       _lib.int_array(fsz), _lib.int_array(nfl), P(W_e), PA(cw), PA(cb), P(W_h), P(W_f),
+                                       P(b_f), W_f.shape[0], P(W_o), P(b_o), P(saved), P(ws), P(dW_e), PA(dcw), PA(dcb),
+                                       P(dW_h), P(db_h), P(dW_f), P(db_f), P(dW_o), P(db_o), P(dinp), want_param,
+                                       accumulate, stream), "gic_disc_bwd")
 
 
 class _DiscForward(torch.autograd.Function):
@@ -70,33 +84,21 @@ class _DiscForward(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, dlogits):
-        lib = _lib.lib()
         N, L, V, De, R, fsz, nfl, drop_p, mode = ctx.meta
         ng = len(fsz)
-        saved, inp, ids, keep, W_e, W_h, b_h, W_f, b_f, W_o, b_o = ctx.saved_tensors[:11]
-        cw = list(ctx.saved_tensors[11:11 + ng])
-        cb = list(ctx.saved_tensors[11 + ng:11 + 2 * ng])
-        dev = saved.device
-        Fd = sum(nfl)
-        dlogits = _f32c(dlogits)
-        ws = torch.empty(lib.gic_disc_bwd_workspace_floats(N, L, De, R, Fd), device=dev)
+        saved, inp, ids, keep, W_e, *rest = ctx.saved_tensors
+        head, cw, cb = rest[:6], rest[6:6 + ng], rest[6 + ng:]
+        ws = torch.empty(_lib.lib().gic_disc_bwd_workspace_floats(N, L, De, R, sum(nfl)), device=saved.device)
         want_inp = inp is not None and ctx.needs_input_grad[0]
         want_param = any(ctx.needs_input_grad[8:])
-        dW_e, dW_h, db_h = torch.empty_like(W_e), torch.empty_like(W_h), torch.empty_like(b_h)
-        dW_f, db_f, dW_o, db_o = torch.empty_like(W_f), torch.empty_like(b_f), torch.empty_like(W_o), torch.empty_like(b_o)
-        dcw = [torch.empty_like(c) for c in cw]
-        dcb = [torch.empty_like(c) for c in cb]
-        dinp = torch.empty(N, L, V, device=dev) if want_inp else None
-        _lib.check(lib.gic_disc_bwd(mode, _lib.ptr(dlogits), _lib.ptr(keep), drop_p, _lib.ptr(inp), _lib.ptr(ids), N, L,
-                                    V, De, R, ng, _lib.int_array(fsz), _lib.int_array(nfl), _lib.ptr(W_e),
-                                    _lib.ptr_array(cw), _lib.ptr_array(cb), _lib.ptr(W_h), _lib.ptr(W_f), _lib.ptr(b_f),
-                                    W_f.shape[0], _lib.ptr(W_o), _lib.ptr(b_o), _lib.ptr(saved), _lib.ptr(ws),
-                                    _lib.ptr(dW_e), _lib.ptr_array(dcw), _lib.ptr_array(dcb), _lib.ptr(dW_h),
-                                    _lib.ptr(db_h), _lib.ptr(dW_f), _lib.ptr(db_f), _lib.ptr(dW_o), _lib.ptr(db_o),
-                                    _lib.ptr(dinp), int(want_param), 0, _lib.stream()), "gic_disc_bwd")
+        dW = (torch.empty_like(W_e), [torch.empty_like(c) for c in cw], [torch.empty_like(c) for c in cb],
+              *(torch.empty_like(t) for t in head))
+        dinp = torch.empty(N, L, V, device=saved.device) if want_inp else None
+        disc_bwd_raw(mode, _f32c(dlogits), keep, drop_p, inp, ids, N, L, V, De, R, fsz, nfl, (W_e, cw, cb, *head), saved,
+                     ws, dW, dinp, int(want_param), 0, _lib.stream())
         if not want_param:
             return (dinp,) + (None,) * (14 + 2 * ng)
-        return (dinp, None, None, None, None, None, None, None, dW_e, dW_h, db_h, dW_f, db_f, dW_o, db_o, *dcw, *dcb)
+        return (dinp, None, None, None, None, None, None, None, dW[0], *dW[3:], *dW[1], *dW[2])
 
 
 class Discriminator(nn.Module):
@@ -128,10 +130,9 @@ class Discriminator(nn.Module):
             # same behaviour as nn.Dropout in train mode: a fresh Bernoulli(1-p) keep mask per call
             dev = (inp if inp is not None else ids).device
             keep = torch.rand(N * self.num_rep, self.feature_dim, device=dev) >= self.dropout.p
-        w = disc_weights(self)
-        ng = len(self.filter_sizes)
+        W_e, cw, cb, *head = disc_weights(self)
         return _DiscForward.apply(inp, ids, keep, self.dropout.p, gic_b200.get_gemm_mode(), self.filter_sizes,
-                                  self.num_filters, self.num_rep, *w[:7], *w[7:7 + ng], *w[7 + ng:])
+                                  self.num_filters, self.num_rep, W_e, *head, *cw, *cb)
 
     def forward(self, inp, keep=None):
         """Get logits of discriminator.  inp: batch_size * seq_len * vocab_size (soft or one-hot) ->

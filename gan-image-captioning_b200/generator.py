@@ -5,6 +5,7 @@ of ``Decoder.sample`` (the live entry point, src/training.py:71,150) runs in lib
 """
 from __future__ import annotations
 
+import ctypes as C
 import math
 
 import torch
@@ -18,6 +19,84 @@ def _f32c(t: torch.Tensor) -> torch.Tensor:
     return t.detach().contiguous().float()
 
 
+def lstm_split(lstm):
+    """Per-layer lists (W_ih, W_hh, b_ih, b_hh) of a flat list in Decoder.lstm_params() order."""
+    return lstm[0::4], lstm[1::4], lstm[2::4], lstm[3::4]
+
+
+# ---- one binding per compute entry point: each owns its ctypes argument list, allocates nothing, never synchronises ----
+def encoder_fwd_raw(mode, pooled, W, b, gamma, beta, eps, lin, mean, rstd, feats, stream):
+    """gic_encoder_fwd: Encoder.linear + Encoder.bn with the batch statistics; lin / mean / rstd are saved for the backward."""
+    B, Fin = pooled.shape
+    P = _lib.ptr
+    _lib.check(_lib.lib().gic_encoder_fwd(mode, P(pooled), B, Fin, W.shape[0], P(W), P(b), P(gamma), P(beta), eps, P(lin),
+                                          P(mean), P(rstd), P(feats), stream), "gic_encoder_fwd")
+
+
+def encoder_fwd_eval_raw(mode, pooled, W, b, gamma, beta, eps, running_mean, running_var, lin, feats, stream):
+    """gic_encoder_fwd_eval: the same projection with the running statistics; lin is workspace."""
+    B, Fin = pooled.shape
+    P = _lib.ptr
+    _lib.check(_lib.lib().gic_encoder_fwd_eval(mode, P(pooled), B, Fin, W.shape[0], P(W), P(b), P(gamma), P(beta), eps,
+                                               P(running_mean), P(running_var), P(lin), P(feats), stream),
+               "gic_encoder_fwd_eval")
+
+
+def encoder_bwd_raw(mode, dfeats, pooled, lin, mean, rstd, W, gamma, dlin, dW, db, dgamma, dbeta, stream):
+    """gic_encoder_bwd of encoder_fwd_raw: dW / db / dgamma / dbeta overwritten, dlin is workspace."""
+    B, Fin = pooled.shape
+    P = _lib.ptr
+    _lib.check(_lib.lib().gic_encoder_bwd(mode, P(dfeats), P(pooled), P(lin), P(mean), P(rstd), P(W), P(gamma), B, Fin,
+                                          W.shape[0], P(dlin), P(dW), P(db), P(dgamma), P(dbeta), 0, stream),
+               "gic_encoder_bwd")
+
+
+def decode_fwd_raw(mode, features, W_emb, lstm, W_out, b_out, u, temperature, pretrain, forced_ids, out, ids, saved, ws,
+                   stream, attn=None):
+    """gic_decode_sample_fwd (Decoder.sample into out[B,L,V] / ids[B,L]), or gic_decode_sample_fwd_attn when attn is the
+    gic_attn_t of the attention cell (_lib.attn_block).  lstm: Decoder.lstm_params() order."""
+    W_ih, W_hh, b_ih, b_hh = lstm_split(lstm)
+    B, L = ids.shape
+    V, H = W_out.shape
+    P, PA = _lib.ptr, _lib.ptr_array
+    args = (mode, P(features), P(W_emb), PA(W_ih), PA(W_hh), PA(b_ih), PA(b_hh), P(W_out), P(b_out), P(u),
+            float(temperature), int(pretrain), P(forced_ids), B, L, V, W_emb.shape[1], H, len(W_ih), P(out), P(ids),
+            P(saved), P(ws), stream)
+    if attn is None:
+        _lib.check(_lib.lib().gic_decode_sample_fwd(*args), "gic_decode_sample_fwd")
+    else:
+        _lib.check(_lib.lib().gic_decode_sample_fwd_attn(C.byref(attn), *args), "gic_decode_sample_fwd_attn")
+
+
+def decode_bwd_raw(mode, dout, out, fed, W_emb, lstm, W_out, temperature, pretrain, saved, ws, dW_emb, dlstm, dW_out,
+                   db_out, dfeat, stream, factored=None, attn=None):
+    """Backward of decode_fwd_raw; the gradients (dlstm in Decoder.lstm_params() order) are overwritten.  The incoming
+    gradient is dout[B,L,V] (gic_decode_sample_bwd), or factored = (demb, emb, W_e, De) with dout = None
+    (gic_decode_sample_bwd_factored).  attn: the forward's gic_attn_t with its backward workspace and gradients
+    (gic_decode_sample_bwd_attn, either form of the incoming gradient)."""
+    W_ih, W_hh = lstm[0::4], lstm[1::4]
+    dW_ih, dW_hh, db_ih, db_hh = lstm_split(dlstm)
+    B, L = fed.shape
+    V, H = W_out.shape
+    E, layers = W_emb.shape[1], len(W_ih)
+    P, PA = _lib.ptr, _lib.ptr_array
+    grads = (P(saved), P(ws), P(dW_emb), PA(dW_ih), PA(dW_hh), PA(db_ih), PA(db_hh), P(dW_out), P(db_out), P(dfeat))
+    if attn is not None:
+        demb, emb, W_e, De = factored or (None, None, None, 0)
+        _lib.check(_lib.lib().gic_decode_sample_bwd_attn(
+            C.byref(attn), mode, P(dout), P(demb), P(emb), P(W_e), De, P(out), P(fed), P(W_emb), PA(W_ih), PA(W_hh),
+            P(W_out), temperature, int(pretrain), B, L, V, E, H, layers, *grads, stream), "gic_decode_sample_bwd_attn")
+    elif factored is not None:
+        demb, emb, W_e, De = factored
+        _lib.check(_lib.lib().gic_decode_sample_bwd_factored(
+            mode, P(demb), P(emb), P(W_e), De, P(out), P(fed), P(W_emb), PA(W_ih), PA(W_hh), P(W_out), temperature, B, L,
+            V, E, H, layers, *grads, 0, stream), "gic_decode_sample_bwd_factored")
+    else:
+        _lib.check(_lib.lib().gic_decode_sample_bwd(
+            mode, P(dout), P(out), P(fed), P(W_emb), PA(W_ih), PA(W_hh), P(W_out), temperature, int(pretrain), B, L, V, E,
+            H, layers, *grads, 0, stream), "gic_decode_sample_bwd")
+
+
 class _EncoderProject(torch.autograd.Function):
     """Encoder.linear + Encoder.bn, train mode (src/generator.py:23-24)."""
 
@@ -25,15 +104,13 @@ class _EncoderProject(torch.autograd.Function):
     def forward(ctx, pooled, W, b, gamma, beta, eps, mode, running=None):
         _lib.require_cuda()
         pooled, W, b, gamma, beta = map(_f32c, (pooled, W, b, gamma, beta))
-        B, Fin = pooled.shape
+        B = pooled.shape[0]
         E = W.shape[0]
         lin = torch.empty(B, E, device=pooled.device)
         mean = torch.empty(E, device=pooled.device)
         rstd = torch.empty(E, device=pooled.device)
         feats = torch.empty(B, E, device=pooled.device)
-        _lib.check(_lib.lib().gic_encoder_fwd(mode, _lib.ptr(pooled), B, Fin, E, _lib.ptr(W), _lib.ptr(b),
-                                              _lib.ptr(gamma), _lib.ptr(beta), eps, _lib.ptr(lin), _lib.ptr(mean),
-                                              _lib.ptr(rstd), _lib.ptr(feats), _lib.stream()), "gic_encoder_fwd")
+        encoder_fwd_raw(mode, pooled, W, b, gamma, beta, eps, lin, mean, rstd, feats, _lib.stream())
         if running is not None:
             bn_running_update(running, mean, rstd, eps, B)
         ctx.save_for_backward(pooled, W, gamma, lin, mean, rstd)
@@ -43,16 +120,11 @@ class _EncoderProject(torch.autograd.Function):
     @staticmethod
     def backward(ctx, dfeats):
         pooled, W, gamma, lin, mean, rstd = ctx.saved_tensors
-        B, Fin = pooled.shape
-        E = W.shape[0]
         dfeats = _f32c(dfeats)
-        ws = torch.empty(B, E, device=pooled.device)
-        dW, db = torch.empty_like(W), torch.empty(E, device=W.device)
+        ws = torch.empty_like(lin)
+        dW, db = torch.empty_like(W), torch.empty_like(mean)
         dgamma, dbeta = torch.empty_like(db), torch.empty_like(db)
-        _lib.check(_lib.lib().gic_encoder_bwd(ctx.mode, _lib.ptr(dfeats), _lib.ptr(pooled), _lib.ptr(lin),
-                                              _lib.ptr(mean), _lib.ptr(rstd), _lib.ptr(W), _lib.ptr(gamma), B, Fin, E,
-                                              _lib.ptr(ws), _lib.ptr(dW), _lib.ptr(db), _lib.ptr(dgamma),
-                                              _lib.ptr(dbeta), 0, _lib.stream()), "gic_encoder_bwd")
+        encoder_bwd_raw(ctx.mode, dfeats, pooled, lin, mean, rstd, W, gamma, ws, dW, db, dgamma, dbeta, _lib.stream())
         return None, dW, db, dgamma, dbeta, None, None, None
 
 
@@ -73,16 +145,13 @@ def encoder_eval(enc, pooled, mode):
     """Encoder.linear + Encoder.bn with the running statistics (gen.eval(), src/training.py:213-214); forward only."""
     _lib.require_cuda()
     pooled = _f32c(pooled)
-    B, Fin = pooled.shape
+    B = pooled.shape[0]
     E = enc.linear.weight.shape[0]
     lin = torch.empty(B, E, device=pooled.device)
     feats = torch.empty(B, E, device=pooled.device)
     bn = enc.bn
-    _lib.check(_lib.lib().gic_encoder_fwd_eval(mode, _lib.ptr(pooled), B, Fin, E, _lib.ptr(_f32c(enc.linear.weight)),
-                                               _lib.ptr(_f32c(enc.linear.bias)), _lib.ptr(_f32c(bn.weight)),
-                                               _lib.ptr(_f32c(bn.bias)), bn.eps, _lib.ptr(bn.running_mean),
-                                               _lib.ptr(bn.running_var), _lib.ptr(lin), _lib.ptr(feats), _lib.stream()),
-               "gic_encoder_fwd_eval")
+    encoder_fwd_eval_raw(mode, pooled, _f32c(enc.linear.weight), _f32c(enc.linear.bias), _f32c(bn.weight), _f32c(bn.bias),
+                         bn.eps, bn.running_mean, bn.running_var, lin, feats, _lib.stream())
     return feats
 
 
@@ -112,17 +181,17 @@ class Encoder(nn.Module):
 
 
 class _DecodeSample(torch.autograd.Function):
-    """Decoder.sample forward/backward through gic_decode_sample_{fwd,bwd}."""
+    """Decoder.sample forward/backward through decode_fwd_raw / decode_bwd_raw."""
 
     @staticmethod
-    def forward(ctx, features, u, temperature, pretrain, L, forced_ids, mode, layers, W_emb, W_out, b_out, *lstm):
+    def forward(ctx, features, u, temperature, pretrain, L, forced_ids, mode, W_emb, W_out, b_out, *lstm):
         _lib.require_cuda()
         lib = _lib.lib()
         dev = features.device
         features = _f32c(features)
         W_emb, W_out, b_out = map(_f32c, (W_emb, W_out, b_out))
         lstm = [_f32c(w) for w in lstm]
-        W_ih, W_hh, b_ih, b_hh = (lstm[i::4] for i in range(4))
+        layers = len(lstm) // 4
         B, E = features.shape
         V, H = W_out.shape
         if u is not None:
@@ -135,58 +204,42 @@ class _DecodeSample(torch.autograd.Function):
         ids = torch.empty(B, L, dtype=torch.int64, device=dev)
         saved = torch.empty(lib.gic_decode_saved_floats(B, L, E, H, layers), device=dev)
         ws = torch.empty(lib.gic_decode_fwd_workspace_floats(B, V, H), device=dev)
-        _lib.check(lib.gic_decode_sample_fwd(
-            mode, _lib.ptr(features), _lib.ptr(W_emb), _lib.ptr_array(W_ih), _lib.ptr_array(W_hh),
-            _lib.ptr_array(b_ih), _lib.ptr_array(b_hh), _lib.ptr(W_out), _lib.ptr(b_out), _lib.ptr(u),
-            float(temperature), int(bool(pretrain)), _lib.ptr(forced_ids), B, L, V, E, H, layers, _lib.ptr(out),
-            _lib.ptr(ids), _lib.ptr(saved), _lib.ptr(ws), _lib.stream()), "gic_decode_sample_fwd")
+        decode_fwd_raw(mode, features, W_emb, lstm, W_out, b_out, u, temperature, pretrain, forced_ids, out, ids, saved, ws,
+                       _lib.stream())
         fed = ids if forced_ids is None else forced_ids
-        ctx.save_for_backward(out, fed, saved, W_emb, W_out, *W_ih, *W_hh)
-        ctx.dims = (B, L, V, E, H, layers, float(temperature), bool(pretrain), mode)
+        ctx.save_for_backward(out, fed, saved, W_emb, W_out, *lstm)
+        ctx.meta = (float(temperature), bool(pretrain), mode)
         ctx.mark_non_differentiable(ids)
         return out, ids
 
     @staticmethod
     def backward(ctx, dout, _dids):
-        lib = _lib.lib()
-        B, L, V, E, H, layers, T, pretrain, mode = ctx.dims
-        out, fed, saved, W_emb, W_out = ctx.saved_tensors[:5]
-        W_ih = ctx.saved_tensors[5:5 + layers]
-        W_hh = ctx.saved_tensors[5 + layers:5 + 2 * layers]
+        T, pretrain, mode = ctx.meta
+        out, fed, saved, W_emb, W_out, *lstm = ctx.saved_tensors
+        B, L, V = out.shape
+        E, H = W_emb.shape[1], W_out.shape[1]
         dev = out.device
-        dout = _f32c(dout)
-        ws = torch.empty(lib.gic_decode_bwd_workspace_floats(B, L, V, E, H, layers), device=dev)
+        ws = torch.empty(_lib.lib().gic_decode_bwd_workspace_floats(B, L, V, E, H, len(lstm) // 4), device=dev)
         dW_emb, dW_out = torch.empty_like(W_emb), torch.empty_like(W_out)
         db_out = torch.empty(V, device=dev)
-        dW_ih = [torch.empty_like(w) for w in W_ih]
-        dW_hh = [torch.empty_like(w) for w in W_hh]
-        db_ih = [torch.empty(4 * H, device=dev) for _ in range(layers)]
-        db_hh = [torch.empty(4 * H, device=dev) for _ in range(layers)]
+        dlstm = [torch.empty_like(w) for w in lstm]
         dfeat = torch.empty(B, E, device=dev)
-        _lib.check(lib.gic_decode_sample_bwd(
-            mode, _lib.ptr(dout), _lib.ptr(out), _lib.ptr(fed), _lib.ptr(W_emb), _lib.ptr_array(W_ih),
-            _lib.ptr_array(W_hh), _lib.ptr(W_out), T, int(pretrain), B, L, V, E, H, layers, _lib.ptr(saved),
-            _lib.ptr(ws), _lib.ptr(dW_emb), _lib.ptr_array(dW_ih), _lib.ptr_array(dW_hh), _lib.ptr_array(db_ih),
-            _lib.ptr_array(db_hh), _lib.ptr(dW_out), _lib.ptr(db_out), _lib.ptr(dfeat), 0, _lib.stream()),
-            "gic_decode_sample_bwd")
-        lstm_grads = []
-        for l in range(layers):
-            lstm_grads += [dW_ih[l], dW_hh[l], db_ih[l], db_hh[l]]
-        return (dfeat, None, None, None, None, None, None, None, dW_emb, dW_out, db_out, *lstm_grads)
+        decode_bwd_raw(mode, _f32c(dout), out, fed, W_emb, lstm, W_out, T, pretrain, saved, ws, dW_emb, dlstm, dW_out,
+                       db_out, dfeat, _lib.stream())
+        return (dfeat, None, None, None, None, None, None, dW_emb, dW_out, db_out, *dlstm)
 
 
 class _DecodeSampleAttn(torch.autograd.Function):
-    """Decoder.sample with the attention cell (EXTENSION, SURVEY.md 8a row B1) through gic_decode_sample_{fwd,bwd}_attn."""
+    """Decoder.sample with the attention cell (EXTENSION, SURVEY.md 8a row B1) through decode_fwd_raw / decode_bwd_raw."""
 
     @staticmethod
-    def forward(ctx, features, grid, u, temperature, L, forced_ids, mode, W_k, W_v, W_q, w_e, W_emb, W_out, b_out, W_ih,
-                W_hh, b_ih, b_hh):
+    def forward(ctx, features, grid, u, temperature, L, forced_ids, mode, W_k, W_v, W_q, w_e, W_emb, W_out, b_out, *lstm):
         _lib.require_cuda()
         lib = _lib.lib()
         dev = features.device
         features, grid, u = _f32c(features), _f32c(grid), _f32c(u)
-        W_k, W_v, W_q, w_e, W_emb, W_out, b_out, W_ih, W_hh, b_ih, b_hh = map(
-            _f32c, (W_k, W_v, W_q, w_e, W_emb, W_out, b_out, W_ih, W_hh, b_ih, b_hh))
+        W_k, W_v, W_q, w_e, W_emb, W_out, b_out = map(_f32c, (W_k, W_v, W_q, w_e, W_emb, W_out, b_out))
+        lstm = [_f32c(w) for w in lstm]
         B, E = features.shape
         V, H = W_out.shape
         Pn, Da = grid.shape[1], W_k.shape[0]
@@ -198,43 +251,34 @@ class _DecodeSampleAttn(torch.autograd.Function):
         asaved = torch.empty(lib.gic_attn_saved_floats(B, L, Pn, Da, E), device=dev)
         ws = torch.empty(lib.gic_decode_fwd_workspace_floats(B, V, H), device=dev)
         blk = _lib.attn_block(grid, W_k, W_v, W_q, w_e.reshape(-1), asaved)
-        import ctypes as C
-        _lib.check(lib.gic_decode_sample_fwd_attn(
-            C.byref(blk), mode, _lib.ptr(features), _lib.ptr(W_emb), _lib.ptr_array([W_ih]), _lib.ptr_array([W_hh]),
-            _lib.ptr_array([b_ih]), _lib.ptr_array([b_hh]), _lib.ptr(W_out), _lib.ptr(b_out), _lib.ptr(u),
-            float(temperature), 0, _lib.ptr(forced_ids), B, L, V, E, H, 1, _lib.ptr(out), _lib.ptr(ids), _lib.ptr(saved),
-            _lib.ptr(ws), _lib.stream()), "gic_decode_sample_fwd_attn")
+        decode_fwd_raw(mode, features, W_emb, lstm, W_out, b_out, u, temperature, 0, forced_ids, out, ids, saved, ws,
+                       _lib.stream(), attn=blk)
         fed = ids if forced_ids is None else forced_ids
-        ctx.save_for_backward(out, fed, saved, asaved, grid, W_k, W_v, W_q, w_e, W_emb, W_out, W_ih, W_hh)
-        ctx.dims = (B, L, V, E, H, Pn, Da, float(temperature), mode)
+        ctx.save_for_backward(out, fed, saved, asaved, grid, W_k, W_v, W_q, w_e, W_emb, W_out, *lstm)
+        ctx.meta = (float(temperature), mode)
         ctx.mark_non_differentiable(ids)
         return out, ids
 
     @staticmethod
     def backward(ctx, dout, _dids):
-        import ctypes as C
-        lib = _lib.lib()
-        B, L, V, E, H, Pn, Da, T, mode = ctx.dims
-        out, fed, saved, asaved, grid, W_k, W_v, W_q, w_e, W_emb, W_out, W_ih, W_hh = ctx.saved_tensors
+        T, mode = ctx.meta
+        out, fed, saved, asaved, grid, W_k, W_v, W_q, w_e, W_emb, W_out, *lstm = ctx.saved_tensors
+        B, L, V = out.shape
+        E, H = W_emb.shape[1], W_out.shape[1]
+        Pn, Da = grid.shape[1], W_k.shape[0]
         dev = out.device
-        dout = _f32c(dout)
+        lib = _lib.lib()
         ws = torch.empty(lib.gic_decode_bwd_workspace_floats(B, L, V, E, H, 1), device=dev)
         aws = torch.empty(lib.gic_attn_bwd_workspace_floats(B, L, Pn, Da, E), device=dev)
         dW_k, dW_v, dW_q, dw_e = (torch.empty_like(t) for t in (W_k, W_v, W_q, w_e))
         dW_emb, dW_out = torch.empty_like(W_emb), torch.empty_like(W_out)
         db_out = torch.empty(V, device=dev)
-        dW_ih, dW_hh = torch.empty_like(W_ih), torch.empty_like(W_hh)
-        db_ih, db_hh = torch.empty(4 * H, device=dev), torch.empty(4 * H, device=dev)
+        dlstm = [torch.empty_like(w) for w in lstm]
         dfeat = torch.empty(B, E, device=dev)
         blk = _lib.attn_block(grid, W_k, W_v, W_q, w_e.reshape(-1), asaved, aws, dW_k, dW_v, dW_q, dw_e)
-        _lib.check(lib.gic_decode_sample_bwd_attn(
-            C.byref(blk), mode, _lib.ptr(dout), None, None, None, 0, _lib.ptr(out), _lib.ptr(fed), _lib.ptr(W_emb),
-            _lib.ptr_array([W_ih]), _lib.ptr_array([W_hh]), _lib.ptr(W_out), T, 0, B, L, V, E, H, 1, _lib.ptr(saved),
-            _lib.ptr(ws), _lib.ptr(dW_emb), _lib.ptr_array([dW_ih]), _lib.ptr_array([dW_hh]), _lib.ptr_array([db_ih]),
-            _lib.ptr_array([db_hh]), _lib.ptr(dW_out), _lib.ptr(db_out), _lib.ptr(dfeat), _lib.stream()),
-            "gic_decode_sample_bwd_attn")
-        return (dfeat, None, None, None, None, None, None, dW_k, dW_v, dW_q, dw_e, dW_emb, dW_out, db_out, dW_ih, dW_hh,
-                db_ih, db_hh)
+        decode_bwd_raw(mode, _f32c(dout), out, fed, W_emb, lstm, W_out, T, 0, saved, ws, dW_emb, dlstm, dW_out, db_out,
+                       dfeat, _lib.stream(), attn=blk)
+        return (dfeat, None, None, None, None, None, None, dW_k, dW_v, dW_q, dw_e, dW_emb, dW_out, db_out, *dlstm)
 
 
 def decode_beam(dec, features, beam_size, max_caption_len, length_penalty=0.0, eos_id=2, mode=None, trace=None):
@@ -249,8 +293,7 @@ def decode_beam(dec, features, beam_size, max_caption_len, length_penalty=0.0, e
     V, H = dec.linear.weight.shape
     layers = dec.lstm.num_layers
     dev = features.device
-    lp = [_f32c(w) for w in dec.lstm_params()]
-    W_ih, W_hh, b_ih, b_hh = lp[0::4], lp[1::4], lp[2::4], lp[3::4]
+    W_ih, W_hh, b_ih, b_hh = lstm_split([_f32c(w) for w in dec.lstm_params()])
     W_emb, W_out, b_out = _f32c(dec.embed.weight), _f32c(dec.linear.weight), _f32c(dec.linear.bias)
     ids = torch.empty(B, K, L, dtype=torch.int64, device=dev)
     scores = torch.empty(B, K, device=dev)
@@ -282,8 +325,7 @@ def score_captions(dec, features, captions, lengths=None, mode=None):
     V, H = dec.linear.weight.shape
     layers = dec.lstm.num_layers
     dev = features.device
-    lp = [_f32c(w) for w in dec.lstm_params()]
-    W_ih, W_hh, b_ih, b_hh = lp[0::4], lp[1::4], lp[2::4], lp[3::4]
+    W_ih, W_hh, b_ih, b_hh = lstm_split([_f32c(w) for w in dec.lstm_params()])
     W_emb, W_out, b_out = _f32c(dec.embed.weight), _f32c(dec.linear.weight), _f32c(dec.linear.bias)
     logp = torch.empty(B, L, device=dev)
     total = torch.empty(B, device=dev)
@@ -348,8 +390,8 @@ class Decoder(nn.Module):
                                            gic_b200.get_gemm_mode(), *self.attn_params(), self.embed.weight,
                                            self.linear.weight, self.linear.bias, *self.lstm_params())
         return _DecodeSample.apply(features, u, float(self.temperature), bool(pretrain), L, forced_ids,
-                                   gic_b200.get_gemm_mode(), self.lstm.num_layers, self.embed.weight,
-                                   self.linear.weight, self.linear.bias, *self.lstm_params())
+                                   gic_b200.get_gemm_mode(), self.embed.weight, self.linear.weight, self.linear.bias,
+                                   *self.lstm_params())
 
     @torch.no_grad()
     def beam_search(self, features, beam_size=3, max_caption_len=34, length_penalty=0.0, eos_id=2):

@@ -20,10 +20,11 @@ import torch.nn as nn
 
 import gic_b200
 from . import _lib, parallel
-from .discriminator import Discriminator, disc_fwd_raw
-from .generator import Generator, bn_running_update, encoder_eval, score_captions
+from .discriminator import Discriminator, disc_bwd_raw, disc_fwd_raw, disc_weights
+from .generator import (Generator, bn_running_update, decode_bwd_raw, decode_fwd_raw, encoder_bwd_raw, encoder_eval,
+                        encoder_fwd_eval_raw, encoder_fwd_raw, lstm_split, score_captions)
 from .tasks import END
-from .utils import get_fixed_temperature, get_losses
+from .utils import gan_loss_raw, get_fixed_temperature, get_losses
 
 
 def _in_ctx(fn):
@@ -70,6 +71,11 @@ class FlatParams:
 
     def homed(self):
         return all(p.data_ptr() == self.flat.data_ptr() + 4 * o for p, o in zip(self.params, self.offsets))
+
+
+def _grad_views(fp, weights):
+    """fp.g of every tensor of a disc_weights()-style tuple, in the same structure (lists stay lists)."""
+    return tuple([fp.g(t) for t in w] if isinstance(w, list) else fp.g(w) for w in weights)
 
 
 class GANInstructor:
@@ -239,49 +245,62 @@ class GANInstructor:
     def _sync_bn_on(self):
         return self.sync_bn and self.world > 1
 
-    def _encoder_fwd(self, mode, pooled, B, Fin, E, lin, mean, rstd, feats, stream):
+    def _features_fwd(self, mode, pooled, B, stream):
+        """Step-0 input of a training step (src/training.py:144-147) -> (feats[B,E], enc).  Conditional: the encoder
+        projection of pooled, enc = (pooled, lin, mean, rstd) for _features_bwd.  Unconditional: embed(<S>) for every
+        row, enc = None."""
+        E = self.args.gen_embed_dim
+        if not self.cgan:
+            return self.gen.decoder.embed.weight[1].expand(B, E).contiguous(), None
         lib, P, enc = _lib.lib(), _lib.ptr, self.gen.encoder
+        W, b, bn = enc.linear.weight, enc.linear.bias, enc.bn
+        if pooled.dim() != 2 or pooled.shape[1] != enc.feature_dim:
+            raise ValueError("the encoder expects pooled CNN features [B, %d]" % enc.feature_dim)
+        pooled = pooled.to(self.device).float().contiguous()
+        lin, mean, rstd = self._buf("enc_lin", B * E).view(B, E), self._buf("enc_mean", E), self._buf("enc_rstd", E)
+        feats = self._buf("feats", B * E).view(B, E)
         if not enc.training:
             # gen.eval() (the reference's validation loops, src/training.py:213-215): running statistics, row-local
-            _lib.check(lib.gic_encoder_fwd_eval(mode, P(pooled), B, Fin, E, P(enc.linear.weight), P(enc.linear.bias),
-                                                P(enc.bn.weight), P(enc.bn.bias), enc.bn.eps, P(enc.bn.running_mean),
-                                                P(enc.bn.running_var), P(lin), P(feats), stream), "gic_encoder_fwd_eval")
-            return
-        if not self._sync_bn_on():
-            _lib.check(lib.gic_encoder_fwd(mode, P(pooled), B, Fin, E, P(enc.linear.weight), P(enc.linear.bias),
-                                           P(enc.bn.weight), P(enc.bn.bias), enc.bn.eps, P(lin), P(mean), P(rstd),
-                                           P(feats), stream), "gic_encoder_fwd")
-            bn_running_update(enc.bn, mean, rstd, enc.bn.eps, B)
-            return
-        # SyncBN: local sums -> all-reduce of [2, E] -> normalise with the global-batch statistics (SURVEY.md 8e)
-        stats = self._buf("enc_stats", 2 * E)
-        _lib.check(lib.gic_encoder_fwd_stats(mode, P(pooled), B, Fin, E, P(enc.linear.weight), P(enc.linear.bias), P(lin),
-                                             P(stats), stream), "gic_encoder_fwd_stats")
-        parallel.allreduce_sum_(stats)
-        _lib.check(lib.gic_encoder_fwd_apply(P(lin), B, E, P(enc.bn.weight), P(enc.bn.bias), enc.bn.eps, P(stats),
-                                             float(B * self.world), P(mean), P(rstd), P(feats), stream), "gic_encoder_fwd_apply")
-        bn_running_update(enc.bn, mean, rstd, enc.bn.eps, B * self.world)
+            encoder_fwd_eval_raw(mode, pooled, W, b, bn.weight, bn.bias, bn.eps, bn.running_mean, bn.running_var, lin,
+                                 feats, stream)
+        elif not self._sync_bn_on():
+            encoder_fwd_raw(mode, pooled, W, b, bn.weight, bn.bias, bn.eps, lin, mean, rstd, feats, stream)
+            bn_running_update(bn, mean, rstd, bn.eps, B)
+        else:
+            # SyncBN: local sums -> all-reduce of [2, E] -> normalise with the global-batch statistics (SURVEY.md 8e)
+            stats = self._buf("enc_stats", 2 * E)
+            _lib.check(lib.gic_encoder_fwd_stats(mode, P(pooled), B, pooled.shape[1], E, P(W), P(b), P(lin), P(stats),
+                                                 stream), "gic_encoder_fwd_stats")
+            parallel.allreduce_sum_(stats)
+            _lib.check(lib.gic_encoder_fwd_apply(P(lin), B, E, P(bn.weight), P(bn.bias), bn.eps, P(stats),
+                                                 float(B * self.world), P(mean), P(rstd), P(feats), stream),
+                       "gic_encoder_fwd_apply")
+            bn_running_update(bn, mean, rstd, bn.eps, B * self.world)
+        return feats, (pooled, lin, mean, rstd)
 
-    def _encoder_bwd(self, mode, dfeat, pooled, lin, mean, rstd, B, E, stream):
-        lib, P, enc = _lib.lib(), _lib.ptr, self.gen.encoder
-        if not enc.training:
+    def _features_bwd(self, mode, dfeat, enc, stream):
+        """Gradients of the step-0 input (enc from _features_fwd) into the flat generator gradient."""
+        gg = self._flat_g.g
+        if enc is None:
+            gg(self.gen.decoder.embed.weight)[1] += dfeat.sum(0)      # features = embed(<S>) for every row (:147)
+            return
+        lib, P, e = _lib.lib(), _lib.ptr, self.gen.encoder
+        if not e.training:
             raise NotImplementedError("training step with the encoder in eval mode: call gen.train() (the reference trains "
                                       "with gen.train(), src/training.py:215)")
-        gg = self._flat_g.g
+        pooled, lin, mean, rstd = enc
+        B, E = lin.shape
         dlin = self._buf("enc_dlin", B * E)
+        grads = (gg(e.linear.weight), gg(e.linear.bias), gg(e.bn.weight), gg(e.bn.bias))
         if not self._sync_bn_on():
-            _lib.check(lib.gic_encoder_bwd(mode, P(dfeat), P(pooled), P(lin), P(mean), P(rstd), P(enc.linear.weight),
-                                           P(enc.bn.weight), B, pooled.shape[1], E, P(dlin), P(gg(enc.linear.weight)),
-                                           P(gg(enc.linear.bias)), P(gg(enc.bn.weight)), P(gg(enc.bn.bias)), 0, stream),
-                       "gic_encoder_bwd")
+            encoder_bwd_raw(mode, dfeat, pooled, lin, mean, rstd, e.linear.weight, e.bn.weight, dlin, *grads, stream)
             return
         stats = self._buf("enc_bstats", 2 * E)
         _lib.check(lib.gic_encoder_bwd_stats(P(dfeat), P(lin), P(mean), P(rstd), B, E, P(stats), stream), "gic_encoder_bwd_stats")
         parallel.allreduce_sum_(stats)
-        _lib.check(lib.gic_encoder_bwd_apply(mode, P(dfeat), P(pooled), P(lin), P(mean), P(rstd), P(enc.bn.weight), B,
+        _lib.check(lib.gic_encoder_bwd_apply(mode, P(dfeat), P(pooled), P(lin), P(mean), P(rstd), P(e.bn.weight), B,
                                              pooled.shape[1], E, P(stats), float(B * self.world), 1.0 / self.world, P(dlin),
-                                             P(gg(enc.linear.weight)), P(gg(enc.linear.bias)), P(gg(enc.bn.weight)),
-                                             P(gg(enc.bn.bias)), stream), "gic_encoder_bwd_apply")
+                                             *map(P, grads), stream), "gic_encoder_bwd_apply")
 
     # ---- flat buffers ---------------------------------------------------------------------------
     def _gen_params(self):
@@ -381,20 +400,14 @@ class GANInstructor:
             return self._adv_step_graph(captions, pooled, u, keep, loss_type, static=(graph == "static"), grid=grid)
         _lib.require_cuda()
         lib = _lib.lib()
-        a, dev = self.args, self.device
         mode = gic_b200.get_gemm_mode()
-        loss_type = loss_type or a.adv_loss_type
+        loss_type = loss_type or self.args.adv_loss_type
         if loss_type not in _lib.LOSS_TYPES:
             raise NotImplementedError("Divergence '%s' is not implemented" % loss_type)
         self._ensure_flat()
-        fg, fd = self._flat_g, self._flat_d
-        dec, disc = self.gen.decoder, self.disc
-        captions = captions.to(dev).long().contiguous()
-        B, L = captions.shape
-        V, E, H, layers = a.vocab_size, a.gen_embed_dim, a.gen_hidden_dim, a.gen_num_layers
-        De, R, Fd = a.disc_embed_dim, a.disc_num_rep, sum(a.disc_num_filters)
-        fsz, nfl = list(a.disc_filter_sizes), list(a.disc_num_filters)
-        T = float(dec.temperature)
+        disc = self.disc
+        captions = captions.to(self.device).long().contiguous()
+        Fd = sum(self.args.disc_num_filters)
         stream = _lib.stream()
         P = _lib.ptr
         if self._in_graph:
@@ -407,17 +420,16 @@ class GANInstructor:
                                         P(disc.out2logits.bias), Fd, P(prep), stream), "gic_disc_prepare")
         lib.gic_disc_set_prepared(P(prep))
         try:
-            return self._adv_step_body(captions, pooled, u, keep, train, forced_ids, loss_type, update, grid, prep)
+            return self._adv_step_body(mode, captions, pooled, u, keep, train, forced_ids, loss_type, update, grid)
         finally:
             lib.gic_disc_set_prepared(None)
             lib.gic_set_rng(0, 0, None)
             if self._in_graph:
                 lib.gic_set_temperature_device(None)
 
-    def _adv_step_body(self, captions, pooled, u, keep, train, forced_ids, loss_type, update, grid, prep):
+    def _adv_step_body(self, mode, captions, pooled, u, keep, train, forced_ids, loss_type, update, grid):
         lib = _lib.lib()
         a, dev = self.args, self.device
-        mode = gic_b200.get_gemm_mode()
         fg, fd = self._flat_g, self._flat_d
         dec, disc = self.gen.decoder, self.disc
         B, L = captions.shape
@@ -446,30 +458,18 @@ class GANInstructor:
             k0, k1, k2 = keep[0], keep[1], keep[2]
         else:
             k0 = k1 = k2 = None
-        cw = [c.weight for c in disc.convs]
-        cb = [c.bias for c in disc.convs]
-        dW = (disc.embeddings.weight, cw, cb, disc.highway.weight, disc.highway.bias, disc.feature2out.weight,
-              disc.feature2out.bias, disc.out2logits.weight, disc.out2logits.bias)
+        dW = disc_weights(disc)
         drop_p = disc.dropout.p
         main = torch.cuda.current_stream()
         side = self._side_stream() if (train and self.overlap) else None
         self._mark("start (masks drawn)")
         # -- backward helper: D parameter gradients from (real, fake); generator gradients through D(gen) (:168-169, Q1)
         bws = self._buf("disc_bws", lib.gic_disc_bwd_workspace_floats(B, L, De, R, Fd))
-        g = fd.g
-        dcw, dcb = [g(c.weight) for c in disc.convs], [g(c.bias) for c in disc.convs]
+        dgrad = _grad_views(fd, dW)
 
-        def disc_bwd(seed, kp, inp, idz, saved, want_param, acc, dinp, bws, stream):
-            _lib.check(lib.gic_disc_bwd(mode, P(seed), P(kp), drop_p, P(inp), P(idz), B, L, V, De, R, len(fsz),
-                                        _lib.int_array(fsz), _lib.int_array(nfl), P(disc.embeddings.weight),
-                                        _lib.ptr_array(cw), _lib.ptr_array(cb), P(disc.highway.weight),
-                                        P(disc.feature2out.weight), P(disc.feature2out.bias),
-                                        disc.feature2out.weight.shape[0], P(disc.out2logits.weight),
-                                        P(disc.out2logits.bias), P(saved), P(bws), P(g(disc.embeddings.weight)),
-                                        _lib.ptr_array(dcw), _lib.ptr_array(dcb), P(g(disc.highway.weight)),
-                                        P(g(disc.highway.bias)), P(g(disc.feature2out.weight)),
-                                        P(g(disc.feature2out.bias)), P(g(disc.out2logits.weight)),
-                                        P(g(disc.out2logits.bias)), P(dinp), want_param, acc, stream), "gic_disc_bwd")
+        def disc_bwd(seed, kp, inp, idz, saved, want_param, acc, bws, stream):
+            disc_bwd_raw(mode, seed, kp, drop_p, inp, idz, B, L, V, De, R, fsz, nfl, dW, saved, bws, dgrad, None, want_param,
+                         acc, stream)
 
         if side is not None:
             side.wait_stream(main)
@@ -482,7 +482,6 @@ class GANInstructor:
         # -- step-0 input (:144-147)
         attn = grid is not None
         if attn:
-            import ctypes as C
             if not dec.attention or layers != 1:
                 raise ValueError("grid given: build the generator with gen_attention=1 and one LSTM layer")
             grid = grid.to(dev).float().contiguous()
@@ -491,15 +490,7 @@ class GANInstructor:
             Pn, Da = grid.shape[1], a.attn_dim
             asaved = self._buf("attn_saved", lib.gic_attn_saved_floats(B, L, Pn, Da, E))
             we = dec.attn_e.weight.view(-1)
-        if self.cgan:
-            enc = self.gen.encoder
-            pooled = pooled.to(dev).float().contiguous()
-            Fin = pooled.shape[1]
-            lin, mean, rstd = self._buf("enc_lin", B * E).view(B, E), self._buf("enc_mean", E), self._buf("enc_rstd", E)
-            feats = self._buf("feats", B * E).view(B, E)
-            self._encoder_fwd(mode, pooled, B, Fin, E, lin, mean, rstd, feats, stream)
-        else:
-            feats = dec.embed.weight[1].expand(B, E).contiguous()
+        feats, enc = self._features_fwd(mode, pooled, B, stream)
         # -- Decoder.sample (:150)
         if u is not None:
             u = u.to(dev).float().contiguous()
@@ -508,22 +499,11 @@ class GANInstructor:
         dsaved = self._buf("dec_saved", lib.gic_decode_saved_floats(B, L, E, H, layers))
         dws = self._buf("dec_ws", lib.gic_decode_fwd_workspace_floats(B, V, H))
         lp = dec.lstm_params()
-        W_ih, W_hh, b_ih, b_hh = lp[0::4], lp[1::4], lp[2::4], lp[3::4]
         if forced_ids is not None:
             forced_ids = forced_ids.to(dev).long().contiguous()
-        if attn:
-            blk = _lib.attn_block(grid, dec.attn_k.weight, dec.attn_v.weight, dec.attn_q.weight, we, asaved)
-            _lib.check(lib.gic_decode_sample_fwd_attn(C.byref(blk), mode, P(feats), P(dec.embed.weight),
-                                                      _lib.ptr_array(W_ih), _lib.ptr_array(W_hh), _lib.ptr_array(b_ih),
-                                                      _lib.ptr_array(b_hh), P(dec.linear.weight), P(dec.linear.bias),
-                                                      P(u), T, 0, P(forced_ids), B, L, V, E, H, layers, P(probs), P(ids),
-                                                      P(dsaved), P(dws), stream), "gic_decode_sample_fwd_attn")
-        else:
-            _lib.check(lib.gic_decode_sample_fwd(mode, P(feats), P(dec.embed.weight), _lib.ptr_array(W_ih),
-                                                 _lib.ptr_array(W_hh), _lib.ptr_array(b_ih), _lib.ptr_array(b_hh),
-                                                 P(dec.linear.weight), P(dec.linear.bias), P(u), T, 0, P(forced_ids), B,
-                                                 L, V, E, H, layers, P(probs), P(ids), P(dsaved), P(dws), stream),
-                       "gic_decode_sample_fwd")
+        blk = _lib.attn_block(grid, dec.attn_k.weight, dec.attn_v.weight, dec.attn_q.weight, we, asaved) if attn else None
+        decode_fwd_raw(mode, feats, dec.embed.weight, lp, dec.linear.weight, dec.linear.bias, u, T, 0, forced_ids, probs,
+                       ids, dsaved, dws, stream, attn=blk)
         self._mark("main: decode done")
         # -- discriminator on the generated captions: fake / gen share one trunk, two dropout masks (:163-164)
         (d_fake, g_out), saved_f = disc_fwd_raw(lib, mode, probs, None, B, L, V, De, R, fsz, nfl, *dW, [k1, k2],
@@ -532,11 +512,9 @@ class GANInstructor:
         if side is not None:
             main.wait_stream(side)
         # -- losses + seeds (:165)
-        n = B * R
         losses = torch.empty(2, device=dev)
-        seeds = self._buf("seeds", 3 * n).view(3, n)
-        _lib.check(lib.gic_gan_loss_fwd_bwd(_lib.LOSS_TYPES[loss_type], P(d_real), P(d_fake), P(g_out), n, P(losses),
-                                            P(seeds[0]), P(seeds[1]), P(seeds[2]), stream), "gic_gan_loss_fwd_bwd")
+        seeds = self._buf("seeds", 3 * B * R).view(3, B * R)
+        gan_loss_raw(_lib.LOSS_TYPES[loss_type], d_real, d_fake, g_out, losses, seeds, stream)
         self._mark("main: losses done")
         out = dict(g_loss=losses[0], d_loss=losses[1], ids=ids, probs=probs, d_real=d_real, d_fake=d_fake,
                    g_out=g_out, features=feats)
@@ -548,7 +526,7 @@ class GANInstructor:
         def gen_chain(ws_d, st):
             # D's input gradient stays factored (demb x W_e): the dense d(probs)[B,L,V] is never written; the
             # decoder backward fuses demb W_e with the tempered-softmax backward (gic_decode_sample_bwd_factored)
-            disc_bwd(seeds[2], k2, probs, None, saved_f, 0, 0, None, ws_d, st)
+            disc_bwd(seeds[2], k2, probs, None, saved_f, 0, 0, ws_d, st)
             self._mark("G chain: D input gradient (demb) done")
             off = lib.gic_disc_bwd_demb_offset_floats(B, L, De, R, Fd)
             demb = ws_d[off:off + B * L * De]
@@ -559,30 +537,17 @@ class GANInstructor:
             fed = ids if forced_ids is None else forced_ids
             if attn:
                 aws = self._buf("attn_ws", lib.gic_attn_bwd_workspace_floats(B, L, Pn, Da, E))
-                blk = _lib.attn_block(grid, dec.attn_k.weight, dec.attn_v.weight, dec.attn_q.weight, we, asaved, aws,
-                                      gg(dec.attn_k.weight), gg(dec.attn_v.weight), gg(dec.attn_q.weight),
-                                      gg(dec.attn_e.weight).view(-1))
-                _lib.check(lib.gic_decode_sample_bwd_attn(
-                    C.byref(blk), mode, None, P(demb), P(emb), P(disc.embeddings.weight), De, P(probs), P(fed),
-                    P(dec.embed.weight), _lib.ptr_array(W_ih), _lib.ptr_array(W_hh), P(dec.linear.weight), T, 0, B, L, V,
-                    E, H, layers, P(dsaved), P(gws), P(gg(dec.embed.weight)), _lib.ptr_array([gg(w) for w in W_ih]),
-                    _lib.ptr_array([gg(w) for w in W_hh]), _lib.ptr_array([gg(w) for w in b_ih]),
-                    _lib.ptr_array([gg(w) for w in b_hh]), P(gg(dec.linear.weight)), P(gg(dec.linear.bias)), P(dfeat),
-                    st), "gic_decode_sample_bwd_attn")
+                gblk = _lib.attn_block(grid, dec.attn_k.weight, dec.attn_v.weight, dec.attn_q.weight, we, asaved, aws,
+                                       gg(dec.attn_k.weight), gg(dec.attn_v.weight), gg(dec.attn_q.weight),
+                                       gg(dec.attn_e.weight).view(-1))
             else:
+                gblk = None
                 self._zero_unwritten_attn_grads()
-                _lib.check(lib.gic_decode_sample_bwd_factored(
-                    mode, P(demb), P(emb), P(disc.embeddings.weight), De, P(probs), P(fed), P(dec.embed.weight),
-                    _lib.ptr_array(W_ih), _lib.ptr_array(W_hh), P(dec.linear.weight), T, B, L, V, E, H, layers,
-                    P(dsaved), P(gws), P(gg(dec.embed.weight)), _lib.ptr_array([gg(w) for w in W_ih]),
-                    _lib.ptr_array([gg(w) for w in W_hh]), _lib.ptr_array([gg(w) for w in b_ih]),
-                    _lib.ptr_array([gg(w) for w in b_hh]), P(gg(dec.linear.weight)), P(gg(dec.linear.bias)), P(dfeat), 0,
-                    st), "gic_decode_sample_bwd_factored")
+            decode_bwd_raw(mode, None, probs, fed, dec.embed.weight, lp, dec.linear.weight, T, 0, dsaved, gws,
+                           gg(dec.embed.weight), [gg(w) for w in lp], gg(dec.linear.weight), gg(dec.linear.bias), dfeat,
+                           st, factored=(demb, emb, disc.embeddings.weight, De), attn=gblk)
             self._mark("G chain: decoder backward done")
-            if self.cgan:
-                self._encoder_bwd(mode, dfeat, pooled, lin, mean, rstd, B, E, st)
-            else:
-                gg(dec.embed.weight)[1] += dfeat.sum(0)      # features = embed(<S>) for every row (:147)
+            self._features_bwd(mode, dfeat, enc, st)
 
         # Two independent chains after the loss: D parameter gradients (real, then fake accumulated) and the generator
         # chain (D input gradient -> decoder BPTT).  The generator chain is latency-bound (L serial BPTT steps), so it
@@ -603,9 +568,9 @@ class GANInstructor:
                     gen_done.record(side)
                 g_bucketed = self._gen_backward_early_bucket(_bwd)
             # the D chain on main: backward(real), then backward(fake) accumulated onto its parameter gradients
-            disc_bwd(seeds[0], k0, None, captions, saved_r, 1, 0, None, bws, main.cuda_stream)
+            disc_bwd(seeds[0], k0, None, captions, saved_r, 1, 0, bws, main.cuda_stream)
             self._mark("D chain: backward(real) done")
-            disc_bwd(seeds[1], k1, probs, None, saved_f, 1, 1, None, bws, main.cuda_stream)
+            disc_bwd(seeds[1], k1, probs, None, saved_f, 1, 1, bws, main.cuda_stream)
             self._mark("D chain: backward(fake) done")
             d_sq = self._allreduce(fd.grad, 0, self._sq_d)
             self._mark("D chain: gradients all-reduced")
@@ -622,8 +587,8 @@ class GANInstructor:
             main.wait_stream(side)
             self._mark("end")
         else:
-            disc_bwd(seeds[0], k0, None, captions, saved_r, 1, 0, None, bws, stream)
-            disc_bwd(seeds[1], k1, probs, None, saved_f, 1, 1, None, bws, stream)
+            disc_bwd(seeds[0], k0, None, captions, saved_r, 1, 0, bws, stream)
+            disc_bwd(seeds[1], k1, probs, None, saved_f, 1, 1, bws, stream)
             if g_has_grad:
                 gen_chain(bws, stream)
             # -- data-parallel exchange: summed gradients, averaged inside the optimizer kernel
@@ -635,23 +600,28 @@ class GANInstructor:
         out["g_has_grad"] = g_has_grad
         return out
 
-    def _clip_adam(self, fp: FlatParams, lr: float, update: bool, dyn_slot: int = 1, sq=None):
-        """sq: square norm of fp.grad already on the device (the peer all-reduce computes it in the same pass)."""
+    def _clip_adam(self, fp: FlatParams, lr: float, update: bool, dyn_slot: int = 1, sq=None, pre=False):
+        """sq: square norm of fp.grad already on the device (the peer all-reduce computes it in the same pass).
+        pre: step with the pre-training optimizer's moments and step count (fp.m_pre / v_pre / step_pre)."""
         lib = _lib.lib()
         stream = _lib.stream()
+        P = _lib.ptr
+        m, v = (fp.m_pre, fp.v_pre) if pre else (fp.m, fp.v)
         if sq is None:
             sq = torch.zeros(1, device=self.device)
-            _lib.check(lib.gic_grad_sqnorm(_lib.ptr(fp.grad), fp.n, _lib.ptr(sq), stream), "gic_grad_sqnorm")
+            _lib.check(lib.gic_grad_sqnorm(P(fp.grad), fp.n, P(sq), stream), "gic_grad_sqnorm")
         if update and self._in_graph:
-            _lib.check(lib.gic_clip_adam_dyn(_lib.ptr(fp.flat), _lib.ptr(fp.grad), _lib.ptr(fp.m), _lib.ptr(fp.v), fp.n,
-                                             _lib.ptr(sq), float(self.args.clip_norm), 1.0 / self.world,
-                                             _lib.ptr(self._dyn[dyn_slot:dyn_slot + 2]), 0.9, 0.999, 1e-8, stream),
-                       "gic_clip_adam_dyn")
+            _lib.check(lib.gic_clip_adam_dyn(P(fp.flat), P(fp.grad), P(m), P(v), fp.n, P(sq), float(self.args.clip_norm),
+                                             1.0 / self.world, P(self._dyn[dyn_slot:dyn_slot + 2]), 0.9, 0.999, 1e-8,
+                                             stream), "gic_clip_adam_dyn")
         elif update:
-            fp.step += 1
-            _lib.check(lib.gic_clip_adam(_lib.ptr(fp.flat), _lib.ptr(fp.grad), _lib.ptr(fp.m), _lib.ptr(fp.v), fp.n,
-                                         _lib.ptr(sq), float(self.args.clip_norm), 1.0 / self.world, fp.step,
-                                         float(lr), 0.9, 0.999, 1e-8, stream), "gic_clip_adam")
+            if pre:
+                fp.step_pre += 1
+            else:
+                fp.step += 1
+            _lib.check(lib.gic_clip_adam(P(fp.flat), P(fp.grad), P(m), P(v), fp.n, P(sq), float(self.args.clip_norm),
+                                         1.0 / self.world, fp.step_pre if pre else fp.step, float(lr), 0.9, 0.999, 1e-8,
+                                         stream), "gic_clip_adam")
         return sq
 
     # ---- CUDA-graph replay of the fused step -------------------------------------------------------
@@ -840,25 +810,14 @@ class GANInstructor:
         V, E, H, layers = a.vocab_size, a.gen_embed_dim, a.gen_hidden_dim, a.gen_num_layers
         stream = _lib.stream()
         P = _lib.ptr
-        if self.cgan:
-            enc = self.gen.encoder
-            pooled = pooled.to(dev).float().contiguous()
-            Fin = pooled.shape[1]
-            lin, mean, rstd = self._buf("enc_lin", B * E).view(B, E), self._buf("enc_mean", E), self._buf("enc_rstd", E)
-            feats = self._buf("feats", B * E).view(B, E)
-            self._encoder_fwd(mode, pooled, B, Fin, E, lin, mean, rstd, feats, stream)
-        else:
-            feats = dec.embed.weight[1].expand(B, E).contiguous()
+        feats, enc = self._features_fwd(mode, pooled, B, stream)
         logits = self._buf("pg_logits", B * L * V).view(B, L, V)
         ids = torch.empty(B, L, dtype=torch.int64, device=dev)
         dsaved = self._buf("dec_saved", lib.gic_decode_saved_floats(B, L, E, H, layers))
         dws = self._buf("dec_ws", lib.gic_decode_fwd_workspace_floats(B, V, H))
         lp = dec.lstm_params()
-        W_ih, W_hh, b_ih, b_hh = lp[0::4], lp[1::4], lp[2::4], lp[3::4]
-        _lib.check(lib.gic_decode_sample_fwd(mode, P(feats), P(dec.embed.weight), _lib.ptr_array(W_ih),
-                                             _lib.ptr_array(W_hh), _lib.ptr_array(b_ih), _lib.ptr_array(b_hh),
-                                             P(dec.linear.weight), P(dec.linear.bias), None, 1.0, 1, None, B, L, V, E, H,
-                                             layers, P(logits), P(ids), P(dsaved), P(dws), stream), "gic_decode_sample_fwd")
+        decode_fwd_raw(mode, feats, dec.embed.weight, lp, dec.linear.weight, dec.linear.bias, None, 1.0, 1, None, logits,
+                       ids, dsaved, dws, stream)
         loss = torch.empty(1, device=dev)
         dlogits = self._buf("pg_dlogits", B * L * V).view(B, L, V)
         _lib.check(lib.gic_ce_loss_fwd_bwd(P(logits), P(captions), B, L, V, P(loss), P(dlogits), stream), "gic_ce_loss_fwd_bwd")
@@ -866,31 +825,14 @@ class GANInstructor:
         fg.grad.zero_()
         gws = self._buf("dec_bws", lib.gic_decode_bwd_workspace_floats(B, L, V, E, H, layers))
         dfeat = self._buf("dfeat", B * E).view(B, E)
-        _lib.check(lib.gic_decode_sample_bwd(
-            mode, P(dlogits), None, P(ids), P(dec.embed.weight), _lib.ptr_array(W_ih), _lib.ptr_array(W_hh),
-            P(dec.linear.weight), 1.0, 1, B, L, V, E, H, layers, P(dsaved), P(gws), P(gg(dec.embed.weight)),
-            _lib.ptr_array([gg(w) for w in W_ih]), _lib.ptr_array([gg(w) for w in W_hh]),
-            _lib.ptr_array([gg(w) for w in b_ih]), _lib.ptr_array([gg(w) for w in b_hh]), P(gg(dec.linear.weight)),
-            P(gg(dec.linear.bias)), P(dfeat), 0, stream), "gic_decode_sample_bwd")
-        if self.cgan:
-            enc = self.gen.encoder
-            _lib.check(lib.gic_encoder_bwd(mode, P(dfeat), P(pooled), P(lin), P(mean), P(rstd), P(enc.linear.weight),
-                                           P(enc.bn.weight), B, pooled.shape[1], E, P(self._buf("enc_dlin", B * E)),
-                                           P(gg(enc.linear.weight)), P(gg(enc.linear.bias)), P(gg(enc.bn.weight)),
-                                           P(gg(enc.bn.bias)), 0, stream), "gic_encoder_bwd")
-        else:
-            gg(dec.embed.weight)[1] += dfeat.sum(0)
+        decode_bwd_raw(mode, dlogits, None, ids, dec.embed.weight, lp, dec.linear.weight, 1.0, 1, dsaved, gws,
+                       gg(dec.embed.weight), [gg(w) for w in lp], gg(dec.linear.weight), gg(dec.linear.bias), dfeat, stream)
+        self._features_bwd(mode, dfeat, enc, stream)
         self._allreduce(fg.grad, 2)
         # pretrain_opt is its own Adam instance in the reference (:24-26): separate moments and step count
         if not hasattr(fg, "m_pre"):
             fg.m_pre, fg.v_pre, fg.step_pre = torch.zeros_like(fg.m), torch.zeros_like(fg.v), 0
-        sq = torch.zeros(1, device=dev)
-        _lib.check(lib.gic_grad_sqnorm(P(fg.grad), fg.n, P(sq), stream), "gic_grad_sqnorm")
-        if update:
-            fg.step_pre += 1
-            _lib.check(lib.gic_clip_adam(P(fg.flat), P(fg.grad), P(fg.m_pre), P(fg.v_pre), fg.n, P(sq),
-                                         float(a.clip_norm), 1.0 / self.world, fg.step_pre, float(a.pretrain_lr), 0.9,
-                                         0.999, 1e-8, stream), "gic_clip_adam")
+        sq = self._clip_adam(fg, a.pretrain_lr, update, pre=True)
         self.pretrain_steps += 1
         return dict(loss=loss[0], ids=ids, logits=logits, sqnorm=sq)
 
@@ -911,36 +853,21 @@ class GANInstructor:
         V, De, R, Fd = a.vocab_size, a.disc_embed_dim, a.disc_num_rep, sum(a.disc_num_filters)
         fsz, nfl = list(a.disc_filter_sizes), list(a.disc_num_filters)
         stream = _lib.stream()
-        P = _lib.ptr
-        cw = [c.weight for c in disc.convs]
-        cb = [c.bias for c in disc.convs]
-        dW = (disc.embeddings.weight, cw, cb, disc.highway.weight, disc.highway.bias, disc.feature2out.weight,
-              disc.feature2out.bias, disc.out2logits.weight, disc.out2logits.bias)
+        dW = disc_weights(disc)
         drop_p = disc.dropout.p
         if keep is None:
             keep = torch.rand(2, B * R, Fd, device=dev) >= drop_p
         keep = keep.to(dev).to(torch.uint8).contiguous()
         (d_real,), saved_r = disc_fwd_raw(lib, mode, None, real_ids, B, L, V, De, R, fsz, nfl, *dW, [keep[0]], drop_p, dev)
         (d_fake,), saved_f = disc_fwd_raw(lib, mode, None, fake_ids, B, L, V, De, R, fsz, nfl, *dW, [keep[1]], drop_p, dev)
-        nn_ = B * R
         losses = torch.empty(2, device=dev)
-        seeds = self._buf("seeds", 3 * nn_).view(3, nn_)
-        _lib.check(lib.gic_gan_loss_fwd_bwd(_lib.LOSS_TYPES["standard"], P(d_real), P(d_fake), P(d_fake), nn_, P(losses),
-                                            P(seeds[0]), P(seeds[1]), P(seeds[2]), stream), "gic_gan_loss_fwd_bwd")
+        seeds = self._buf("seeds", 3 * B * R).view(3, B * R)
+        gan_loss_raw(_lib.LOSS_TYPES["standard"], d_real, d_fake, d_fake, losses, seeds, stream)
         bws = self._buf("disc_bws", lib.gic_disc_bwd_workspace_floats(B, L, De, R, Fd))
-        g = fd.g
-        dcw, dcb = [g(c.weight) for c in disc.convs], [g(c.bias) for c in disc.convs]
+        dgrad = _grad_views(fd, dW)
         for seed, kp, idz, saved, acc in ((seeds[0], keep[0], real_ids, saved_r, 0), (seeds[1], keep[1], fake_ids, saved_f, 1)):
-            _lib.check(lib.gic_disc_bwd(mode, P(seed), P(kp), drop_p, None, P(idz), B, L, V, De, R, len(fsz),
-                                        _lib.int_array(fsz), _lib.int_array(nfl), P(disc.embeddings.weight),
-                                        _lib.ptr_array(cw), _lib.ptr_array(cb), P(disc.highway.weight),
-                                        P(disc.feature2out.weight), P(disc.feature2out.bias),
-                                        disc.feature2out.weight.shape[0], P(disc.out2logits.weight),
-                                        P(disc.out2logits.bias), P(saved), P(bws), P(g(disc.embeddings.weight)),
-                                        _lib.ptr_array(dcw), _lib.ptr_array(dcb), P(g(disc.highway.weight)),
-                                        P(g(disc.highway.bias)), P(g(disc.feature2out.weight)),
-                                        P(g(disc.feature2out.bias)), P(g(disc.out2logits.weight)),
-                                        P(g(disc.out2logits.bias)), None, 1, acc, stream), "gic_disc_bwd")
+            disc_bwd_raw(mode, seed, kp, drop_p, None, idz, B, L, V, De, R, fsz, nfl, dW, saved, bws, dgrad, None, 1, acc,
+                         stream)
         self._allreduce(fd.grad, 0)
         return dict(d_loss=losses[1], d_real=d_real, d_fake=d_fake, d_sqnorm=self._clip_adam(fd, a.disc_lr, update, 1))
 
@@ -961,23 +888,20 @@ class GANInstructor:
         a, dev = self.args, self.device
         mode = gic_b200.get_gemm_mode()
         self._ensure_flat()
-        fg, fd = self._flat_g, self._flat_d
+        fg = self._flat_g
         dec, disc = self.gen.decoder, self.disc
         captions = captions.to(dev).long().contiguous()
         B, L = captions.shape
         V, E, H, layers = a.vocab_size, a.gen_embed_dim, a.gen_hidden_dim, a.gen_num_layers
         if layers != 1:
             raise NotImplementedError("rollouts support a single-layer decoder")
-        De, R, Fd = a.disc_embed_dim, a.disc_num_rep, sum(a.disc_num_filters)
+        De, R = a.disc_embed_dim, a.disc_num_rep
         fsz, nfl = list(a.disc_filter_sizes), list(a.disc_num_filters)
         stream = _lib.stream()
         P = _lib.ptr
         n = int(n_roll)
         Mmax = (L - 1) * B * n
-        if self.cgan:
-            feats = self.gen.encoder(pooled.to(dev).float()).detach().contiguous()
-        else:
-            feats = dec.embed.weight[1].expand(B, E).contiguous()
+        feats, _ = self._features_fwd(mode, pooled, B, stream)
         if u is None:
             u = torch.rand(L, B, device=dev)
         if u_roll is None:
@@ -989,7 +913,7 @@ class GANInstructor:
         dsaved = self._buf("dec_saved", lib.gic_decode_saved_floats(B, L, E, H, layers))
         dws = self._buf("dec_ws", lib.gic_decode_fwd_workspace_floats(B, V, H))
         lp = dec.lstm_params()
-        W_ih, W_hh, b_ih, b_hh = lp[0::4], lp[1::4], lp[2::4], lp[3::4]
+        W_ih, W_hh, b_ih, b_hh = lstm_split(lp)
         _lib.check(lib.gic_decode_sample_cdf_fwd(mode, P(feats), P(dec.embed.weight), _lib.ptr_array(W_ih),
                                                  _lib.ptr_array(W_hh), _lib.ptr_array(b_ih), _lib.ptr_array(b_hh),
                                                  P(dec.linear.weight), P(dec.linear.bias), P(u), None, B, L, V, E, H,
@@ -1001,10 +925,7 @@ class GANInstructor:
                                            P(b_ih[0]), P(b_hh[0]), P(dec.linear.weight), P(dec.linear.bias), P(u_roll),
                                            B, L, V, E, H, n, P(roll_ids), P(rws), stream), "gic_decode_rollouts")
         # -- D scores of every rollout and of the captions themselves (eval mode, hard-token gather path)
-        cw = [c.weight for c in disc.convs]
-        cb = [c.bias for c in disc.convs]
-        dW = (disc.embeddings.weight, cw, cb, disc.highway.weight, disc.highway.bias, disc.feature2out.weight,
-              disc.feature2out.bias, disc.out2logits.weight, disc.out2logits.bias)
+        dW = disc_weights(disc)
         drop_p = disc.dropout.p
         roll_logits = torch.empty(Mmax * R, device=dev)
         for m0 in range(0, Mmax, score_chunk):
@@ -1023,12 +944,8 @@ class GANInstructor:
         self._zero_unwritten_attn_grads()
         gws = self._buf("dec_bws", lib.gic_decode_bwd_workspace_floats(B, L, V, E, H, layers))
         dfeat = self._buf("dfeat", B * E).view(B, E)
-        _lib.check(lib.gic_decode_sample_bwd(
-            mode, P(dlogits), None, P(ids), P(dec.embed.weight), _lib.ptr_array(W_ih), _lib.ptr_array(W_hh),
-            P(dec.linear.weight), 1.0, 1, B, L, V, E, H, layers, P(dsaved), P(gws), P(gg(dec.embed.weight)),
-            _lib.ptr_array([gg(w) for w in W_ih]), _lib.ptr_array([gg(w) for w in W_hh]),
-            _lib.ptr_array([gg(w) for w in b_ih]), _lib.ptr_array([gg(w) for w in b_hh]), P(gg(dec.linear.weight)),
-            P(gg(dec.linear.bias)), P(dfeat), 0, stream), "gic_decode_sample_bwd")
+        decode_bwd_raw(mode, dlogits, None, ids, dec.embed.weight, lp, dec.linear.weight, 1.0, 1, dsaved, gws,
+                       gg(dec.embed.weight), [gg(w) for w in lp], gg(dec.linear.weight), gg(dec.linear.bias), dfeat, stream)
         if self.cgan:
             enc = self.gen.encoder
             for p_ in (enc.linear.weight, enc.linear.bias, enc.bn.weight, enc.bn.bias):

@@ -8,6 +8,13 @@ import torch
 from . import _lib
 
 
+def gan_loss_raw(loss_type, d_real, d_fake, g_out, losses, seeds, stream):
+    """gic_gan_loss_fwd_bwd: losses[2] = (g_loss, d_loss) and the backward seeds[3, n] of d_real, d_fake and g_out."""
+    P = _lib.ptr
+    _lib.check(_lib.lib().gic_gan_loss_fwd_bwd(loss_type, P(d_real), P(d_fake), P(g_out), d_real.numel(), P(losses),
+                                               P(seeds[0]), P(seeds[1]), P(seeds[2]), stream), "gic_gan_loss_fwd_bwd")
+
+
 class _GanLoss(torch.autograd.Function):
     @staticmethod
     def forward(ctx, d_real, d_fake, g_out, loss_type):
@@ -19,9 +26,7 @@ class _GanLoss(torch.autograd.Function):
         dev = d_real.device
         losses = torch.empty(2, device=dev)
         seeds = torch.empty(3, n, device=dev)
-        _lib.check(_lib.lib().gic_gan_loss_fwd_bwd(loss_type, _lib.ptr(d_real), _lib.ptr(d_fake), _lib.ptr(g_out), n,
-                                                   _lib.ptr(losses), _lib.ptr(seeds[0]), _lib.ptr(seeds[1]),
-                                                   _lib.ptr(seeds[2]), _lib.stream()), "gic_gan_loss_fwd_bwd")
+        gan_loss_raw(loss_type, d_real, d_fake, g_out, losses, seeds, _lib.stream())
         ctx.save_for_backward(seeds)
         ctx.shapes = (d_real.shape, d_fake.shape, g_out.shape)
         ctx.rsgan = (loss_type == _lib.LOSS_TYPES["rsgan"])

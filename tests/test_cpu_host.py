@@ -60,6 +60,22 @@ def test_product_never_imports_oracle():
             assert "oracle" not in src.replace("oracle/", ""), f
 
 
+def test_each_compute_entry_point_has_one_call_site():
+    """Every C ABI call that takes a stream is spelled out once in the package: the autograd modules and the fused steps
+    share one binding per entry point instead of repeating its ctypes argument list."""
+    import re
+    header = open(os.path.join(ROOT, "include", "gic_b200.h")).read()
+    header = re.sub(r"/\*.*?\*/", "", header, flags=re.S)
+    names = [m.group(1) for m in re.finditer(r"\b(gic_[a-z0-9_]+)\s*\(([^;{]*)\)\s*;", header)
+             if "gic_stream_t" in m.group(2)]
+    assert len(names) >= 30
+    pkg = os.path.join(ROOT, "gan-image-captioning_b200")
+    lines = [line for f in sorted(os.listdir(pkg)) if f.endswith(".py")
+             for line in open(os.path.join(pkg, f)).read().splitlines()]
+    many = {n: c for n in names if (c := sum(("." + n + "(") in line for line in lines)) > 1}
+    assert not many, many
+
+
 def test_args_surface_matches_reference_defaults(built):
     from gic_b200.args import default_args, get_args
     a = get_args([])

@@ -622,6 +622,20 @@ def test_pretrain_step_vs_oracle(cfg_name):
     assert not torch.equal(w0, inst.gen.decoder.linear.weight.detach())
 
 
+def test_pretrain_step_refuses_an_eval_mode_encoder():
+    """The encoder backward needs the batch statistics of a train-mode forward: a conditional pre-training step with
+    gen.eval() raises, as adv_step does, instead of computing encoder gradients from stale statistics."""
+    from gic_b200.training import GANInstructor
+    inp = rp.make_inputs(rp.CONFIGS["c1"])
+    a = inp["args"]
+    a.device = "cuda"
+    assert a.conditional_gan
+    inst = GANInstructor(a, device="cuda:0")
+    inst.gen.eval()
+    with pytest.raises(NotImplementedError):
+        inst.pretrain_step(inp["captions"], pooled=inp["pooled"])
+
+
 # ------------------------------------------------------------------------------------------------
 # full-size properties (BASELINE.json configs[1], c2): sizes the oracle cannot reach in seconds
 # ------------------------------------------------------------------------------------------------
