@@ -60,7 +60,7 @@ F = C.c_float
 Z = C.c_size_t
 
 
-RNG_TAG_GUMBEL, RNG_TAG_DROPOUT = 0x47, 0x44
+RNG_TAG_GUMBEL, RNG_TAG_DROPOUT, RNG_TAG_SAMPLE = 0x47, 0x44, 0x53
 
 
 def _declare(L):
@@ -178,6 +178,12 @@ def _declare(L):
     L.gic_score_captions_workspace_floats.restype = Z
     L.gic_score_captions_workspace_floats.argtypes = [I] * 6
     L.gic_score_captions.argtypes = [I, P, P, P, P, P, P, P, P, P, P, I, I, I, I, I, I, P, P, P, P, P]
+    L.gic_vocab_sample_workspace_floats.restype = Z
+    L.gic_vocab_sample_workspace_floats.argtypes = [I] * 3
+    L.gic_vocab_sample.argtypes = [I, P, P, P, I, I, I, I, F, I, F, P, P, P, P]
+    L.gic_sample_captions_workspace_floats.restype = Z
+    L.gic_sample_captions_workspace_floats.argtypes = [I] * 7
+    L.gic_sample_captions.argtypes = [I, P, P, P, P, P, P, P, P, I, I, I, I, I, I, I, C.c_int64, F, I, F, P, P, P, P, P]
     for name in header_symbols():      # every declared entry point must be exported
         getattr(L, name)
 

@@ -19,7 +19,14 @@
 //                      in registers, one row per thread.  Nothing of size V leaves the chip and no CTA waits on another.
 //   row_topk_kernel    (exact-fp32 mode, and shapes TMA rejects) the logits from gemm(...) in workspace, one block per row,
 //                      the same layout as ONE slice.
+//
+// Sampled caption generation (oracle/ref_sample.py sample_captions) reuses both producers: at top_k = 0 their Gumbel
+// instantiations (vocab_gumbel_kernel, row_gumbel_kernel) keep per slice the best key z / T + g(u) instead of a top-K
+// list; at top_k > 0 the plain instantiations supply the top_k largest logits.  sample_rows_kernel (one warp per row)
+// then draws the token: the slices' Gumbel winner, or the Gumbel argmax over the top-k / nucleus set recomputed for those
+// columns only; it writes the token, its logp at temperature 1 and, in the decode, ids / EOS state / the next input.
 #include "tcgen05_common.cuh"
+#include "philox.cuh"
 
 namespace gic {
 namespace tc {
@@ -73,9 +80,19 @@ __device__ __forceinline__ void ms_combine(float& M, float& S, float m, float s)
   else S += s * expf(m - M);
 }
 
-template <int KMAX, bool TGT>
-__global__ void __launch_bounds__(TK_THREADS, 1)
-vocab_topk_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, TKArgs a) {
+// Gumbel instantiation (sampling over the full vocabulary): per element the key z / T + g(u[t, m, n]), u element
+// (t M + m) V + n of the logical stream RNG_TAG_SAMPLE; the slice keeps its best key (ties -> lower column) and the raw
+// logit of that column.  (m, s) stay on the raw logits: the log-sum-exp is at temperature 1.
+struct GumArgs {
+  float T;                  // temperature (divides the logits)
+  int t;                    // RNG step
+  RngState rng;
+  float* part_z;            // [slices][Mpad] raw logit of the slice's winner; part_cand holds (key, column), K = 1
+};
+__device__ __forceinline__ float gumbel_of(float u) { return -logf(-logf(u + 1e-10f) + 1e-10f); }   // Decoder.add_gumbel
+
+template <int KMAX, bool TGT, bool GUM>
+__device__ __forceinline__ void vocab_topk_body(const CUtensorMap& tmA, const CUtensorMap& tmB, TKArgs a, GumArgs gm) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
   uint64_t* full = reinterpret_cast<uint64_t*>(smem + TK_STAGES * TK_STAGE);
@@ -168,6 +185,12 @@ vocab_topk_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
       const int64_t t64 = a.targets[m];
       if (t64 >= 0 && t64 < a.N) tgt = (int)t64;
     }
+    float gz = 0.f;                              // GUM: raw logit of the best key (tv[0], ti[0])
+    unsigned long long rseed = 0ull, roff = 0ull, e_row = 0ull;
+    if (GUM) {
+      rng_load(gm.rng, rseed, roff);
+      e_row = ((unsigned long long)gm.t * a.M + (unsigned long long)m) * a.N;
+    }
     for (int j = 0; j < nt; ++j) {
       const int buf = j & 1;
       mbar_wait(&tfull[buf], (j >> 1) & 1);
@@ -217,7 +240,23 @@ vocab_topk_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
 #pragma unroll
           for (int e = 0; e < 16; ++e) cs += __expf(z[e] - m_new);
           s_run += cs;
-          if (cm > tv[KMAX - 1]) {
+          if (GUM) {
+            if (m < a.M) {
+#pragma unroll
+              for (int k = 0; k < 4; ++k) {
+                const int n = nb + 4 * k;
+                if (n >= a.N) continue;
+                const float4 u4 = philox_uniform4(rseed, roff, RNG_TAG_SAMPLE, (e_row + n) >> 2);   // N % 4 == 0
+                const float uu[4] = {u4.x, u4.y, u4.z, u4.w};
+#pragma unroll
+                for (int c = 0; c < 4; ++c) {
+                  const float zz = z[4 * k + c];
+                  const float key = zz / gm.T + gumbel_of(uu[c]);
+                  if (key > tv[0]) { tv[0] = key; ti[0] = n + c; gz = zz; }
+                }
+              }
+            }
+          } else if (cm > tv[KMAX - 1]) {
 #pragma unroll
             for (int e = 0; e < 16; ++e) topk_insert<KMAX>(tv, ti, z[e], nb + e);
           }
@@ -230,8 +269,25 @@ vocab_topk_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
 #pragma unroll
     for (int i = 0; i < KMAX; ++i) xs[(g * BM + row) * KMAX + i] = make_float2(tv[i], __int_as_float(ti[i]));
     xm[g * BM + row] = make_float2(m_run, s_run);
+    float* xz = reinterpret_cast<float*>(xm + TK_G * BM);          // GUM: [TK_G][BM] raw logit of each group's best key
+    if (GUM) xz[g * BM + row] = gz;
     tk_epi_bar();
-    if (g == 0 && m < a.M) {
+    if (GUM) {
+      if (g == 0 && m < a.M) {
+        float M = -INFINITY, S = 0.f;
+        int best = 0;
+#pragma unroll
+        for (int h = 0; h < TK_G; ++h) {
+          const float2 v = xm[h * BM + row];
+          ms_combine(M, S, v.x, v.y);
+          const float2 c = xs[(h * BM + row) * KMAX], bc = xs[(best * BM + row) * KMAX];
+          if (cand_before(c.x, __float_as_int(c.y), bc.x, __float_as_int(bc.y))) best = h;
+        }
+        a.part_ms[(size_t)slice * a.Mpad + m] = make_float2(M, S);
+        a.part_cand[(size_t)slice * a.Mpad + m] = xs[(best * BM + row) * KMAX];
+        gm.part_z[(size_t)slice * a.Mpad + m] = xz[best * BM + row];
+      }
+    } else if (g == 0 && m < a.M) {
       float M = -INFINITY, S = 0.f;
 #pragma unroll
       for (int h = 0; h < TK_G; ++h) { const float2 v = xm[h * BM + row]; ms_combine(M, S, v.x, v.y); }
@@ -262,12 +318,72 @@ vocab_topk_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
   }
 }
 
+template <int KMAX, bool TGT>
+__global__ void __launch_bounds__(TK_THREADS, 1)
+vocab_topk_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, TKArgs a) {
+  vocab_topk_body<KMAX, TGT, false>(tmA, tmB, a, GumArgs{});
+}
+__global__ void __launch_bounds__(TK_THREADS, 1)
+vocab_gumbel_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, TKArgs a, GumArgs gm) {
+  vocab_topk_body<1, false, true>(tmA, tmB, a, gm);
+}
+
 }  // namespace tc
 
 // ---------------------------------------------------------------------------------------------------------
 // CUDA-core producer: logits[M, V] already in memory (gemm(...) with the bias), one block per row -> slice 0
 // ---------------------------------------------------------------------------------------------------------
 constexpr int RT_THREADS = 256;
+
+// Gumbel instantiation: block m keeps the best key z / T + g(u[t, m, n]) of its row (u element (t M + m) V + n, M =
+// gridDim.x; a Philox group may straddle two rows when V % 4 != 0) and the raw logit of that column.
+__global__ void __launch_bounds__(RT_THREADS)
+row_gumbel_kernel(const float* __restrict__ logits, int V, float2* part_ms, float2* part_cand, tc::GumArgs gm) {
+  using namespace tc;
+  __shared__ float2 s_ms[RT_THREADS / 32];
+  __shared__ float s_key[RT_THREADS / 32], s_z[RT_THREADS / 32];
+  __shared__ int s_col[RT_THREADS / 32];
+  const int m = blockIdx.x, tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
+  const float* row = logits + (size_t)m * V;
+  unsigned long long rseed, roff;
+  rng_load(gm.rng, rseed, roff);
+  const unsigned long long e_row = ((unsigned long long)gm.t * gridDim.x + m) * (unsigned long long)V;
+  float M = -INFINITY, S = 0.f, bk = -INFINITY, bz = 0.f;
+  int bc = 0x7fffffff;
+  for (int n = tid; n < V; n += RT_THREADS) {
+    const float z = row[n];
+    if (z == -INFINITY) continue;
+    if (z > M) { S = S * expf(M - z) + 1.f; M = z; }
+    else S += expf(z - M);
+    const unsigned long long e = e_row + n;
+    const float4 u4 = philox_uniform4(rseed, roff, RNG_TAG_SAMPLE, e >> 2);
+    const int c = (int)(e & 3);
+    const float u = c == 0 ? u4.x : c == 1 ? u4.y : c == 2 ? u4.z : u4.w;
+    const float key = z / gm.T + gumbel_of(u);
+    if (key > bk) { bk = key; bc = n; bz = z; }
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    const float om = __shfl_xor_sync(0xffffffffu, M, o), os = __shfl_xor_sync(0xffffffffu, S, o);
+    ms_combine(M, S, om, os);
+    const float ok = __shfl_xor_sync(0xffffffffu, bk, o), oz = __shfl_xor_sync(0xffffffffu, bz, o);
+    const int oc = __shfl_xor_sync(0xffffffffu, bc, o);
+    if (cand_before(ok, oc, bk, bc)) { bk = ok; bc = oc; bz = oz; }
+  }
+  if (lane == 0) { s_ms[w] = make_float2(M, S); s_key[w] = bk; s_col[w] = bc; s_z[w] = bz; }
+  __syncthreads();
+  if (tid == 0) {
+    float Mb = -INFINITY, Sb = 0.f;
+    int best = 0;
+    for (int i = 0; i < RT_THREADS / 32; ++i) {
+      ms_combine(Mb, Sb, s_ms[i].x, s_ms[i].y);
+      if (cand_before(s_key[i], s_col[i], s_key[best], s_col[best])) best = i;
+    }
+    part_ms[m] = make_float2(Mb, Sb);
+    part_cand[m] = make_float2(s_key[best], __int_as_float(s_col[best]));
+    gm.part_z[m] = s_z[best];
+  }
+}
 
 template <int KMAX, bool TGT>
 __global__ void __launch_bounds__(RT_THREADS)
@@ -453,6 +569,144 @@ score_rows_kernel(const float2* part_ms, const float2* part_cand, const float* p
   }
 }
 
+// gic_vocab_sample / gic_sample_captions: one warp per row draws the token of step t (oracle/ref_sample.py):
+//   topk == 0: the best (key, column) over the slices of the Gumbel producer, and part_z, that column's raw logit;
+//   topk >= 1: the row's topk largest logits (ties -> lower column), lane r holding the r-th; with top_p < 1 the shortest
+//              prefix of softmax(z / T) whose mass reaches top_p (at least one); the Gumbel key z / T + g(u[t, m, w]) of
+//              the kept columns only, the same u element the Gumbel producer reads.
+// The token is the best key (ties -> lower column); logp = z_tok - lse at temperature 1.  In the decode (d.ids != NULL) a
+// frozen row writes PAD; a live row appends its token, adds logp, freezes at d.eos and sets x = embed[token].
+struct SampleRowsArgs {
+  const float2* part_ms; const float2* part_cand; const float* part_z;
+  int slices, Mpad, topk, M, V, t;
+  float T, top_p;
+  RngState rng;
+  int64_t* tokens; float* logp;       // one step (d.ids == NULL)
+  SampleDecode d;
+};
+constexpr int SS_WARPS = 4;
+constexpr int SS_HEADS = 8;        // slice heads per lane: up to 256 slices
+__global__ void __launch_bounds__(SS_WARPS * 32)
+sample_rows_kernel(SampleRowsArgs a) {
+  const int lane = threadIdx.x & 31;
+  const int m = blockIdx.x * SS_WARPS + (threadIdx.x >> 5);
+  if (m >= a.M) return;                                    // warp-uniform
+  const bool decode = a.d.ids != nullptr;
+  if (decode && a.d.fin[m]) {
+    if (lane == 0) a.d.ids[(size_t)m * a.d.L + a.t] = 0;
+    return;
+  }
+  const float lse = row_lse(a.part_ms, a.slices, a.Mpad, m, lane);
+  float bk = -INFINITY, bz = 0.f;
+  int bc = 0x7fffffff;
+  if (a.topk == 0) {
+    for (int s = lane; s < a.slices; s += 32) {
+      const float2 c = a.part_cand[(size_t)s * a.Mpad + m];
+      const int col = __float_as_int(c.y);
+      if (tc::cand_before(c.x, col, bk, bc)) { bk = c.x; bc = col; bz = a.part_z[(size_t)s * a.Mpad + m]; }
+    }
+  } else {
+    // k-way merge of the slices' descending lists: lane owns slices lane + 32 j and holds their current heads; round r
+    // emits the warp's best head (lane r keeps it) and the owner advances that slice (a column lives in one slice only)
+    float hv[SS_HEADS];
+    int hc[SS_HEADS], hp[SS_HEADS];
+    const float2* row = a.part_cand + (size_t)m * a.topk;
+    const size_t sstride = (size_t)a.Mpad * a.topk;
+#pragma unroll
+    for (int j = 0; j < SS_HEADS; ++j) {
+      const int s = lane + 32 * j;
+      hp[j] = 0; hv[j] = -INFINITY; hc[j] = 0x7fffffff;
+      if (s < a.slices) { const float2 x = row[s * sstride]; hv[j] = x.x; hc[j] = __float_as_int(x.y); }
+    }
+    float cz = -INFINITY;
+    int cw = 0x7fffffff;
+    for (int r = 0; r < a.topk; ++r) {
+      float v = -INFINITY;
+      int c = 0x7fffffff, jb = -1;
+#pragma unroll
+      for (int j = 0; j < SS_HEADS; ++j)
+        if (tc::cand_before(hv[j], hc[j], v, c)) { v = hv[j]; c = hc[j]; jb = j; }
+      float bv = v;
+      int bc = c;
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) {
+        const float ov = __shfl_xor_sync(0xffffffffu, bv, o);
+        const int oc = __shfl_xor_sync(0xffffffffu, bc, o);
+        if (tc::cand_before(ov, oc, bv, bc)) { bv = ov; bc = oc; }
+      }
+      if (jb >= 0 && c == bc && v == bv) {
+#pragma unroll
+        for (int j = 0; j < SS_HEADS; ++j) {
+          if (j != jb) continue;
+          ++hp[j];
+          hv[j] = -INFINITY; hc[j] = 0x7fffffff;
+          if (hp[j] < a.topk) {
+            const float2 x = row[(lane + 32 * j) * sstride + hp[j]];
+            hv[j] = x.x; hc[j] = __float_as_int(x.y);
+          }
+        }
+      }
+      if (lane == r) { cz = bv; cw = bc; }
+    }
+    const bool have = lane < a.topk && cw < a.V;
+    const float y = cz / a.T;
+    bool keep = have;
+    if (a.top_p < 1.f) {
+      const float y0 = __shfl_sync(0xffffffffu, y, 0);
+      const float e = have ? expf(y - y0) : 0.f;
+      float inc = e;
+#pragma unroll
+      for (int o = 1; o < 32; o <<= 1) {
+        const float v = __shfl_up_sync(0xffffffffu, inc, o);
+        if (lane >= o) inc += v;
+      }
+      const float tot = __shfl_sync(0xffffffffu, inc, 31);
+      float excl = __shfl_up_sync(0xffffffffu, inc, 1);
+      if (lane == 0) excl = 0.f;
+      keep = have && (lane == 0 || excl < a.top_p * tot);
+    }
+    if (keep) {
+      unsigned long long seed, off;
+      rng_load(a.rng, seed, off);
+      const unsigned long long e = ((unsigned long long)a.t * a.M + m) * (unsigned long long)a.V + cw;
+      const float4 u4 = philox_uniform4(seed, off, RNG_TAG_SAMPLE, e >> 2);
+      const int q = (int)(e & 3);
+      bk = y + tc::gumbel_of(q == 0 ? u4.x : q == 1 ? u4.y : q == 2 ? u4.z : u4.w);
+      bc = cw; bz = cz;
+    }
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    const float ok = __shfl_xor_sync(0xffffffffu, bk, o), oz = __shfl_xor_sync(0xffffffffu, bz, o);
+    const int oc = __shfl_xor_sync(0xffffffffu, bc, o);
+    if (tc::cand_before(ok, oc, bk, bc)) { bk = ok; bc = oc; bz = oz; }
+  }
+  const int tok = (bc >= 0 && bc < a.V) ? bc : 0;          // no finite key in the row: stay in bounds
+  const float lp = bz - lse;
+  if (!decode) {
+    if (lane == 0) { a.tokens[m] = tok; a.logp[m] = lp; }
+    return;
+  }
+  if (lane == 0) {
+    a.d.ids[(size_t)m * a.d.L + a.t] = tok;
+    a.d.caption_logp[m] += lp;
+    if (tok == a.d.eos) { a.d.fin[m] = 1; a.d.len[m] = a.t + 1; }
+  }
+  if (a.t + 1 < a.d.L)
+    for (int u = lane; u < a.d.E; u += 32) a.d.x[(size_t)m * a.d.E + u] = __ldg(a.d.embed + (size_t)tok * a.d.E + u);
+}
+
+// decode start: row m = b n + j reads features[b]; nothing frozen, length L, caption_logp 0
+__global__ void sample_init_kernel(const float* features, int n, SampleDecode d) {
+  const int m = blockIdx.x, b = m / n;
+  for (int u = threadIdx.x; u < d.E; u += blockDim.x) d.x[(size_t)m * d.E + u] = features[(size_t)b * d.E + u];
+  if (threadIdx.x == 0) { d.fin[m] = 0; d.len[m] = d.L; d.caption_logp[m] = 0.f; }
+}
+int sample_init(const float* features, int n, int M, const SampleDecode& d, cudaStream_t s) {
+  sample_init_kernel<<<M, 128, 0, s>>>(features, n, d);
+  return check_launch("sample_init_kernel");
+}
+
 constexpr int BEAM_MAX_LAYERS = 8;
 struct BeamState {
   float* hA[BEAM_MAX_LAYERS]; float* cA[BEAM_MAX_LAYERS];       // state the next step reads (gathered by the merge)
@@ -614,11 +868,23 @@ static int launch_tk(const CUtensorMap& ta, const CUtensorMap& tb, const tc::TKA
   return check_launch("vocab_topk_kernel");
 }
 
+static int launch_gumbel(const CUtensorMap& ta, const CUtensorMap& tb, const tc::TKArgs& a, const tc::GumArgs& gm, dim3 grid,
+                         cudaStream_t s) {
+  static bool attr = false;
+  if (!attr) {
+    cudaFuncSetAttribute(tc::vocab_gumbel_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::TK_SMEM);
+    attr = true;
+  }
+  tc::vocab_gumbel_kernel<<<grid, tc::TK_THREADS, tc::TK_SMEM, s>>>(ta, tb, a, gm);
+  return check_launch("vocab_gumbel_kernel");
+}
+
 // Per-slice (m, s) and top-K candidates of the rows of h[M, H] W_out^T + b_out into ws; *slices = how many slices.
 // targets[M] (K = 1 only, else NULL): also the logit of column targets[m] into part_tgt[m].
+// gum (K = 1 only, else NULL): the Gumbel instantiations, (key, column) in part_cand and the raw logit in gum->part_z.
 static int vocab_topk_partials(int mode, const float* h, const float* W_out, const float* b_out, int M, int V, int H, int K,
                                float* ws, cudaStream_t s, int* slices, const int64_t* targets = nullptr,
-                               float* part_tgt = nullptr) {
+                               float* part_tgt = nullptr, const tc::GumArgs* gum = nullptr) {
   using namespace tc;
   const TopkWs w(M, V, K);
   float2* part_ms = reinterpret_cast<float2*>(ws + w.ms);
@@ -638,6 +904,7 @@ static int vocab_topk_partials(int mode, const float* h, const float* W_out, con
       a.bias = b_out; a.part_ms = part_ms; a.part_cand = part_cand; a.targets = targets; a.part_tgt = part_tgt;
       const dim3 grid(ns, tiles_m);
       *slices = ns;
+      if (gum) return launch_gumbel(ta, tb, a, *gum, grid, s);
       if (targets) return launch_tk<1, true>(ta, tb, a, grid, s);
       if (K <= 4) return launch_tk<4>(ta, tb, a, grid, s);
       if (K <= 8) return launch_tk<8>(ta, tb, a, grid, s);
@@ -647,6 +914,10 @@ static int vocab_topk_partials(int mode, const float* h, const float* W_out, con
   float* logits = ws + w.logits;
   GIC_TRY(gemm(mode, false, true, M, V, H, 1.f, h, H, W_out, H, 0.f, logits, V, b_out, s, PROF_GEMM_DECODE));
   *slices = 1;
+  if (gum) {
+    row_gumbel_kernel<<<M, RT_THREADS, 0, s>>>(logits, V, part_ms, part_cand, *gum);
+    return check_launch("row_gumbel_kernel");
+  }
   if (targets) row_topk_kernel<1, true><<<M, RT_THREADS, 0, s>>>(logits, V, K, part_ms, part_cand, targets, part_tgt);
   else if (K <= 4) row_topk_kernel<4, false><<<M, RT_THREADS, 0, s>>>(logits, V, K, part_ms, part_cand, nullptr, nullptr);
   else if (K <= 8) row_topk_kernel<8, false><<<M, RT_THREADS, 0, s>>>(logits, V, K, part_ms, part_cand, nullptr, nullptr);
@@ -683,6 +954,41 @@ int vocab_target_scores(int mode, const float* h, const float* W_out, const floa
       reinterpret_cast<const float2*>(ws + w.tk.ms), reinterpret_cast<const float2*>(ws + w.tk.cand), ws + w.tgt, slices,
       w.tk.Mpad, V, targets, L, lengths, logp, lse, argmax, correct, caption_logp);
   return check_launch("score_rows_kernel");
+}
+
+// workspace of one sampling step (floats): the candidate producers' at K = max(top_k, 1) | part_z[slices][Mpad]
+struct SampleWs {
+  TopkWs tk;
+  size_t z, total;
+  SampleWs(int M, int V, int top_k) : tk(M, V, top_k > 0 ? top_k : 1) { z = tk.total; total = z + a4((size_t)tk.smax * tk.Mpad); }
+};
+size_t vocab_sample_ws_floats(int M, int V, int top_k) { return SampleWs(M, V, top_k).total; }
+
+RngState rng_state();   // decode.cu: the current context's gic_set_rng state
+
+// Step t of the sampling definition for the rows of h[M, H]: top_k = 0 runs the Gumbel producer, top_k >= 1 the plain
+// producer at K = top_k; then sample_rows_kernel.  d == NULL: tokens[M], logp[M]; else the decode state of d.
+int vocab_sample(int mode, const float* h, const float* W_out, const float* b_out, int M, int V, int H, int t, float T,
+                 int top_k, float top_p, int64_t* tokens, float* logp, const SampleDecode* d, float* ws, cudaStream_t s) {
+  // sample_rows_kernel merges at most 32 * SS_HEADS slices; vocab_topk_partials launches at most num_sms() of them
+  GIC_REQUIRE(num_sms() <= 32 * SS_HEADS, GIC_ERR_UNSUPPORTED, "vocab_sample: %d SMs, the slice merge handles %d", num_sms(),
+              32 * SS_HEADS);
+  const SampleWs w(M, V, top_k);
+  tc::GumArgs gm;
+  gm.T = T; gm.t = t; gm.rng = rng_state(); gm.part_z = ws + w.z;
+  int slices = 1;
+  GIC_TRY(vocab_topk_partials(mode, h, W_out, b_out, M, V, H, top_k > 0 ? top_k : 1, ws, s, &slices, nullptr, nullptr,
+                              top_k > 0 ? nullptr : &gm));
+  SampleRowsArgs a;
+  a.part_ms = reinterpret_cast<const float2*>(ws + w.tk.ms);
+  a.part_cand = reinterpret_cast<const float2*>(ws + w.tk.cand);
+  a.part_z = ws + w.z;
+  a.slices = slices; a.Mpad = w.tk.Mpad; a.topk = top_k; a.M = M; a.V = V; a.t = t;
+  a.T = T; a.top_p = top_p; a.rng = gm.rng;
+  a.tokens = tokens; a.logp = logp;
+  a.d = d ? *d : SampleDecode{};
+  sample_rows_kernel<<<cdiv(M, SS_WARPS), SS_WARPS * 32, 0, s>>>(a);
+  return check_launch("sample_rows_kernel");
 }
 
 // lstm_cell_fwd / lstm_step_tc live in decode.cu / lstm_tcgen05.cu

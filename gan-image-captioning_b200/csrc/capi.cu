@@ -63,6 +63,10 @@ int vocab_target_scores(int mode, const float* h, const float* W_out, const floa
                         float* caption_logp, float* ws, cudaStream_t s);
 int teacher_inputs(const float* features, const int64_t* captions, const float* embed, int B, int L, int E, int V, float* x,
                    cudaStream_t s);
+size_t vocab_sample_ws_floats(int M, int V, int top_k);
+int vocab_sample(int mode, const float* h, const float* W_out, const float* b_out, int M, int V, int H, int t, float T,
+                 int top_k, float top_p, int64_t* tokens, float* logp, const SampleDecode* d, float* ws, cudaStream_t s);
+int sample_init(const float* features, int n, int M, const SampleDecode& d, cudaStream_t s);
 // disc.cu
 int scale_inplace(float*, size_t, float, cudaStream_t);
 // loss_optim.cu
@@ -337,6 +341,53 @@ static int score_captions(int mode, const float* features, const int64_t* captio
   }
   return vocab_target_scores(mode, ws + w.htop, W_out, b_out, captions, B * L, V, H, L, lengths, logp, nullptr, nullptr,
                              correct, caption_logp, ws + w.prod, s);
+}
+
+// sampled-caption workspace (floats): x[M][E] | per layer: h[2][M][H] (ping-pong), c[M][H] (updated in place)
+// | gates[M][4H] | fin[M] | sampling-step workspace, M = B n
+struct SampleCaptionsWs {
+  size_t x, state, per_layer, gates, fin, step, total;
+  SampleCaptionsWs(int M, int V, int E, int H, int layers, int top_k) {
+    const size_t MH = a4((size_t)M * H);
+    x = 0;
+    state = a4((size_t)M * E);
+    per_layer = 3 * MH;
+    gates = state + (size_t)layers * per_layer;
+    fin = gates + a4((size_t)M * 4 * H);
+    step = fin + a4((size_t)M);
+    total = step + vocab_sample_ws_floats(M, V, top_k);
+  }
+};
+
+// n sampled captions per image (gic_sample_captions): rows m = b n + j start from features[b] with h = c = 0; every step
+// runs the LSTM stack (lstm_stack_step, as scoring does), the producer and sample_rows_kernel, which appends the token and
+// writes the next input.  Always L steps, no host sync.
+static int sample_captions(int mode, const float* features, const float* W_emb, const float* const* W_ih,
+                           const float* const* W_hh, const float* const* b_ih, const float* const* b_hh, const float* W_out,
+                           const float* b_out, int B, int n, int L, int V, int E, int H, int layers, int eos, float T,
+                           int top_k, float top_p, int64_t* ids, float* caption_logp, int32_t* lengths, float* ws,
+                           cudaStream_t s) {
+  const int M = B * n;
+  const SampleCaptionsWs w(M, V, E, H, layers, top_k);
+  const size_t MH = a4((size_t)M * H);
+  SampleDecode d = {ids, reinterpret_cast<int*>(ws + w.fin), lengths, caption_logp, ws + w.x, W_emb, L, E, eos};
+  GIC_TRY(sample_init(features, n, M, d, s));
+  for (int l = 0; l < layers; ++l) {
+    float* st = ws + w.state + (size_t)l * w.per_layer;
+    cudaMemsetAsync(st, 0, (size_t)M * H * sizeof(float), s);                    // h of step -1
+    cudaMemsetAsync(st + 2 * MH, 0, (size_t)M * H * sizeof(float), s);          // c
+  }
+  for (int t = 0; t < L; ++t) {
+    LstmLayerIO io[8];
+    for (int l = 0; l < layers; ++l) {
+      float* st = ws + w.state + (size_t)l * w.per_layer;
+      io[l] = {st + (t & 1) * MH, st + 2 * MH, st + ((t + 1) & 1) * MH, st + 2 * MH, nullptr};
+    }
+    GIC_TRY(lstm_stack_step(mode, ws + w.x, io, layers, W_ih, W_hh, b_ih, b_hh, M, E, H, nullptr, ws + w.gates, L, t, s));
+    GIC_TRY(vocab_sample(mode, io[layers - 1].h_new, W_out, b_out, M, V, H, t, T, top_k, top_p, nullptr, nullptr, &d,
+                         ws + w.step, s));
+  }
+  return GIC_OK;
 }
 
 // backward workspace (floats):
@@ -930,6 +981,45 @@ int gic_vocab_target_logp(int mode, const float* h, const float* W_out, const fl
   return vocab_target_scores(mode, h, W_out, b_out, targets, M, V, H, 1, nullptr, logp, lse, argmax, nullptr, nullptr,
                              workspace, S(stream));
 }
+static bool sample_args_ok(float temperature, int top_k, float top_p, int V) {
+  return isfinite(temperature) && temperature > 0.f && top_p > 0.f && top_p <= 1.f && top_k >= 0 && top_k <= 16 &&
+         top_k <= V && !(top_p < 1.f && top_k == 0);
+}
+size_t gic_vocab_sample_workspace_floats(int M, int V, int top_k) { return vocab_sample_ws_floats(M, V, top_k); }
+int gic_vocab_sample(int mode, const float* h, const float* W_out, const float* b_out, int M, int V, int H, int step,
+                     float temperature, int top_k, float top_p, int64_t* tokens, float* logp, float* workspace,
+                     gic_stream_t stream) {
+  GIC_REQUIRE(M >= 0 && V >= 1 && H >= 1 && step >= 0, GIC_ERR_SHAPE, "vocab_sample: bad shape M=%d V=%d H=%d step=%d", M, V,
+              H, step);
+  GIC_REQUIRE(sample_args_ok(temperature, top_k, top_p, V), GIC_ERR_SHAPE,
+              "vocab_sample: bad sampling arguments temperature=%g top_k=%d top_p=%g V=%d", temperature, top_k, top_p, V);
+  if (M == 0) return GIC_OK;
+  GIC_REQUIRE(h && W_out && b_out && tokens && logp && workspace, GIC_ERR_NULL, "vocab_sample: NULL pointer");
+  return vocab_sample(mode, h, W_out, b_out, M, V, H, step, temperature, top_k, top_p, tokens, logp, nullptr, workspace,
+                      S(stream));
+}
+size_t gic_sample_captions_workspace_floats(int B, int n, int V, int E, int H, int layers, int top_k) {
+  return SampleCaptionsWs(B * n, V, E, H, layers, top_k).total;
+}
+int gic_sample_captions(int mode, const float* features, const float* W_emb, const float* const* W_ih,
+                        const float* const* W_hh, const float* const* b_ih, const float* const* b_hh, const float* W_out,
+                        const float* b_out, int B, int n, int L, int V, int E, int H, int layers, int64_t eos_id,
+                        float temperature, int top_k, float top_p, int64_t* ids, float* caption_logp, int32_t* lengths,
+                        float* workspace, gic_stream_t stream) {
+  GIC_REQUIRE(B >= 0 && n >= 1 && L >= 1 && V >= 1 && E >= 1 && H >= 1 && layers >= 1 && layers <= 8 && eos_id >= 0 &&
+                  eos_id < V, GIC_ERR_SHAPE, "sample_captions: bad shape B=%d n=%d L=%d V=%d E=%d H=%d layers=%d eos_id=%lld",
+              B, n, L, V, E, H, layers, (long long)eos_id);
+  GIC_REQUIRE(sample_args_ok(temperature, top_k, top_p, V), GIC_ERR_SHAPE,
+              "sample_captions: bad sampling arguments temperature=%g top_k=%d top_p=%g V=%d", temperature, top_k, top_p, V);
+  if (B == 0) return GIC_OK;
+  GIC_REQUIRE(features && W_emb && W_ih && W_hh && b_ih && b_hh && W_out && b_out && ids && caption_logp && lengths &&
+                  workspace, GIC_ERR_NULL, "sample_captions: NULL pointer");
+  for (int l = 0; l < layers; ++l)
+    GIC_REQUIRE(W_ih[l] && W_hh[l] && b_ih[l] && b_hh[l], GIC_ERR_NULL, "sample_captions: NULL weight of layer %d", l);
+  return sample_captions(mode, features, W_emb, W_ih, W_hh, b_ih, b_hh, W_out, b_out, B, n, L, V, E, H, layers, (int)eos_id,
+                         temperature, top_k, top_p, ids, caption_logp, lengths, workspace, S(stream));
+}
+
 size_t gic_score_captions_workspace_floats(int B, int L, int V, int E, int H, int layers) {
   return ScoreWs(B, L, V, E, H, layers).total;
 }

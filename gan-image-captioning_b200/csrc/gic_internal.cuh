@@ -105,6 +105,13 @@ int vocab_sample_tc(const float* htop, int lda, const float* W_out, const float*
                     const float* T_dev, int B, int V, int H, int L, int t, float* out, int64_t* ids, const int64_t* forced,
                     const float* embed, int E, float* x_next, float* scratch, cudaStream_t stream, bool* handled);
 
+// Per-row state of the sampled-caption decode (beam_tcgen05.cu sample_rows_kernel): ids[M,L] (PAD after EOS), the frozen
+// flag, lengths, caption log-likelihoods and the next LSTM input x[M,E] = embed[token].
+struct SampleDecode {
+  int64_t* ids; int* fin; int32_t* len; float* caption_logp; float* x; const float* embed;
+  int L, E, eos;
+};
+
 // dz (bf16) = T p (demb W_e - dot) and db_out = colsum(dz) in one streaming tcgen05 kernel (dz_fused_tcgen05.cu)
 int dz_fused_tc(const float* demb, int K, const float* W_e, const float* p, const float* dot, float T, const float* T_dev,
                 int M, int V, void* dz_bf, int Vp, float* db_out, int accumulate, cudaStream_t stream, bool* handled);

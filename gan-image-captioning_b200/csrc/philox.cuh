@@ -8,7 +8,7 @@
 
 namespace gic {
 
-enum : uint32_t { RNG_TAG_GUMBEL = 0x47u, RNG_TAG_DROPOUT = 0x44u };
+enum : uint32_t { RNG_TAG_GUMBEL = 0x47u, RNG_TAG_DROPOUT = 0x44u, RNG_TAG_SAMPLE = 0x53u };
 
 struct RngState {
   unsigned long long seed, offset;

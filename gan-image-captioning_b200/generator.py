@@ -338,6 +338,51 @@ def score_captions(dec, features, captions, lengths=None, mode=None):
     return logp, total, corr
 
 
+def check_sample_args(num_samples, max_caption_len, temperature, top_k, top_p, eos_id, V):
+    """ValueError for sampling arguments gic_sample_captions rejects (checked on the host, before any GPU work)."""
+    if int(num_samples) < 1:
+        raise ValueError("num_samples must be >= 1")
+    if int(max_caption_len) < 1:
+        raise ValueError("max_caption_len must be >= 1")
+    if not (math.isfinite(float(temperature)) and float(temperature) > 0):
+        raise ValueError("temperature must be finite and > 0")
+    if not 0 <= int(top_k) <= min(16, V):
+        raise ValueError("top_k must lie in [0, min(16, V)] = [0, %d]" % min(16, V))
+    if not 0 < float(top_p) <= 1:
+        raise ValueError("top_p must lie in (0, 1]")
+    if float(top_p) < 1 and int(top_k) == 0:
+        raise ValueError("top_p < 1 needs 1 <= top_k <= 16: nucleus sampling works inside the top 16 tokens")
+    if not 0 <= int(eos_id) < V:
+        raise ValueError("eos_id must lie in [0, %d)" % V)
+
+
+def sample_captions(dec, features, num_samples=1, max_caption_len=34, temperature=1.0, top_k=0, top_p=1.0, eos_id=2,
+                    mode=None):
+    """gic_sample_captions over the decoder's weights -> (ids[B,n,L] int64, caption_logp[B,n], lengths[B,n] int32).  The
+    draws read the library's Philox state (gic_set_rng) of the current context."""
+    _lib.require_cuda()
+    lib = _lib.lib()
+    mode = gic_b200.get_gemm_mode() if mode is None else mode
+    features = _f32c(features)
+    B, E = features.shape
+    n, L = int(num_samples), int(max_caption_len)
+    V, H = dec.linear.weight.shape
+    layers = dec.lstm.num_layers
+    dev = features.device
+    W_ih, W_hh, b_ih, b_hh = lstm_split([_f32c(w) for w in dec.lstm_params()])
+    W_emb, W_out, b_out = _f32c(dec.embed.weight), _f32c(dec.linear.weight), _f32c(dec.linear.bias)
+    ids = torch.empty(B, n, L, dtype=torch.int64, device=dev)
+    logp = torch.empty(B, n, device=dev)
+    lengths = torch.empty(B, n, dtype=torch.int32, device=dev)
+    ws = torch.empty(lib.gic_sample_captions_workspace_floats(B, n, V, E, H, layers, int(top_k)), device=dev)
+    _lib.check(lib.gic_sample_captions(mode, _lib.ptr(features), _lib.ptr(W_emb), _lib.ptr_array(W_ih), _lib.ptr_array(W_hh),
+                                       _lib.ptr_array(b_ih), _lib.ptr_array(b_hh), _lib.ptr(W_out), _lib.ptr(b_out), B, n, L,
+                                       V, E, H, layers, int(eos_id), float(temperature), int(top_k), float(top_p),
+                                       _lib.ptr(ids), _lib.ptr(logp), _lib.ptr(lengths), _lib.ptr(ws), _lib.stream()),
+               "gic_sample_captions")
+    return ids, logp, lengths
+
+
 class Decoder(nn.Module):
     """LSTM caption decoder (src/generator.py:27-96).  ``embed``/``lstm``/``linear`` are parameter
     containers with the reference's state_dict keys; ``sample`` runs on the B200 kernels."""
@@ -418,6 +463,21 @@ class Decoder(nn.Module):
             raise ValueError("caption ids must lie in [0, %d)" % V)
         logp, total, corr = score_captions(self, features, captions, lengths)
         return logp, total, corr.bool()
+
+    @torch.no_grad()
+    def sample_captions(self, features, num_samples=1, max_caption_len=34, temperature=1.0, top_k=0, top_p=1.0, eos_id=2):
+        """Draw num_samples captions per row of features[B,E] (EXTENSION; oracle/ref_sample.py sample_captions defines it)
+        -> (ids[B,n,L], caption_logp[B,n], lengths[B,n]).  Each step draws from softmax(logits / temperature) restricted
+        to the top_k tokens (0: the whole vocabulary), then to the smallest prefix of them holding top_p of the mass
+        (top_p < 1 needs top_k >= 1).  ``temperature`` divides the logits; it is not ``Decoder.temperature``, which scales
+        the Gumbel-softmax output of ``sample``.  A caption stops at <E> (eos_id): PAD (0) follows, lengths count tokens up
+        to and including <E>, and caption_logp is the caption's log-likelihood under the unfiltered model at temperature 1.
+        Draws come from the library's Philox stream (gic_set_rng); GANInstructor.sample_captions seeds it.  Raises
+        ValueError on an invalid argument before any GPU work."""
+        if self.attention:
+            raise NotImplementedError("caption sampling is implemented for the plain LSTM decoder, not the attention cell")
+        check_sample_args(num_samples, max_caption_len, temperature, top_k, top_p, eos_id, self.linear.out_features)
+        return sample_captions(self, features, num_samples, max_caption_len, temperature, top_k, top_p, eos_id)
 
     def add_gumbel(self, o_t, eps=1e-10, gpu=0):
         """Kept for interface parity (src/generator.py:84-96); the hot path fuses this into the sampler."""

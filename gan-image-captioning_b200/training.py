@@ -734,6 +734,40 @@ class GANInstructor:
         feats = self._start_features(pooled, batch_size)
         return dec.beam_search(feats, beam_size=beam_size, max_caption_len=max_caption_len, length_penalty=length_penalty)
 
+    # ---- EXTENSION: sampled caption generation (temperature / top-k / top-p draws, several captions per image) ----------
+    @_in_ctx
+    @torch.no_grad()
+    def sample_captions(self, pooled=None, batch_size=None, num_samples=1, max_caption_len=34, temperature=1.0, top_k=0,
+                        top_p=1.0, seed=None):
+        """num_samples drawn captions per image -> (ids[B,n,L], caption_logp[B,n], lengths[B,n]) (Decoder.sample_captions),
+        from the step-0 input generate uses (eval-mode encoder projection of pooled, or embed.weight[1] when unconditional).
+        ``seed`` keys the library's Philox stream for this call; None takes one draw from torch's default generator, so
+        torch.manual_seed makes the call reproducible.  ``temperature`` divides the logits (not Decoder.temperature).
+        Leaves parameters, gradients, optimizer state, step counters, temperature and the instructor's random stream as
+        they were; raises ValueError on an invalid argument before any GPU work."""
+        from .generator import check_sample_args
+        dec = self.gen.decoder
+        if dec.attention:
+            raise NotImplementedError("caption sampling is implemented for the plain LSTM decoder, not the attention cell")
+        check_sample_args(num_samples, max_caption_len, temperature, top_k, top_p, END, dec.linear.out_features)
+        if not self.cgan and batch_size is None:
+            if pooled is None:
+                raise ValueError("unconditional generation needs batch_size")
+            batch_size = pooled.shape[0]
+        if self.cgan and pooled is None:
+            raise ValueError("conditional generation needs the pooled image features")
+        _lib.require_cuda()
+        if seed is None:
+            seed = int(torch.randint(0, 2 ** 62, (1,)).item())
+        feats = self._start_features(pooled, batch_size)
+        lib = _lib.lib()
+        lib.gic_set_rng(int(seed) & ((1 << 64) - 1), 0, None)
+        try:
+            return dec.sample_captions(feats, num_samples=num_samples, max_caption_len=max_caption_len,
+                                       temperature=temperature, top_k=top_k, top_p=top_p, eos_id=END)
+        finally:
+            lib.gic_set_rng(0, 0, None)
+
     def _start_features(self, pooled, batch_size):
         """Step-0 input of inference: the eval-mode encoder projection of pooled (conditional), or embed.weight[1]."""
         dec = self.gen.decoder

@@ -299,6 +299,38 @@ int gic_score_captions(int mode, const float* features, const int64_t* captions 
                        int layers, float* logp /*[B,L]*/, float* caption_logp /*[B]*/, uint8_t* correct /*[B,L] or NULL*/,
                        float* workspace, gic_stream_t stream);
 
+/* ---- sampled caption generation (EXTENSION, parity unpinned by reference: oracle/ref_sample.py sample_captions defines
+ * it).  For a row m at step t, with z = h_top W_out^T + b_out over the full vocabulary and lse = logsumexp(z) (temperature 1,
+ * no filter):
+ *   candidate set S: top_k = 0, the whole vocabulary; 1 <= top_k <= 16, the top_k largest z (ties -> lower token); then, if
+ *     top_p < 1, the shortest prefix of S in descending order whose cumulative softmax(z_S / temperature) is >= top_p (at
+ *     least one token).  top_p < 1 needs top_k >= 1: nucleus sampling works inside the top 16.
+ *   token: argmax over w in S of z_w / temperature + g(u[t, m, w]) (ties -> lower token), g(u) = -log(-log(u + 1e-10) +
+ *     1e-10) (Decoder.add_gumbel), u[t, m, w] = element (t M + m) V + w of the logical stream GIC_RNG_TAG_SAMPLE at the
+ *     gic_set_rng state: gic_philox_uniform(GIC_RNG_TAG_SAMPLE, L M V, ...) reproduces every draw.  With S the whole
+ *     vocabulary this is an exact draw from softmax(z / temperature), with a filter from the renormalised filtered one.
+ *   logp = z_token - lse: the log-likelihood under the unfiltered model at temperature 1.
+ * gic_vocab_sample: step `step` of the definition for the rows of h[M,H] -> tokens[M], logp[M].  workspace:
+ *   gic_vocab_sample_workspace_floats(M, V, top_k).
+ * gic_sample_captions: n captions per image under Decoder.sample's LSTM (any number of layers): row m = b n + j starts from
+ *   features[b,E] with h = c = 0; the next input is embed[token].  A row that emits eos_id is frozen: its later ids are PAD
+ *   (0), lengths[m] counts tokens up to and including EOS (L when none), caption_logp[m] sums logp over its live steps.
+ *   Always L steps, no host sync (the call can be captured into a CUDA graph).  ids[B n, L]; workspace:
+ *   gic_sample_captions_workspace_floats(B, n, V, E, H, layers, top_k).  n = 1, temperature 1, top_k 0 draws the ids of
+ *   Decoder.sample with u = the GIC_RNG_TAG_SAMPLE stream (up to the first EOS); top_k = 1 is greedy decoding.
+ * GIC_ERR_SHAPE (both): temperature not finite and > 0, top_p outside (0, 1], top_k outside [0, 16] or > V, top_p < 1 with
+ *   top_k = 0; gic_sample_captions also n < 1, L < 1, eos_id outside [0, V), layers outside 1..8.  M = 0 / B = 0 is a no-op. */
+size_t gic_vocab_sample_workspace_floats(int M, int V, int top_k);
+int gic_vocab_sample(int mode, const float* h /*[M,H]*/, const float* W_out, const float* b_out, int M, int V, int H, int step,
+                     float temperature, int top_k, float top_p, int64_t* tokens /*[M]*/, float* logp /*[M]*/,
+                     float* workspace, gic_stream_t stream);
+size_t gic_sample_captions_workspace_floats(int B, int n, int V, int E, int H, int layers, int top_k);
+int gic_sample_captions(int mode, const float* features /*[B,E]*/, const float* W_emb, const float* const* W_ih,
+                        const float* const* W_hh, const float* const* b_ih, const float* const* b_hh, const float* W_out,
+                        const float* b_out, int B, int n, int L, int V, int E, int H, int layers, int64_t eos_id,
+                        float temperature, int top_k, float top_p, int64_t* ids /*[B n, L]*/, float* caption_logp /*[B n]*/,
+                        int32_t* lengths /*[B n]*/, float* workspace, gic_stream_t stream);
+
 /* ---- B1 (EXTENSION, parity unpinned by reference): additive attention over the CNN feature grid in the decode step.
  * The reference feeds one pooled vector at step 0 (src/generator.py:19-25,58) and has no attention.  Definition:
  *   once per image: Ak = grid W_k^T [B,P,Da], Av = grid W_v^T [B,P,E];  every step: q = h_{t-1} W_q^T,
@@ -376,7 +408,8 @@ int gic_ctx_get_option(const char* name, int dflt);
  * By-value scalars are frozen when a launch is captured into a CUDA graph, but the reference changes two of them every
  * batch: the temperature (update_temperature, src/training.py:183,190-191) and Adam's bias corrections (step count).
  * gic_set_temperature_device(t_dev): while t_dev is non-NULL every entry point that takes `temperature` reads it from
- *   *t_dev when its kernels run and ignores the by-value argument (current context; pass NULL to switch back).
+ *   *t_dev when its kernels run and ignores the by-value argument (current context; pass NULL to switch back).  The
+ *   sampling temperature of gic_vocab_sample / gic_sample_captions is not Decoder.temperature and is always by value.
  * gic_clip_adam_dyn: gic_clip_adam with the step-dependent factors read from device memory:
  *   bias_corr_dev[0] = lr / (1 - beta1^t), bias_corr_dev[1] = 1 / sqrt(1 - beta2^t). */
 void gic_set_temperature_device(const float* t_dev);
@@ -409,6 +442,7 @@ void gic_disc_set_prepared(const float* prepared);
  * gic_philox_keep_mask(tag, n, p, out): uint8 keep masks out[i] = (u_i >= p) for nn.Dropout(p) (GIC_RNG_TAG_DROPOUT). */
 #define GIC_RNG_TAG_GUMBEL 0x47u
 #define GIC_RNG_TAG_DROPOUT 0x44u
+#define GIC_RNG_TAG_SAMPLE 0x53u    /* gic_vocab_sample, gic_sample_captions */
 void gic_set_rng(unsigned long long seed, unsigned long long offset, const unsigned long long* state_dev);
 int gic_philox_uniform(unsigned int tag, size_t n, float* out, gic_stream_t stream);
 int gic_philox_keep_mask(unsigned int tag, size_t n, float p, uint8_t* out, gic_stream_t stream);
