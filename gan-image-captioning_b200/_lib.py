@@ -32,6 +32,11 @@ def attn_block(grid, W_k, W_v, W_q, w_e, saved, ws=None, dW_k=None, dW_v=None, d
                      ptr(dW_k), ptr(dW_v), ptr(dW_q), ptr(dw_e))
 
 
+class DecodeConstraints(C.Structure):
+    """gic_decode_constraints_t (include/gic_b200.h): constrained beam search / sampling."""
+    _fields_ = [("min_length", C.c_int), ("no_repeat_ngram_size", C.c_int), ("bad_ids", C.c_void_p), ("n_bad", C.c_int)]
+
+
 class GicError(RuntimeError):
     pass
 
@@ -184,6 +189,17 @@ def _declare(L):
     L.gic_sample_captions_workspace_floats.restype = Z
     L.gic_sample_captions_workspace_floats.argtypes = [I] * 7
     L.gic_sample_captions.argtypes = [I, P, P, P, P, P, P, P, P, I, I, I, I, I, I, I, C.c_int64, F, I, F, P, P, P, P, P]
+    CP = C.POINTER(DecodeConstraints)
+    L.gic_vocab_topk_masked.argtypes = [I, P, P, P, I, I, I, I, P, P, P, P, P, P]
+    L.gic_vocab_sample_masked.argtypes = [I, P, P, P, I, I, I, I, F, I, F, P, P, P, P, P]
+    L.gic_decode_beam_constrained_workspace_floats.restype = Z
+    L.gic_decode_beam_constrained_workspace_floats.argtypes = [I] * 7 + [CP]
+    L.gic_decode_beam_constrained.argtypes = [I, P, P, P, P, P, P, P, P, I, I, I, I, I, I, I, C.c_int64, F, CP, P, P, P, P,
+                                              P, P]
+    L.gic_sample_captions_constrained_workspace_floats.restype = Z
+    L.gic_sample_captions_constrained_workspace_floats.argtypes = [I] * 8 + [CP]
+    L.gic_sample_captions_constrained.argtypes = [I, P, P, P, P, P, P, P, P, I, I, I, I, I, I, I, C.c_int64, F, I, F, CP, P,
+                                                  P, P, P, P]
     for name in header_symbols():      # every declared entry point must be exported
         getattr(L, name)
 

@@ -25,6 +25,13 @@
 // list; at top_k > 0 the plain instantiations supply the top_k largest logits.  sample_rows_kernel (one warp per row)
 // then draws the token: the slices' Gumbel winner, or the Gumbel argmax over the top-k / nucleus set recomputed for those
 // columns only; it writes the token, its logp at temperature 1 and, in the decode, ids / EOS state / the next input.
+//
+// Constrained generation (gic_decode_constraints_t) masks the candidates inside the producers: their BAN instantiations
+// (vocab_topk_ban_kernel, vocab_gumbel_ban_kernel, row_topk_ban_kernel, row_gumbel_ban_kernel) read a per-row bitmap
+// ban[M][ceil(V/32)] (bit w set: column w is banned), keep (m, s) over the unmasked logits and leave banned columns out of
+// the top-K list / the Gumbel key.  ban_rows_kernel rebuilds the bitmap every step from the call's bad-id bitmap, the
+// minimum length and the row's prefix (no-repeat n-grams).  The consumers are unchanged: a slice left without allowed
+// columns emits (-inf, 0x7fffffff) entries, which they already skip.
 #include "tcgen05_common.cuh"
 #include "philox.cuh"
 
@@ -91,8 +98,15 @@ struct GumArgs {
 };
 __device__ __forceinline__ float gumbel_of(float u) { return -logf(-logf(u + 1e-10f) + 1e-10f); }   // Decoder.add_gumbel
 
-template <int KMAX, bool TGT, bool GUM>
-__device__ __forceinline__ void vocab_topk_body(const CUtensorMap& tmA, const CUtensorMap& tmB, TKArgs a, GumArgs gm) {
+// BAN instantiations: row m's banned columns, bit (w & 31) of ban[m * words + (w >> 5)]
+struct BanArgs {
+  const uint32_t* ban;
+  int words;                // ceil(V / 32)
+};
+
+template <int KMAX, bool TGT, bool GUM, bool BAN>
+__device__ __forceinline__ void vocab_topk_body(const CUtensorMap& tmA, const CUtensorMap& tmB, TKArgs a, GumArgs gm,
+                                                BanArgs bn) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
   uint64_t* full = reinterpret_cast<uint64_t*>(smem + TK_STAGES * TK_STAGE);
@@ -240,8 +254,18 @@ __device__ __forceinline__ void vocab_topk_body(const CUtensorMap& tmA, const CU
 #pragma unroll
           for (int e = 0; e < 16; ++e) cs += __expf(z[e] - m_new);
           s_run += cs;
+          if (BAN) {
+            // nb is 16-aligned: the unit's 16 bits sit in one word; (m, s) above stay on the unmasked logits
+            const uint32_t bits = (m < a.M) ? (__ldg(bn.ban + (size_t)m * bn.words + (nb >> 5)) >> (nb & 16)) & 0xffffu : 0u;
+            cm = -INFINITY;
+#pragma unroll
+            for (int e = 0; e < 16; ++e) {
+              if ((bits >> e) & 1u) z[e] = -INFINITY;
+              cm = fmaxf(cm, z[e]);
+            }
+          }
           if (GUM) {
-            if (m < a.M) {
+            if (m < a.M && (!BAN || cm > -INFINITY)) {
 #pragma unroll
               for (int k = 0; k < 4; ++k) {
                 const int n = nb + 4 * k;
@@ -321,11 +345,21 @@ __device__ __forceinline__ void vocab_topk_body(const CUtensorMap& tmA, const CU
 template <int KMAX, bool TGT>
 __global__ void __launch_bounds__(TK_THREADS, 1)
 vocab_topk_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, TKArgs a) {
-  vocab_topk_body<KMAX, TGT, false>(tmA, tmB, a, GumArgs{});
+  vocab_topk_body<KMAX, TGT, false, false>(tmA, tmB, a, GumArgs{}, BanArgs{});
 }
 __global__ void __launch_bounds__(TK_THREADS, 1)
 vocab_gumbel_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, TKArgs a, GumArgs gm) {
-  vocab_topk_body<1, false, true>(tmA, tmB, a, gm);
+  vocab_topk_body<1, false, true, false>(tmA, tmB, a, gm, BanArgs{});
+}
+template <int KMAX>
+__global__ void __launch_bounds__(TK_THREADS, 1)
+vocab_topk_ban_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, TKArgs a, BanArgs bn) {
+  vocab_topk_body<KMAX, false, false, true>(tmA, tmB, a, GumArgs{}, bn);
+}
+__global__ void __launch_bounds__(TK_THREADS, 1)
+vocab_gumbel_ban_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, TKArgs a, GumArgs gm,
+                        BanArgs bn) {
+  vocab_topk_body<1, false, true, true>(tmA, tmB, a, gm, bn);
 }
 
 }  // namespace tc
@@ -335,10 +369,14 @@ vocab_gumbel_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
 // ---------------------------------------------------------------------------------------------------------
 constexpr int RT_THREADS = 256;
 
+// Bit n of row m's ban bitmap (BAN instantiations)
+__device__ __forceinline__ bool banned(const uint32_t* ban_row, int n) { return (__ldg(ban_row + (n >> 5)) >> (n & 31)) & 1u; }
+
 // Gumbel instantiation: block m keeps the best key z / T + g(u[t, m, n]) of its row (u element (t M + m) V + n, M =
 // gridDim.x; a Philox group may straddle two rows when V % 4 != 0) and the raw logit of that column.
-__global__ void __launch_bounds__(RT_THREADS)
-row_gumbel_kernel(const float* __restrict__ logits, int V, float2* part_ms, float2* part_cand, tc::GumArgs gm) {
+template <bool BAN>
+__device__ __forceinline__ void row_gumbel_body(const float* __restrict__ logits, int V, float2* part_ms, float2* part_cand,
+                                                tc::GumArgs gm, const uint32_t* ban) {
   using namespace tc;
   __shared__ float2 s_ms[RT_THREADS / 32];
   __shared__ float s_key[RT_THREADS / 32], s_z[RT_THREADS / 32];
@@ -355,6 +393,7 @@ row_gumbel_kernel(const float* __restrict__ logits, int V, float2* part_ms, floa
     if (z == -INFINITY) continue;
     if (z > M) { S = S * expf(M - z) + 1.f; M = z; }
     else S += expf(z - M);
+    if (BAN && banned(ban + (size_t)m * ((V + 31) >> 5), n)) continue;
     const unsigned long long e = e_row + n;
     const float4 u4 = philox_uniform4(rseed, roff, RNG_TAG_SAMPLE, e >> 2);
     const int c = (int)(e & 3);
@@ -383,6 +422,15 @@ row_gumbel_kernel(const float* __restrict__ logits, int V, float2* part_ms, floa
     part_cand[m] = make_float2(s_key[best], __int_as_float(s_col[best]));
     gm.part_z[m] = s_z[best];
   }
+}
+__global__ void __launch_bounds__(RT_THREADS)
+row_gumbel_kernel(const float* __restrict__ logits, int V, float2* part_ms, float2* part_cand, tc::GumArgs gm) {
+  row_gumbel_body<false>(logits, V, part_ms, part_cand, gm, nullptr);
+}
+__global__ void __launch_bounds__(RT_THREADS)
+row_gumbel_ban_kernel(const float* __restrict__ logits, int V, float2* part_ms, float2* part_cand, tc::GumArgs gm,
+                      const uint32_t* __restrict__ ban) {
+  row_gumbel_body<true>(logits, V, part_ms, part_cand, gm, ban);
 }
 
 template <int KMAX, bool TGT>
@@ -452,6 +500,131 @@ row_topk_kernel(const float* __restrict__ logits, int V, int topk, float2* part_
     if (tid == bo) ++head;
     __syncthreads();
   }
+}
+
+// BAN instantiation of row_topk_kernel (a copy rather than a shared template body: the shared body changes the SASS of
+// the plain kernels)
+template <int KMAX>
+__global__ void __launch_bounds__(RT_THREADS)
+row_topk_ban_kernel(const float* __restrict__ logits, int V, int topk, float2* part_ms, float2* part_cand,
+                    const uint32_t* __restrict__ ban) {
+  using namespace tc;
+  __shared__ float2 s_list[RT_THREADS * KMAX];
+  __shared__ float2 s_ms[RT_THREADS / 32];
+  __shared__ float2 s_win[RT_THREADS / 32];
+  __shared__ int s_wt[RT_THREADS / 32];
+  const int m = blockIdx.x, tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
+  const float* row = logits + (size_t)m * V;
+  float tv[KMAX];
+  int ti[KMAX];
+#pragma unroll
+  for (int i = 0; i < KMAX; ++i) { tv[i] = -INFINITY; ti[i] = 0x7fffffff; }
+  float M = -INFINITY, S = 0.f;
+  for (int n = tid; n < V; n += RT_THREADS) {
+    const float z = row[n];
+    if (z == -INFINITY) continue;
+    if (z > M) { S = S * expf(M - z) + 1.f; M = z; }
+    else S += expf(z - M);
+    if (!banned(ban + (size_t)m * ((V + 31) >> 5), n)) topk_insert<KMAX>(tv, ti, z, n);
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    const float om = __shfl_xor_sync(0xffffffffu, M, o), os = __shfl_xor_sync(0xffffffffu, S, o);
+    ms_combine(M, S, om, os);
+  }
+  if (lane == 0) s_ms[w] = make_float2(M, S);
+#pragma unroll
+  for (int i = 0; i < KMAX; ++i) s_list[tid * KMAX + i] = make_float2(tv[i], __int_as_float(ti[i]));
+  __syncthreads();
+  if (tid == 0) {
+    float Mb = -INFINITY, Sb = 0.f;
+    for (int i = 0; i < RT_THREADS / 32; ++i) ms_combine(Mb, Sb, s_ms[i].x, s_ms[i].y);
+    part_ms[m] = make_float2(Mb, Sb);
+  }
+  // K rounds: every thread offers the head of its list, the block's best is emitted and its owner advances
+  int head = 0;
+  float2* out = part_cand + (size_t)m * topk;
+  for (int k = 0; k < topk; ++k) {
+    float2 v = (head < KMAX) ? s_list[tid * KMAX + head] : make_float2(-INFINITY, __int_as_float(0x7fffffff));
+    int owner = tid;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      const float ov = __shfl_xor_sync(0xffffffffu, v.x, o);
+      const int oc = __shfl_xor_sync(0xffffffffu, __float_as_int(v.y), o);
+      const int ow = __shfl_xor_sync(0xffffffffu, owner, o);
+      if (cand_before(ov, oc, v.x, __float_as_int(v.y)) || (ov == v.x && oc == __float_as_int(v.y) && ow < owner)) {
+        v = make_float2(ov, __int_as_float(oc)); owner = ow;
+      }
+    }
+    if (lane == 0) { s_win[w] = v; s_wt[w] = owner; }
+    __syncthreads();
+    float2 b = s_win[0];
+    int bo = s_wt[0];
+    for (int i = 1; i < RT_THREADS / 32; ++i)
+      if (cand_before(s_win[i].x, __float_as_int(s_win[i].y), b.x, __float_as_int(b.y)) ||
+          (s_win[i].x == b.x && __float_as_int(s_win[i].y) == __float_as_int(b.y) && s_wt[i] < bo)) { b = s_win[i]; bo = s_wt[i]; }
+    if (tid == 0) out[k] = b;
+    if (tid == bo) ++head;
+    __syncthreads();
+  }
+}
+
+// Per-row ban bitmap of step t (constrained generation, one warp per row): the call's bad-id bitmap, the EOS bit while
+// t + 1 < min_length, and for n = ngram >= 1 the token that would complete an n-gram already in the row's prefix.  The
+// prefix is ids[m, :t] (sampling), or the beam's tokens backtracked through trace (beam search: rows m = b K + k).  Frozen
+// rows are skipped: no consumer reads their candidates.
+struct BanRowsArgs {
+  uint32_t* ban;              // [M][words]
+  const uint32_t* base;       // [words] bad ids
+  const int* fin;             // [M]
+  const int64_t* ids;         // sampling: [M][L], or NULL
+  const int2* trace;          // beam search: [L][B][K] (parent slot, token), or NULL
+  int* prefix;                // [M][L] scratch: the row's prefix (ngram >= 1)
+  int M, words, V, L, K, B, t, eos, min_length, ngram;
+};
+constexpr int BR_WARPS = 4;
+__global__ void __launch_bounds__(BR_WARPS * 32)
+ban_rows_kernel(BanRowsArgs a) {
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  const int m = blockIdx.x * BR_WARPS + w;
+  if (m >= a.M || a.fin[m]) return;                        // warp-uniform
+  uint32_t* row = a.ban + (size_t)m * a.words;
+  for (int i = lane; i < a.words; i += 32) row[i] = a.base[i];
+  __syncwarp();
+  if (lane == 0 && a.t + 1 < a.min_length) atomicOr(row + (a.eos >> 5), 1u << (a.eos & 31));
+  const int n = a.ngram, t = a.t;
+  if (n < 1 || t < n - 1) return;
+  int* y = a.prefix + (size_t)m * a.L;
+  if (a.ids) {
+    for (int s = lane; s < t; s += 32) y[s] = (int)a.ids[(size_t)m * a.L + s];
+  } else if (lane == 0) {
+    const int b = m / a.K;
+    int slot = m - b * a.K;
+    for (int s = t - 1; s >= 0; --s) {
+      const int2 pt = a.trace[((size_t)s * a.B + b) * a.K + slot];
+      y[s] = pt.y;
+      slot = pt.x;
+    }
+  }
+  __syncwarp();
+  for (int s = lane; s <= t - n; s += 32) {
+    bool match = true;
+    for (int j = 0; j < n - 1 && match; ++j) match = y[s + j] == y[t - n + 1 + j];
+    const int tok = y[s + n - 1];
+    if (match && tok >= 0 && tok < a.V) atomicOr(row + (tok >> 5), 1u << (tok & 31));
+  }
+}
+
+// the call's bad-id bitmap: word i of base[words] from every id of bad_ids[n_bad] inside [0, V)
+__global__ void ban_base_kernel(const int64_t* bad_ids, int n_bad, int V, int words, uint32_t* base) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= words) return;
+  uint32_t bits = 0u;
+  for (int j = 0; j < n_bad; ++j) {
+    const int64_t id = bad_ids[j];
+    if (id >= 0 && id < V && (int)(id >> 5) == i) bits |= 1u << (id & 31);
+  }
+  base[i] = bits;
 }
 
 // ---------------------------------------------------------------------------------------------------------
@@ -879,12 +1052,36 @@ static int launch_gumbel(const CUtensorMap& ta, const CUtensorMap& tb, const tc:
   return check_launch("vocab_gumbel_kernel");
 }
 
+template <int KMAX>
+static int launch_tk_ban(const CUtensorMap& ta, const CUtensorMap& tb, const tc::TKArgs& a, const tc::BanArgs& bn, dim3 grid,
+                         cudaStream_t s) {
+  static bool attr = false;
+  if (!attr) {
+    cudaFuncSetAttribute(tc::vocab_topk_ban_kernel<KMAX>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::TK_SMEM);
+    attr = true;
+  }
+  tc::vocab_topk_ban_kernel<KMAX><<<grid, tc::TK_THREADS, tc::TK_SMEM, s>>>(ta, tb, a, bn);
+  return check_launch("vocab_topk_ban_kernel");
+}
+
+static int launch_gumbel_ban(const CUtensorMap& ta, const CUtensorMap& tb, const tc::TKArgs& a, const tc::GumArgs& gm,
+                             const tc::BanArgs& bn, dim3 grid, cudaStream_t s) {
+  static bool attr = false;
+  if (!attr) {
+    cudaFuncSetAttribute(tc::vocab_gumbel_ban_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, tc::TK_SMEM);
+    attr = true;
+  }
+  tc::vocab_gumbel_ban_kernel<<<grid, tc::TK_THREADS, tc::TK_SMEM, s>>>(ta, tb, a, gm, bn);
+  return check_launch("vocab_gumbel_ban_kernel");
+}
+
 // Per-slice (m, s) and top-K candidates of the rows of h[M, H] W_out^T + b_out into ws; *slices = how many slices.
 // targets[M] (K = 1 only, else NULL): also the logit of column targets[m] into part_tgt[m].
 // gum (K = 1 only, else NULL): the Gumbel instantiations, (key, column) in part_cand and the raw logit in gum->part_z.
+// ban[M][ceil(V/32)] (not with targets, else NULL): the BAN instantiations, banned columns left out of the candidates.
 static int vocab_topk_partials(int mode, const float* h, const float* W_out, const float* b_out, int M, int V, int H, int K,
                                float* ws, cudaStream_t s, int* slices, const int64_t* targets = nullptr,
-                               float* part_tgt = nullptr, const tc::GumArgs* gum = nullptr) {
+                               float* part_tgt = nullptr, const tc::GumArgs* gum = nullptr, const uint32_t* ban = nullptr) {
   using namespace tc;
   const TopkWs w(M, V, K);
   float2* part_ms = reinterpret_cast<float2*>(ws + w.ms);
@@ -904,6 +1101,13 @@ static int vocab_topk_partials(int mode, const float* h, const float* W_out, con
       a.bias = b_out; a.part_ms = part_ms; a.part_cand = part_cand; a.targets = targets; a.part_tgt = part_tgt;
       const dim3 grid(ns, tiles_m);
       *slices = ns;
+      if (ban) {
+        const BanArgs bn = {ban, (V + 31) >> 5};
+        if (gum) return launch_gumbel_ban(ta, tb, a, *gum, bn, grid, s);
+        if (K <= 4) return launch_tk_ban<4>(ta, tb, a, bn, grid, s);
+        if (K <= 8) return launch_tk_ban<8>(ta, tb, a, bn, grid, s);
+        return launch_tk_ban<16>(ta, tb, a, bn, grid, s);
+      }
       if (gum) return launch_gumbel(ta, tb, a, *gum, grid, s);
       if (targets) return launch_tk<1, true>(ta, tb, a, grid, s);
       if (K <= 4) return launch_tk<4>(ta, tb, a, grid, s);
@@ -914,6 +1118,16 @@ static int vocab_topk_partials(int mode, const float* h, const float* W_out, con
   float* logits = ws + w.logits;
   GIC_TRY(gemm(mode, false, true, M, V, H, 1.f, h, H, W_out, H, 0.f, logits, V, b_out, s, PROF_GEMM_DECODE));
   *slices = 1;
+  if (ban) {
+    if (gum) {
+      row_gumbel_ban_kernel<<<M, RT_THREADS, 0, s>>>(logits, V, part_ms, part_cand, *gum, ban);
+      return check_launch("row_gumbel_ban_kernel");
+    }
+    if (K <= 4) row_topk_ban_kernel<4><<<M, RT_THREADS, 0, s>>>(logits, V, K, part_ms, part_cand, ban);
+    else if (K <= 8) row_topk_ban_kernel<8><<<M, RT_THREADS, 0, s>>>(logits, V, K, part_ms, part_cand, ban);
+    else row_topk_ban_kernel<16><<<M, RT_THREADS, 0, s>>>(logits, V, K, part_ms, part_cand, ban);
+    return check_launch("row_topk_ban_kernel");
+  }
   if (gum) {
     row_gumbel_kernel<<<M, RT_THREADS, 0, s>>>(logits, V, part_ms, part_cand, *gum);
     return check_launch("row_gumbel_kernel");
@@ -926,9 +1140,9 @@ static int vocab_topk_partials(int mode, const float* h, const float* W_out, con
 }
 
 int vocab_topk(int mode, const float* h, const float* W_out, const float* b_out, int M, int V, int H, int K, float* logp,
-               int64_t* tokens, float* lse, float* ws, cudaStream_t s) {
+               int64_t* tokens, float* lse, const uint32_t* ban, float* ws, cudaStream_t s) {
   int slices = 1;
-  GIC_TRY(vocab_topk_partials(mode, h, W_out, b_out, M, V, H, K, ws, s, &slices));
+  GIC_TRY(vocab_topk_partials(mode, h, W_out, b_out, M, V, H, K, ws, s, &slices, nullptr, nullptr, nullptr, ban));
   const TopkWs w(M, V, K);
   topk_rows_kernel<<<M, TR_THREADS, 0, s>>>(reinterpret_cast<const float2*>(ws + w.ms), reinterpret_cast<const float2*>(ws + w.cand),
                                             slices, w.Mpad, K, V, logp, tokens, lse);
@@ -967,9 +1181,11 @@ size_t vocab_sample_ws_floats(int M, int V, int top_k) { return SampleWs(M, V, t
 RngState rng_state();   // decode.cu: the current context's gic_set_rng state
 
 // Step t of the sampling definition for the rows of h[M, H]: top_k = 0 runs the Gumbel producer, top_k >= 1 the plain
-// producer at K = top_k; then sample_rows_kernel.  d == NULL: tokens[M], logp[M]; else the decode state of d.
+// producer at K = top_k; then sample_rows_kernel.  d == NULL: tokens[M], logp[M]; else the decode state of d.  ban (or
+// NULL): the rows' ban bitmaps, read by the producers' BAN instantiations.
 int vocab_sample(int mode, const float* h, const float* W_out, const float* b_out, int M, int V, int H, int t, float T,
-                 int top_k, float top_p, int64_t* tokens, float* logp, const SampleDecode* d, float* ws, cudaStream_t s) {
+                 int top_k, float top_p, int64_t* tokens, float* logp, const SampleDecode* d, const uint32_t* ban, float* ws,
+                 cudaStream_t s) {
   // sample_rows_kernel merges at most 32 * SS_HEADS slices; vocab_topk_partials launches at most num_sms() of them
   GIC_REQUIRE(num_sms() <= 32 * SS_HEADS, GIC_ERR_UNSUPPORTED, "vocab_sample: %d SMs, the slice merge handles %d", num_sms(),
               32 * SS_HEADS);
@@ -978,7 +1194,7 @@ int vocab_sample(int mode, const float* h, const float* W_out, const float* b_ou
   gm.T = T; gm.t = t; gm.rng = rng_state(); gm.part_z = ws + w.z;
   int slices = 1;
   GIC_TRY(vocab_topk_partials(mode, h, W_out, b_out, M, V, H, top_k > 0 ? top_k : 1, ws, s, &slices, nullptr, nullptr,
-                              top_k > 0 ? nullptr : &gm));
+                              top_k > 0 ? nullptr : &gm, ban));
   SampleRowsArgs a;
   a.part_ms = reinterpret_cast<const float2*>(ws + w.tk.ms);
   a.part_cand = reinterpret_cast<const float2*>(ws + w.tk.cand);
@@ -997,11 +1213,11 @@ int lstm_step_tc(const float*, int, const float*, const float*, const float*, co
                  int, int, float*, float*, float*, float*, int, int, cudaStream_t, bool*);
 
 // decode_beam workspace (floats): x[BK,E] | per layer hA, cA, hB, cB [BK,H] | gates[BK,4H] | score[BK] | fin[BK] | len[BK]
-// | trace[L,B,K,2] | candidate-producer workspace
+// | trace[L,B,K,2] | candidate-producer workspace | ban bitmaps (BanWs, size 0 unconstrained)
 struct BeamWs {
-  size_t x, state, gates, score, fin, len, trace, topk, total;
+  size_t x, state, gates, score, fin, len, trace, topk, ban, total;
   size_t BKH;
-  BeamWs(int B, int K, int L, int V, int E, int H, int layers) {
+  BeamWs(int B, int K, int L, int V, int E, int H, int layers, const gic_decode_constraints_t* c = nullptr) {
     const size_t BK = (size_t)B * K;
     BKH = a4(BK * H);
     x = 0;
@@ -1012,18 +1228,20 @@ struct BeamWs {
     len = fin + a4(BK);
     trace = len + a4(BK);
     topk = trace + a4((size_t)2 * L * BK);
-    total = topk + TopkWs((int)BK, V, K).total;
+    ban = topk + TopkWs((int)BK, V, K).total;
+    total = ban + BanWs((int)BK, V, L, c).total;
   }
 };
-size_t decode_beam_ws_floats(int B, int K, int L, int V, int E, int H, int layers) {
-  return BeamWs(B, K, L, V, E, H, layers).total;
+size_t decode_beam_ws_floats(int B, int K, int L, int V, int E, int H, int layers, const gic_decode_constraints_t* c) {
+  return BeamWs(B, K, L, V, E, H, layers, c).total;
 }
 
 int decode_beam(int mode, const float* features, const float* W_emb, const float* const* W_ih, const float* const* W_hh,
                 const float* const* b_ih, const float* const* b_hh, const float* W_out, const float* b_out, int B, int K,
-                int L, int V, int E, int H, int layers, int64_t eos, float length_penalty, int64_t* ids, float* scores,
-                int32_t* lengths, int32_t* trace, float* ws, cudaStream_t s) {
-  const BeamWs w(B, K, L, V, E, H, layers);
+                int L, int V, int E, int H, int layers, int64_t eos, float length_penalty,
+                const gic_decode_constraints_t* c, int64_t* ids, float* scores, int32_t* lengths, int32_t* trace, float* ws,
+                cudaStream_t s) {
+  const BeamWs w(B, K, L, V, E, H, layers, c);
   const int BK = B * K;
   BeamState st;
   for (int l = 0; l < BEAM_MAX_LAYERS; ++l) {
@@ -1047,6 +1265,8 @@ int decode_beam(int mode, const float* features, const float* W_emb, const float
   const TopkWs tw(BK, V, K);
   float* tws = ws + w.topk;
   float* gates = ws + w.gates;
+  const BanWs bw(BK, V, L, c);
+  if (c) GIC_TRY(ban_base(c, V, bw, ws + w.ban, s));
   for (int t = 0; t < L; ++t) {
     for (int l = 0; l < layers; ++l) {
       const float* xin = (l == 0) ? st.x : st.hB[l - 1];
@@ -1063,13 +1283,36 @@ int decode_beam(int mode, const float* features, const float* W_emb, const float
       }
     }
     int slices = 1;
-    GIC_TRY(vocab_topk_partials(mode, st.hB[layers - 1], W_out, b_out, BK, V, H, K, tws, s, &slices));
+    if (c)
+      GIC_TRY(ban_rows(c, BK, V, L, t, st.eos, st.fin, nullptr, reinterpret_cast<const int32_t*>(st.trace), B, K, bw, ws + w.ban,
+                       s));
+    GIC_TRY(vocab_topk_partials(mode, st.hB[layers - 1], W_out, b_out, BK, V, H, K, tws, s, &slices, nullptr, nullptr, nullptr,
+                                c ? reinterpret_cast<const uint32_t*>(ws + w.ban + bw.ban) : nullptr));
     beam_merge_kernel<<<B, BM_THREADS, 0, s>>>(reinterpret_cast<const float2*>(tws + tw.ms),
                                                reinterpret_cast<const float2*>(tws + tw.cand), slices, tw.Mpad, t, st);
     GIC_TRY(check_launch("beam_merge_kernel"));
   }
   beam_finalize_kernel<<<B, 32, 0, s>>>(st, length_penalty, ids, scores, lengths);
   return check_launch("beam_finalize_kernel");
+}
+
+int ban_base(const gic_decode_constraints_t* c, int V, const BanWs& bw, float* region, cudaStream_t s) {
+  ban_base_kernel<<<cdiv(bw.words, 128), 128, 0, s>>>(c->bad_ids, c->n_bad, V, bw.words,
+                                                     reinterpret_cast<uint32_t*>(region + bw.base));
+  return check_launch("ban_base_kernel");
+}
+
+int ban_rows(const gic_decode_constraints_t* c, int M, int V, int L, int t, int eos, const int* fin, const int64_t* ids,
+             const int32_t* trace, int B, int K, const BanWs& bw, float* region, cudaStream_t s) {
+  BanRowsArgs a;
+  a.ban = reinterpret_cast<uint32_t*>(region + bw.ban);
+  a.base = reinterpret_cast<const uint32_t*>(region + bw.base);
+  a.fin = fin; a.ids = ids; a.trace = reinterpret_cast<const int2*>(trace);
+  a.prefix = reinterpret_cast<int*>(region + bw.prefix);
+  a.M = M; a.words = bw.words; a.V = V; a.L = L; a.K = K; a.B = B; a.t = t; a.eos = eos;
+  a.min_length = c->min_length; a.ngram = c->no_repeat_ngram_size;
+  ban_rows_kernel<<<cdiv(M, BR_WARPS), BR_WARPS * 32, 0, s>>>(a);
+  return check_launch("ban_rows_kernel");
 }
 
 }  // namespace gic

@@ -51,12 +51,13 @@ int lstm_step_tc(const float*, int, const float*, const float*, const float*, co
 // beam_tcgen05.cu
 size_t vocab_topk_ws_floats(int M, int V, int K);
 int vocab_topk(int mode, const float* h, const float* W_out, const float* b_out, int M, int V, int H, int K, float* logp,
-               int64_t* tokens, float* lse, float* ws, cudaStream_t s);
-size_t decode_beam_ws_floats(int B, int K, int L, int V, int E, int H, int layers);
+               int64_t* tokens, float* lse, const uint32_t* ban, float* ws, cudaStream_t s);
+size_t decode_beam_ws_floats(int B, int K, int L, int V, int E, int H, int layers, const gic_decode_constraints_t* c);
 int decode_beam(int mode, const float* features, const float* W_emb, const float* const* W_ih, const float* const* W_hh,
                 const float* const* b_ih, const float* const* b_hh, const float* W_out, const float* b_out, int B, int K,
-                int L, int V, int E, int H, int layers, int64_t eos, float length_penalty, int64_t* ids, float* scores,
-                int32_t* lengths, int32_t* trace, float* ws, cudaStream_t s);
+                int L, int V, int E, int H, int layers, int64_t eos, float length_penalty,
+                const gic_decode_constraints_t* c, int64_t* ids, float* scores, int32_t* lengths, int32_t* trace, float* ws,
+                cudaStream_t s);
 size_t vocab_target_ws_floats(int M, int V);
 int vocab_target_scores(int mode, const float* h, const float* W_out, const float* b_out, const int64_t* targets, int M, int V,
                         int H, int L, const int32_t* lengths, float* logp, float* lse, int64_t* argmax, uint8_t* correct,
@@ -65,7 +66,8 @@ int teacher_inputs(const float* features, const int64_t* captions, const float* 
                    cudaStream_t s);
 size_t vocab_sample_ws_floats(int M, int V, int top_k);
 int vocab_sample(int mode, const float* h, const float* W_out, const float* b_out, int M, int V, int H, int t, float T,
-                 int top_k, float top_p, int64_t* tokens, float* logp, const SampleDecode* d, float* ws, cudaStream_t s);
+                 int top_k, float top_p, int64_t* tokens, float* logp, const SampleDecode* d, const uint32_t* ban, float* ws,
+                 cudaStream_t s);
 int sample_init(const float* features, int n, int M, const SampleDecode& d, cudaStream_t s);
 // disc.cu
 int scale_inplace(float*, size_t, float, cudaStream_t);
@@ -344,10 +346,10 @@ static int score_captions(int mode, const float* features, const int64_t* captio
 }
 
 // sampled-caption workspace (floats): x[M][E] | per layer: h[2][M][H] (ping-pong), c[M][H] (updated in place)
-// | gates[M][4H] | fin[M] | sampling-step workspace, M = B n
+// | gates[M][4H] | fin[M] | sampling-step workspace | ban bitmaps (BanWs, size 0 unconstrained), M = B n
 struct SampleCaptionsWs {
-  size_t x, state, per_layer, gates, fin, step, total;
-  SampleCaptionsWs(int M, int V, int E, int H, int layers, int top_k) {
+  size_t x, state, per_layer, gates, fin, step, ban, total;
+  SampleCaptionsWs(int M, int V, int E, int H, int layers, int top_k, int L = 1, const gic_decode_constraints_t* c = nullptr) {
     const size_t MH = a4((size_t)M * H);
     x = 0;
     state = a4((size_t)M * E);
@@ -355,20 +357,23 @@ struct SampleCaptionsWs {
     gates = state + (size_t)layers * per_layer;
     fin = gates + a4((size_t)M * 4 * H);
     step = fin + a4((size_t)M);
-    total = step + vocab_sample_ws_floats(M, V, top_k);
+    ban = step + vocab_sample_ws_floats(M, V, top_k);
+    total = ban + BanWs(M, V, L, c).total;
   }
 };
 
 // n sampled captions per image (gic_sample_captions): rows m = b n + j start from features[b] with h = c = 0; every step
 // runs the LSTM stack (lstm_stack_step, as scoring does), the producer and sample_rows_kernel, which appends the token and
-// writes the next input.  Always L steps, no host sync.
+// writes the next input.  Always L steps, no host sync.  With constraints (c != NULL) ban_rows_kernel rebuilds the rows'
+// ban bitmaps before the producer of every step.
 static int sample_captions(int mode, const float* features, const float* W_emb, const float* const* W_ih,
                            const float* const* W_hh, const float* const* b_ih, const float* const* b_hh, const float* W_out,
                            const float* b_out, int B, int n, int L, int V, int E, int H, int layers, int eos, float T,
-                           int top_k, float top_p, int64_t* ids, float* caption_logp, int32_t* lengths, float* ws,
-                           cudaStream_t s) {
+                           int top_k, float top_p, const gic_decode_constraints_t* c, int64_t* ids, float* caption_logp,
+                           int32_t* lengths, float* ws, cudaStream_t s) {
   const int M = B * n;
-  const SampleCaptionsWs w(M, V, E, H, layers, top_k);
+  const SampleCaptionsWs w(M, V, E, H, layers, top_k, L, c);
+  const BanWs bw(M, V, L, c);
   const size_t MH = a4((size_t)M * H);
   SampleDecode d = {ids, reinterpret_cast<int*>(ws + w.fin), lengths, caption_logp, ws + w.x, W_emb, L, E, eos};
   GIC_TRY(sample_init(features, n, M, d, s));
@@ -377,6 +382,7 @@ static int sample_captions(int mode, const float* features, const float* W_emb, 
     cudaMemsetAsync(st, 0, (size_t)M * H * sizeof(float), s);                    // h of step -1
     cudaMemsetAsync(st + 2 * MH, 0, (size_t)M * H * sizeof(float), s);          // c
   }
+  if (c) GIC_TRY(ban_base(c, V, bw, ws + w.ban, s));
   for (int t = 0; t < L; ++t) {
     LstmLayerIO io[8];
     for (int l = 0; l < layers; ++l) {
@@ -384,8 +390,9 @@ static int sample_captions(int mode, const float* features, const float* W_emb, 
       io[l] = {st + (t & 1) * MH, st + 2 * MH, st + ((t + 1) & 1) * MH, st + 2 * MH, nullptr};
     }
     GIC_TRY(lstm_stack_step(mode, ws + w.x, io, layers, W_ih, W_hh, b_ih, b_hh, M, E, H, nullptr, ws + w.gates, L, t, s));
+    if (c) GIC_TRY(ban_rows(c, M, V, L, t, eos, d.fin, ids, nullptr, B, n, bw, ws + w.ban, s));
     GIC_TRY(vocab_sample(mode, io[layers - 1].h_new, W_out, b_out, M, V, H, t, T, top_k, top_p, nullptr, nullptr, &d,
-                         ws + w.step, s));
+                         c ? reinterpret_cast<const uint32_t*>(ws + w.ban + bw.ban) : nullptr, ws + w.step, s));
   }
   return GIC_OK;
 }
@@ -939,6 +946,24 @@ int gic_pg_loss_fwd_bwd(const float* logits, const int64_t* ids, const float* Q,
   return pg_loss(logits, ids, Q, baseline_mode, B, L, V, loss, dlogits, logp, S(stream));
 }
 
+// Constrained generation: a constraint block with every constraint off is no constraint (NULL).
+static const gic_decode_constraints_t* active_constraints(const gic_decode_constraints_t* c) {
+  return (c && (c->min_length != 0 || c->no_repeat_ngram_size != 0 || c->n_bad != 0)) ? c : nullptr;
+}
+// GIC_ERR_SHAPE unless 0 <= min_length <= L, no_repeat_ngram_size >= 0, n_bad >= 0 and every step keeps at least
+// max(width, 1) allowed columns; GIC_ERR_NULL for n_bad > 0 without bad_ids
+static int constraints_check(const gic_decode_constraints_t* c, int L, int V, int width, const char* who) {
+  if (!c) return GIC_OK;
+  GIC_REQUIRE(c->min_length >= 0 && c->min_length <= L && c->no_repeat_ngram_size >= 0 && c->n_bad >= 0, GIC_ERR_SHAPE,
+              "%s: bad constraints min_length=%d no_repeat_ngram_size=%d n_bad=%d L=%d", who, c->min_length,
+              c->no_repeat_ngram_size, c->n_bad, L);
+  const long long allowed = (long long)V - c->n_bad - (c->min_length > 0 ? 1 : 0) - (c->no_repeat_ngram_size > 0 ? L - 1 : 0);
+  GIC_REQUIRE((width > 1 ? width : 1) <= allowed, GIC_ERR_SHAPE,
+              "%s: constraints may leave %lld allowed tokens of V=%d, fewer than %d", who, allowed, V, width > 1 ? width : 1);
+  GIC_REQUIRE(c->n_bad == 0 || c->bad_ids, GIC_ERR_NULL, "%s: NULL bad_ids with n_bad=%d", who, c->n_bad);
+  return GIC_OK;
+}
+
 size_t gic_vocab_topk_workspace_floats(int M, int V, int K) { return vocab_topk_ws_floats(M, V, K); }
 int gic_vocab_topk(int mode, const float* h, const float* W_out, const float* b_out, int M, int V, int H, int K,
                    float* logp, int64_t* tokens, float* lse, float* workspace, gic_stream_t stream) {
@@ -947,28 +972,52 @@ int gic_vocab_topk(int mode, const float* h, const float* W_out, const float* b_
               "vocab_topk: bad shape M=%d V=%d H=%d K=%d", M, V, H, K);
   if (M == 0) return GIC_OK;
   GIC_REQUIRE(h && W_out && b_out && logp && tokens && workspace, GIC_ERR_NULL, "vocab_topk: NULL pointer");
-  return vocab_topk(mode, h, W_out, b_out, M, V, H, K, logp, tokens, lse, workspace, S(stream));
+  return vocab_topk(mode, h, W_out, b_out, M, V, H, K, logp, tokens, lse, nullptr, workspace, S(stream));
+}
+int gic_vocab_topk_masked(int mode, const float* h, const float* W_out, const float* b_out, int M, int V, int H, int K,
+                          float* logp, int64_t* tokens, float* lse, const uint32_t* ban, float* workspace, gic_stream_t stream) {
+  GIC_TRY(require_device());
+  GIC_REQUIRE(M >= 0 && V >= 1 && H >= 1 && K >= 1 && K <= 16 && K <= V, GIC_ERR_SHAPE,
+              "vocab_topk_masked: bad shape M=%d V=%d H=%d K=%d", M, V, H, K);
+  if (M == 0) return GIC_OK;
+  GIC_REQUIRE(h && W_out && b_out && logp && tokens && ban && workspace, GIC_ERR_NULL, "vocab_topk_masked: NULL pointer");
+  return vocab_topk(mode, h, W_out, b_out, M, V, H, K, logp, tokens, lse, ban, workspace, S(stream));
 }
 size_t gic_decode_beam_workspace_floats(int B, int K, int L, int V, int E, int H, int layers) {
-  return decode_beam_ws_floats(B, K, L, V, E, H, layers);
+  return decode_beam_ws_floats(B, K, L, V, E, H, layers, nullptr);
+}
+size_t gic_decode_beam_constrained_workspace_floats(int B, int K, int L, int V, int E, int H, int layers,
+                                                    const gic_decode_constraints_t* c) {
+  return decode_beam_ws_floats(B, K, L, V, E, H, layers, active_constraints(c));
 }
 int gic_decode_beam(int mode, const float* features, const float* W_emb, const float* const* W_ih,
                     const float* const* W_hh, const float* const* b_ih, const float* const* b_hh,
                     const float* W_out, const float* b_out, int B, int K, int L, int V, int E, int H, int layers,
                     int64_t eos_id, float length_penalty, int64_t* ids, float* scores, int32_t* lengths, int32_t* trace,
                     float* workspace, gic_stream_t stream) {
+  return gic_decode_beam_constrained(mode, features, W_emb, W_ih, W_hh, b_ih, b_hh, W_out, b_out, B, K, L, V, E, H, layers,
+                                     eos_id, length_penalty, nullptr, ids, scores, lengths, trace, workspace, stream);
+}
+int gic_decode_beam_constrained(int mode, const float* features, const float* W_emb, const float* const* W_ih,
+                                const float* const* W_hh, const float* const* b_ih, const float* const* b_hh,
+                                const float* W_out, const float* b_out, int B, int K, int L, int V, int E, int H, int layers,
+                                int64_t eos_id, float length_penalty, const gic_decode_constraints_t* constraints,
+                                int64_t* ids, float* scores, int32_t* lengths, int32_t* trace, float* workspace,
+                                gic_stream_t stream) {
   GIC_TRY(require_device());
   GIC_REQUIRE(B >= 0 && K >= 1 && K <= 16 && K <= V && L >= 1 && V >= 1 && E >= 1 && H >= 1 && layers >= 1 && layers <= 8 &&
                   eos_id >= 0 && eos_id < V,
               GIC_ERR_SHAPE, "decode_beam: bad shape B=%d K=%d L=%d V=%d E=%d H=%d layers=%d eos_id=%lld", B, K, L, V, E, H,
               layers, (long long)eos_id);
+  const gic_decode_constraints_t* c = active_constraints(constraints);
+  GIC_TRY(constraints_check(c, L, V, K, "decode_beam"));
   if (B == 0) return GIC_OK;
   GIC_REQUIRE(features && W_emb && W_ih && W_hh && b_ih && b_hh && W_out && b_out && ids && scores && lengths && workspace,
               GIC_ERR_NULL, "decode_beam: NULL pointer");
   for (int l = 0; l < layers; ++l)
     GIC_REQUIRE(W_ih[l] && W_hh[l] && b_ih[l] && b_hh[l], GIC_ERR_NULL, "decode_beam: NULL weight of layer %d", l);
   return decode_beam(mode, features, W_emb, W_ih, W_hh, b_ih, b_hh, W_out, b_out, B, K, L, V, E, H, layers, eos_id,
-                     length_penalty, ids, scores, lengths, trace, workspace, S(stream));
+                     length_penalty, c, ids, scores, lengths, trace, workspace, S(stream));
 }
 
 size_t gic_vocab_target_logp_workspace_floats(int M, int V) { return vocab_target_ws_floats(M, V); }
@@ -995,29 +1044,58 @@ int gic_vocab_sample(int mode, const float* h, const float* W_out, const float* 
               "vocab_sample: bad sampling arguments temperature=%g top_k=%d top_p=%g V=%d", temperature, top_k, top_p, V);
   if (M == 0) return GIC_OK;
   GIC_REQUIRE(h && W_out && b_out && tokens && logp && workspace, GIC_ERR_NULL, "vocab_sample: NULL pointer");
-  return vocab_sample(mode, h, W_out, b_out, M, V, H, step, temperature, top_k, top_p, tokens, logp, nullptr, workspace,
+  return vocab_sample(mode, h, W_out, b_out, M, V, H, step, temperature, top_k, top_p, tokens, logp, nullptr, nullptr,
+                      workspace, S(stream));
+}
+int gic_vocab_sample_masked(int mode, const float* h, const float* W_out, const float* b_out, int M, int V, int H, int step,
+                            float temperature, int top_k, float top_p, int64_t* tokens, float* logp, const uint32_t* ban,
+                            float* workspace, gic_stream_t stream) {
+  GIC_REQUIRE(M >= 0 && V >= 1 && H >= 1 && step >= 0, GIC_ERR_SHAPE, "vocab_sample_masked: bad shape M=%d V=%d H=%d step=%d",
+              M, V, H, step);
+  GIC_REQUIRE(sample_args_ok(temperature, top_k, top_p, V), GIC_ERR_SHAPE,
+              "vocab_sample_masked: bad sampling arguments temperature=%g top_k=%d top_p=%g V=%d", temperature, top_k, top_p,
+              V);
+  if (M == 0) return GIC_OK;
+  GIC_REQUIRE(h && W_out && b_out && tokens && logp && ban && workspace, GIC_ERR_NULL, "vocab_sample_masked: NULL pointer");
+  return vocab_sample(mode, h, W_out, b_out, M, V, H, step, temperature, top_k, top_p, tokens, logp, nullptr, ban, workspace,
                       S(stream));
 }
 size_t gic_sample_captions_workspace_floats(int B, int n, int V, int E, int H, int layers, int top_k) {
   return SampleCaptionsWs(B * n, V, E, H, layers, top_k).total;
+}
+size_t gic_sample_captions_constrained_workspace_floats(int B, int n, int L, int V, int E, int H, int layers, int top_k,
+                                                        const gic_decode_constraints_t* c) {
+  return SampleCaptionsWs(B * n, V, E, H, layers, top_k, L, active_constraints(c)).total;
 }
 int gic_sample_captions(int mode, const float* features, const float* W_emb, const float* const* W_ih,
                         const float* const* W_hh, const float* const* b_ih, const float* const* b_hh, const float* W_out,
                         const float* b_out, int B, int n, int L, int V, int E, int H, int layers, int64_t eos_id,
                         float temperature, int top_k, float top_p, int64_t* ids, float* caption_logp, int32_t* lengths,
                         float* workspace, gic_stream_t stream) {
+  return gic_sample_captions_constrained(mode, features, W_emb, W_ih, W_hh, b_ih, b_hh, W_out, b_out, B, n, L, V, E, H, layers,
+                                         eos_id, temperature, top_k, top_p, nullptr, ids, caption_logp, lengths, workspace,
+                                         stream);
+}
+int gic_sample_captions_constrained(int mode, const float* features, const float* W_emb, const float* const* W_ih,
+                                    const float* const* W_hh, const float* const* b_ih, const float* const* b_hh,
+                                    const float* W_out, const float* b_out, int B, int n, int L, int V, int E, int H,
+                                    int layers, int64_t eos_id, float temperature, int top_k, float top_p,
+                                    const gic_decode_constraints_t* constraints, int64_t* ids, float* caption_logp,
+                                    int32_t* lengths, float* workspace, gic_stream_t stream) {
   GIC_REQUIRE(B >= 0 && n >= 1 && L >= 1 && V >= 1 && E >= 1 && H >= 1 && layers >= 1 && layers <= 8 && eos_id >= 0 &&
                   eos_id < V, GIC_ERR_SHAPE, "sample_captions: bad shape B=%d n=%d L=%d V=%d E=%d H=%d layers=%d eos_id=%lld",
               B, n, L, V, E, H, layers, (long long)eos_id);
   GIC_REQUIRE(sample_args_ok(temperature, top_k, top_p, V), GIC_ERR_SHAPE,
               "sample_captions: bad sampling arguments temperature=%g top_k=%d top_p=%g V=%d", temperature, top_k, top_p, V);
+  const gic_decode_constraints_t* c = active_constraints(constraints);
+  GIC_TRY(constraints_check(c, L, V, top_k, "sample_captions"));
   if (B == 0) return GIC_OK;
   GIC_REQUIRE(features && W_emb && W_ih && W_hh && b_ih && b_hh && W_out && b_out && ids && caption_logp && lengths &&
                   workspace, GIC_ERR_NULL, "sample_captions: NULL pointer");
   for (int l = 0; l < layers; ++l)
     GIC_REQUIRE(W_ih[l] && W_hh[l] && b_ih[l] && b_hh[l], GIC_ERR_NULL, "sample_captions: NULL weight of layer %d", l);
   return sample_captions(mode, features, W_emb, W_ih, W_hh, b_ih, b_hh, W_out, b_out, B, n, L, V, E, H, layers, (int)eos_id,
-                         temperature, top_k, top_p, ids, caption_logp, lengths, workspace, S(stream));
+                         temperature, top_k, top_p, c, ids, caption_logp, lengths, workspace, S(stream));
 }
 
 size_t gic_score_captions_workspace_floats(int B, int L, int V, int E, int H, int layers) {

@@ -112,6 +112,27 @@ struct SampleDecode {
   int L, E, eos;
 };
 
+// Constrained generation (beam_tcgen05.cu ban_rows_kernel): the ban-bitmap regions of a decode's workspace, in floats from
+// the region's start; all of size 0 when c == NULL (unconstrained).  base[words] (the bad ids) | ban[M][words] (per row,
+// rebuilt every step) | prefix[M][L] (int, the rows' prefixes; no_repeat_ngram_size >= 1 only), words = ceil(V / 32).
+struct BanWs {
+  size_t base, ban, prefix, total;
+  int words;
+  BanWs(int M, int V, int L, const gic_decode_constraints_t* c) {
+    words = (V + 31) / 32;
+    const bool on = c != nullptr;
+    base = 0;
+    ban = on ? a4((size_t)words) : 0;
+    prefix = ban + (on ? a4((size_t)M * words) : 0);
+    total = prefix + ((on && c->no_repeat_ngram_size > 0) ? a4((size_t)M * L) : 0);
+  }
+};
+// base bitmap of c->bad_ids (once per call), then per step the bitmap of rows m < M; fin[M] marks frozen rows (skipped),
+// the prefix is ids[m, :t] (ids[M][L], sampling) or the trace[L][B][K] backtrack of beam slot m % K (ids == NULL)
+int ban_base(const gic_decode_constraints_t* c, int V, const BanWs& bw, float* region, cudaStream_t s);
+int ban_rows(const gic_decode_constraints_t* c, int M, int V, int L, int t, int eos, const int* fin, const int64_t* ids,
+             const int32_t* trace, int B, int K, const BanWs& bw, float* region, cudaStream_t s);
+
 // dz (bf16) = T p (demb W_e - dot) and db_out = colsum(dz) in one streaming tcgen05 kernel (dz_fused_tcgen05.cu)
 int dz_fused_tc(const float* demb, int K, const float* W_e, const float* p, const float* dot, float T, const float* T_dev,
                 int M, int V, void* dz_bf, int Vp, float* db_out, int accumulate, cudaStream_t stream, bool* handled);

@@ -281,9 +281,41 @@ class _DecodeSampleAttn(torch.autograd.Function):
         return (dfeat, None, None, None, None, None, None, dW_k, dW_v, dW_q, dw_e, dW_emb, dW_out, db_out, *dlstm)
 
 
-def decode_beam(dec, features, beam_size, max_caption_len, length_penalty=0.0, eos_id=2, mode=None, trace=None):
-    """gic_decode_beam over the decoder's weights -> (ids[B,K,L] int64, scores[B,K], lengths[B,K] int32).  trace[L,B,K,2]
-    (int32, optional) receives the (parent slot, token) chosen at every step."""
+def check_constraints(min_length, no_repeat_ngram_size, bad_ids, max_caption_len, V, width):
+    """ValueError for constraints gic_decode_beam_constrained / gic_sample_captions_constrained reject, and bad ids outside
+    [0, V) (checked on the host, before any GPU work); width = beam_size, or top_k for sampling."""
+    L = int(max_caption_len)
+    if not 0 <= int(min_length) <= L:
+        raise ValueError("min_length must lie in [0, max_caption_len] = [0, %d]" % L)
+    if int(no_repeat_ngram_size) < 0:
+        raise ValueError("no_repeat_ngram_size must be >= 0")
+    bad = [int(w) for w in (bad_ids if bad_ids is not None else ())]
+    if any(not 0 <= w < V for w in bad):
+        raise ValueError("bad_ids must lie in [0, %d)" % V)
+    allowed = V - len(bad) - (int(min_length) > 0) - (L - 1 if int(no_repeat_ngram_size) > 0 else 0)
+    if max(int(width), 1) > allowed:
+        raise ValueError("the constraints may leave %d allowed tokens per step, fewer than %d" % (allowed, max(int(width), 1)))
+
+
+def _constraints(min_length, no_repeat_ngram_size, bad_ids, dev):
+    """(gic_decode_constraints_t or None, the device bad ids it points at).  bad_ids is a host sequence, copied here, or
+    an int64 tensor already on the device (no copy: the call stays capturable into a CUDA graph)."""
+    if torch.is_tensor(bad_ids) and bad_ids.is_cuda:
+        ids = bad_ids.to(torch.int64).contiguous()
+    else:
+        bad = [int(w) for w in (bad_ids if bad_ids is not None else ())]
+        ids = torch.tensor(bad, dtype=torch.int64, device=dev) if bad else None
+    n_bad = 0 if ids is None else ids.numel()
+    if int(min_length) == 0 and int(no_repeat_ngram_size) == 0 and n_bad == 0:
+        return None, None
+    return _lib.DecodeConstraints(int(min_length), int(no_repeat_ngram_size), _lib.ptr(ids), n_bad), ids
+
+
+def decode_beam(dec, features, beam_size, max_caption_len, length_penalty=0.0, eos_id=2, mode=None, trace=None,
+                min_length=0, no_repeat_ngram_size=0, bad_ids=None):
+    """gic_decode_beam_constrained over the decoder's weights -> (ids[B,K,L] int64, scores[B,K], lengths[B,K] int32).
+    trace[L,B,K,2] (int32, optional) receives the (parent slot, token) chosen at every step.  min_length /
+    no_repeat_ngram_size / bad_ids: the constraints of include/gic_b200.h gic_decode_constraints_t (none by default)."""
     _lib.require_cuda()
     lib = _lib.lib()
     mode = gic_b200.get_gemm_mode() if mode is None else mode
@@ -298,11 +330,15 @@ def decode_beam(dec, features, beam_size, max_caption_len, length_penalty=0.0, e
     ids = torch.empty(B, K, L, dtype=torch.int64, device=dev)
     scores = torch.empty(B, K, device=dev)
     lengths = torch.empty(B, K, dtype=torch.int32, device=dev)
-    ws = torch.empty(lib.gic_decode_beam_workspace_floats(B, K, L, V, E, H, layers), device=dev)
-    _lib.check(lib.gic_decode_beam(mode, _lib.ptr(features), _lib.ptr(W_emb), _lib.ptr_array(W_ih), _lib.ptr_array(W_hh),
-                                   _lib.ptr_array(b_ih), _lib.ptr_array(b_hh), _lib.ptr(W_out), _lib.ptr(b_out), B, K, L, V,
-                                   E, H, layers, int(eos_id), float(length_penalty), _lib.ptr(ids), _lib.ptr(scores),
-                                   _lib.ptr(lengths), _lib.ptr(trace), _lib.ptr(ws), _lib.stream()), "gic_decode_beam")
+    c, _bad = _constraints(min_length, no_repeat_ngram_size, bad_ids, dev)
+    cp = None if c is None else C.byref(c)
+    ws = torch.empty(lib.gic_decode_beam_constrained_workspace_floats(B, K, L, V, E, H, layers, cp), device=dev)
+    _lib.check(lib.gic_decode_beam_constrained(mode, _lib.ptr(features), _lib.ptr(W_emb), _lib.ptr_array(W_ih),
+                                               _lib.ptr_array(W_hh), _lib.ptr_array(b_ih), _lib.ptr_array(b_hh),
+                                               _lib.ptr(W_out), _lib.ptr(b_out), B, K, L, V, E, H, layers, int(eos_id),
+                                               float(length_penalty), cp, _lib.ptr(ids), _lib.ptr(scores),
+                                               _lib.ptr(lengths), _lib.ptr(trace), _lib.ptr(ws), _lib.stream()),
+               "gic_decode_beam_constrained")
     return ids, scores, lengths
 
 
@@ -357,9 +393,10 @@ def check_sample_args(num_samples, max_caption_len, temperature, top_k, top_p, e
 
 
 def sample_captions(dec, features, num_samples=1, max_caption_len=34, temperature=1.0, top_k=0, top_p=1.0, eos_id=2,
-                    mode=None):
-    """gic_sample_captions over the decoder's weights -> (ids[B,n,L] int64, caption_logp[B,n], lengths[B,n] int32).  The
-    draws read the library's Philox state (gic_set_rng) of the current context."""
+                    mode=None, min_length=0, no_repeat_ngram_size=0, bad_ids=None):
+    """gic_sample_captions_constrained over the decoder's weights -> (ids[B,n,L] int64, caption_logp[B,n], lengths[B,n]
+    int32).  The draws read the library's Philox state (gic_set_rng) of the current context.  min_length /
+    no_repeat_ngram_size / bad_ids: the constraints of include/gic_b200.h gic_decode_constraints_t (none by default)."""
     _lib.require_cuda()
     lib = _lib.lib()
     mode = gic_b200.get_gemm_mode() if mode is None else mode
@@ -374,12 +411,16 @@ def sample_captions(dec, features, num_samples=1, max_caption_len=34, temperatur
     ids = torch.empty(B, n, L, dtype=torch.int64, device=dev)
     logp = torch.empty(B, n, device=dev)
     lengths = torch.empty(B, n, dtype=torch.int32, device=dev)
-    ws = torch.empty(lib.gic_sample_captions_workspace_floats(B, n, V, E, H, layers, int(top_k)), device=dev)
-    _lib.check(lib.gic_sample_captions(mode, _lib.ptr(features), _lib.ptr(W_emb), _lib.ptr_array(W_ih), _lib.ptr_array(W_hh),
-                                       _lib.ptr_array(b_ih), _lib.ptr_array(b_hh), _lib.ptr(W_out), _lib.ptr(b_out), B, n, L,
-                                       V, E, H, layers, int(eos_id), float(temperature), int(top_k), float(top_p),
-                                       _lib.ptr(ids), _lib.ptr(logp), _lib.ptr(lengths), _lib.ptr(ws), _lib.stream()),
-               "gic_sample_captions")
+    c, _bad = _constraints(min_length, no_repeat_ngram_size, bad_ids, dev)
+    cp = None if c is None else C.byref(c)
+    ws = torch.empty(lib.gic_sample_captions_constrained_workspace_floats(B, n, L, V, E, H, layers, int(top_k), cp),
+                     device=dev)
+    _lib.check(lib.gic_sample_captions_constrained(mode, _lib.ptr(features), _lib.ptr(W_emb), _lib.ptr_array(W_ih),
+                                                   _lib.ptr_array(W_hh), _lib.ptr_array(b_ih), _lib.ptr_array(b_hh),
+                                                   _lib.ptr(W_out), _lib.ptr(b_out), B, n, L, V, E, H, layers, int(eos_id),
+                                                   float(temperature), int(top_k), float(top_p), cp, _lib.ptr(ids),
+                                                   _lib.ptr(logp), _lib.ptr(lengths), _lib.ptr(ws), _lib.stream()),
+               "gic_sample_captions_constrained")
     return ids, logp, lengths
 
 
@@ -439,14 +480,23 @@ class Decoder(nn.Module):
                                    *self.lstm_params())
 
     @torch.no_grad()
-    def beam_search(self, features, beam_size=3, max_caption_len=34, length_penalty=0.0, eos_id=2):
+    def beam_search(self, features, beam_size=3, max_caption_len=34, length_penalty=0.0, eos_id=2, min_length=0,
+                    no_repeat_ngram_size=0, bad_ids=None):
         """The most likely captions of features[B,E] (the step-0 input, as in sample) by beam search (EXTENSION; the
         reference has none, oracle/ref_beam.py defines it) -> (ids[B,K,L], scores[B,K], lengths[B,K]), the K beams of each
         image best first by score / length ** length_penalty.  ids hold PAD (0) after <E> (eos_id); scores are sums of
-        log-probabilities; lengths count tokens up to and including <E>.  beam_size = 1 is greedy decoding."""
+        log-probabilities; lengths count tokens up to and including <E>.  beam_size = 1 is greedy decoding.
+
+        Optional constraints (oracle/ref_constrain.py banned_tokens), none by default: ``min_length`` bans <E> until the
+        caption has that many tokens; ``no_repeat_ngram_size`` = n bans every token that would repeat an n-gram of the
+        caption; ``bad_ids`` (a host sequence of ids) are never emitted -- ``bad_ids=(0, 1, 3)`` keeps PAD, <S> and <UNK>
+        out of captions.  Scores stay log-probabilities of the unconstrained model.  Raises ValueError on an invalid
+        constraint before any GPU work."""
         if self.attention:
             raise NotImplementedError("beam search is implemented for the plain LSTM decoder, not the attention cell")
-        return decode_beam(self, features, beam_size, max_caption_len, length_penalty, eos_id)
+        check_constraints(min_length, no_repeat_ngram_size, bad_ids, max_caption_len, self.linear.out_features, beam_size)
+        return decode_beam(self, features, beam_size, max_caption_len, length_penalty, eos_id, min_length=min_length,
+                           no_repeat_ngram_size=no_repeat_ngram_size, bad_ids=bad_ids)
 
     @torch.no_grad()
     def score(self, features, captions, lengths=None):
@@ -465,19 +515,25 @@ class Decoder(nn.Module):
         return logp, total, corr.bool()
 
     @torch.no_grad()
-    def sample_captions(self, features, num_samples=1, max_caption_len=34, temperature=1.0, top_k=0, top_p=1.0, eos_id=2):
+    def sample_captions(self, features, num_samples=1, max_caption_len=34, temperature=1.0, top_k=0, top_p=1.0, eos_id=2,
+                        min_length=0, no_repeat_ngram_size=0, bad_ids=None):
         """Draw num_samples captions per row of features[B,E] (EXTENSION; oracle/ref_sample.py sample_captions defines it)
         -> (ids[B,n,L], caption_logp[B,n], lengths[B,n]).  Each step draws from softmax(logits / temperature) restricted
         to the top_k tokens (0: the whole vocabulary), then to the smallest prefix of them holding top_p of the mass
         (top_p < 1 needs top_k >= 1).  ``temperature`` divides the logits; it is not ``Decoder.temperature``, which scales
         the Gumbel-softmax output of ``sample``.  A caption stops at <E> (eos_id): PAD (0) follows, lengths count tokens up
         to and including <E>, and caption_logp is the caption's log-likelihood under the unfiltered model at temperature 1.
-        Draws come from the library's Philox stream (gic_set_rng); GANInstructor.sample_captions seeds it.  Raises
-        ValueError on an invalid argument before any GPU work."""
+        Draws come from the library's Philox stream (gic_set_rng); GANInstructor.sample_captions seeds it.  The optional
+        constraints ``min_length``, ``no_repeat_ngram_size`` and ``bad_ids`` are those of beam_search (e.g.
+        ``bad_ids=(0, 1, 3)`` for PAD, <S> and <UNK>): banned tokens leave the candidate set before top_k / top_p are
+        applied.  Raises ValueError on an invalid argument before any GPU work."""
         if self.attention:
             raise NotImplementedError("caption sampling is implemented for the plain LSTM decoder, not the attention cell")
-        check_sample_args(num_samples, max_caption_len, temperature, top_k, top_p, eos_id, self.linear.out_features)
-        return sample_captions(self, features, num_samples, max_caption_len, temperature, top_k, top_p, eos_id)
+        V = self.linear.out_features
+        check_sample_args(num_samples, max_caption_len, temperature, top_k, top_p, eos_id, V)
+        check_constraints(min_length, no_repeat_ngram_size, bad_ids, max_caption_len, V, top_k)
+        return sample_captions(self, features, num_samples, max_caption_len, temperature, top_k, top_p, eos_id,
+                               min_length=min_length, no_repeat_ngram_size=no_repeat_ngram_size, bad_ids=bad_ids)
 
     def add_gumbel(self, o_t, eps=1e-10, gpu=0):
         """Kept for interface parity (src/generator.py:84-96); the hot path fuses this into the sampler."""

@@ -719,37 +719,45 @@ class GANInstructor:
     # ---- EXTENSION: caption generation by beam search (the reference has none) -------------------------------------
     @_in_ctx
     @torch.no_grad()
-    def generate(self, pooled=None, batch_size=None, beam_size=3, max_caption_len=34, length_penalty=0.0):
+    def generate(self, pooled=None, batch_size=None, beam_size=3, max_caption_len=34, length_penalty=0.0, min_length=0,
+                 no_repeat_ngram_size=0, bad_ids=None):
         """Captions of a trained generator -> (ids[B,K,L], scores[B,K], lengths[B,K]) (Decoder.beam_search).  Conditional
         mode: the pooled CNN features [B, feature_dim] go through the encoder projection in eval mode (running statistics,
         as gen.eval() would); unconditional mode: every caption starts from embed.weight[1] (<S>), batch_size of them.
-        Inference only: parameters, gradients, optimizer state, step counters, temperature and the library's random stream
-        are left as they were."""
-        _lib.require_cuda()
+        min_length / no_repeat_ngram_size / bad_ids constrain the search as in Decoder.beam_search (none by default;
+        ``bad_ids=(tasks.PAD, tasks.START, tasks.UNK)`` keeps those tokens out of the captions).  Inference only: parameters, gradients,
+        optimizer state, step counters, temperature and the library's random stream are left as they were."""
+        from .generator import check_constraints
         dec = self.gen.decoder
+        check_constraints(min_length, no_repeat_ngram_size, bad_ids, max_caption_len, dec.linear.out_features, beam_size)
+        _lib.require_cuda()
         if not self.cgan and batch_size is None:
             if pooled is None:
                 raise ValueError("unconditional generation needs batch_size")
             batch_size = pooled.shape[0]
         feats = self._start_features(pooled, batch_size)
-        return dec.beam_search(feats, beam_size=beam_size, max_caption_len=max_caption_len, length_penalty=length_penalty)
+        return dec.beam_search(feats, beam_size=beam_size, max_caption_len=max_caption_len, length_penalty=length_penalty,
+                               min_length=min_length, no_repeat_ngram_size=no_repeat_ngram_size, bad_ids=bad_ids)
 
     # ---- EXTENSION: sampled caption generation (temperature / top-k / top-p draws, several captions per image) ----------
     @_in_ctx
     @torch.no_grad()
     def sample_captions(self, pooled=None, batch_size=None, num_samples=1, max_caption_len=34, temperature=1.0, top_k=0,
-                        top_p=1.0, seed=None):
+                        top_p=1.0, seed=None, min_length=0, no_repeat_ngram_size=0, bad_ids=None):
         """num_samples drawn captions per image -> (ids[B,n,L], caption_logp[B,n], lengths[B,n]) (Decoder.sample_captions),
         from the step-0 input generate uses (eval-mode encoder projection of pooled, or embed.weight[1] when unconditional).
         ``seed`` keys the library's Philox stream for this call; None takes one draw from torch's default generator, so
         torch.manual_seed makes the call reproducible.  ``temperature`` divides the logits (not Decoder.temperature).
-        Leaves parameters, gradients, optimizer state, step counters, temperature and the instructor's random stream as
-        they were; raises ValueError on an invalid argument before any GPU work."""
-        from .generator import check_sample_args
+        min_length / no_repeat_ngram_size / bad_ids constrain the draws as in Decoder.sample_captions (none by default;
+        ``bad_ids=(tasks.PAD, tasks.START, tasks.UNK)`` keeps those tokens out of the captions).  Leaves parameters, gradients, optimizer
+        state, step counters, temperature and the instructor's random stream as they were; raises ValueError on an invalid
+        argument before any GPU work."""
+        from .generator import check_constraints, check_sample_args
         dec = self.gen.decoder
         if dec.attention:
             raise NotImplementedError("caption sampling is implemented for the plain LSTM decoder, not the attention cell")
         check_sample_args(num_samples, max_caption_len, temperature, top_k, top_p, END, dec.linear.out_features)
+        check_constraints(min_length, no_repeat_ngram_size, bad_ids, max_caption_len, dec.linear.out_features, top_k)
         if not self.cgan and batch_size is None:
             if pooled is None:
                 raise ValueError("unconditional generation needs batch_size")
@@ -764,7 +772,8 @@ class GANInstructor:
         lib.gic_set_rng(int(seed) & ((1 << 64) - 1), 0, None)
         try:
             return dec.sample_captions(feats, num_samples=num_samples, max_caption_len=max_caption_len,
-                                       temperature=temperature, top_k=top_k, top_p=top_p, eos_id=END)
+                                       temperature=temperature, top_k=top_k, top_p=top_p, eos_id=END, min_length=min_length,
+                                       no_repeat_ngram_size=no_repeat_ngram_size, bad_ids=bad_ids)
         finally:
             lib.gic_set_rng(0, 0, None)
 

@@ -331,6 +331,60 @@ int gic_sample_captions(int mode, const float* features /*[B,E]*/, const float* 
                         float temperature, int top_k, float top_p, int64_t* ids /*[B n, L]*/, float* caption_logp /*[B n]*/,
                         int32_t* lengths /*[B n]*/, float* workspace, gic_stream_t stream);
 
+/* ---- constrained caption generation (EXTENSION, parity unpinned by reference: oracle/ref_constrain.py defines
+ * it).  Three optional constraints for beam search and sampled generation, all off by default (c == NULL, or every field 0,
+ * gives the unconstrained outputs bit for bit).  For row m at step t with generated prefix y[0..t-1] (sampling: ids[m, :t];
+ * beam search: the tokens along the slot's trace; the step-0 input is not part of it) the banned set Ban(m, t) is the union
+ * of
+ *   bad_ids inside [0, V) (ids outside are ignored);
+ *   {eos_id} while t + 1 < min_length: every returned length is >= min(min_length, L);
+ *   for n = no_repeat_ngram_size >= 1 and t >= n - 1: { y[s + n - 1] : 0 <= s <= t - n, y[s .. s + n - 2] ==
+ *     y[t - n + 1 .. t - 1] }: no n-gram occurs twice in a caption (n = 1 bans every token already emitted).
+ * Banned tokens are removed from the candidates and nothing else changes:
+ *   beam search: a live beam k offers (k, w) only for w outside Ban, at score_k + log_softmax(z)[w] (scores stay
+ *     log-probabilities of the unfiltered model); frozen beams still offer (k, PAD).
+ *   sampling: S is the top_k largest allowed z (every allowed column at top_k = 0), then the nucleus inside it; the keys
+ *     z / T + g(u[t, m, w]) read the same uniforms; at top_k = 0 this is an exact draw from softmax(z / T) renormalised over
+ *     the allowed columns.  caption_logp stays unfiltered at temperature 1, and lse is always over the full vocabulary.
+ * gic_decode_beam_constrained / gic_sample_captions_constrained take the arguments of gic_decode_beam / gic_sample_captions
+ *   plus the constraint block (may be NULL), with workspaces of their own queries.  The call stays free of host syncs.
+ *   GIC_ERR_SHAPE (before any work): min_length outside [0, L], no_repeat_ngram_size < 0, n_bad < 0, or
+ *   max(K, top_k, 1) > V - n_bad - (min_length > 0) - (no_repeat_ngram_size > 0 ? L - 1 : 0) (every step must keep enough
+ *   allowed candidates); GIC_ERR_NULL: n_bad > 0 with bad_ids NULL.
+ * gic_vocab_topk_masked / gic_vocab_sample_masked: gic_vocab_topk / gic_vocab_sample of one step with the banned columns
+ *   given directly: bit (w & 31) of ban[m * ceil(V / 32) + (w >> 5)] set bans column w of row m.  Same workspaces as the
+ *   unmasked calls.  lse stays over the full vocabulary.  A row with fewer than K allowed columns gets logp -inf and token
+ *   2^31 - 1 in the missing places (topk); a row without an allowed candidate draws token 0 (sample). */
+typedef struct gic_decode_constraints_t {
+  int min_length;              /* 0 = off */
+  int no_repeat_ngram_size;    /* 0 = off */
+  const int64_t* bad_ids;      /* device [n_bad]; ids outside [0, V) ignored */
+  int n_bad;
+} gic_decode_constraints_t;
+size_t gic_decode_beam_constrained_workspace_floats(int B, int K, int L, int V, int E, int H, int layers,
+                                                    const gic_decode_constraints_t* c);
+int gic_decode_beam_constrained(int mode, const float* features, const float* W_emb, const float* const* W_ih,
+                                const float* const* W_hh, const float* const* b_ih, const float* const* b_hh,
+                                const float* W_out, const float* b_out, int B, int K, int L, int V, int E, int H, int layers,
+                                int64_t eos_id, float length_penalty, const gic_decode_constraints_t* c,
+                                int64_t* ids /*[B,K,L]*/, float* scores /*[B,K]*/, int32_t* lengths /*[B,K]*/,
+                                int32_t* trace /*[L,B,K,2] or NULL*/, float* workspace, gic_stream_t stream);
+size_t gic_sample_captions_constrained_workspace_floats(int B, int n, int L, int V, int E, int H, int layers, int top_k,
+                                                        const gic_decode_constraints_t* c);
+int gic_sample_captions_constrained(int mode, const float* features /*[B,E]*/, const float* W_emb, const float* const* W_ih,
+                                    const float* const* W_hh, const float* const* b_ih, const float* const* b_hh,
+                                    const float* W_out, const float* b_out, int B, int n, int L, int V, int E, int H,
+                                    int layers, int64_t eos_id, float temperature, int top_k, float top_p,
+                                    const gic_decode_constraints_t* c, int64_t* ids /*[B n, L]*/,
+                                    float* caption_logp /*[B n]*/, int32_t* lengths /*[B n]*/, float* workspace,
+                                    gic_stream_t stream);
+int gic_vocab_topk_masked(int mode, const float* h /*[M,H]*/, const float* W_out, const float* b_out, int M, int V, int H,
+                          int K, float* logp, int64_t* tokens, float* lse, const uint32_t* ban /*[M, ceil(V/32)]*/,
+                          float* workspace, gic_stream_t stream);
+int gic_vocab_sample_masked(int mode, const float* h /*[M,H]*/, const float* W_out, const float* b_out, int M, int V, int H,
+                            int step, float temperature, int top_k, float top_p, int64_t* tokens /*[M]*/, float* logp /*[M]*/,
+                            const uint32_t* ban /*[M, ceil(V/32)]*/, float* workspace, gic_stream_t stream);
+
 /* ---- B1 (EXTENSION, parity unpinned by reference): additive attention over the CNN feature grid in the decode step.
  * The reference feeds one pooled vector at step 0 (src/generator.py:19-25,58) and has no attention.  Definition:
  *   once per image: Ak = grid W_k^T [B,P,Da], Av = grid W_v^T [B,P,E];  every step: q = h_{t-1} W_q^T,
